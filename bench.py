@@ -2,6 +2,7 @@
 """Benchmark of the rnascan_b200 hot path (contract: see the task statement / DESIGN.md).
 
     python bench.py --gpus 1 --steps 10 --warmup 3              # this framework (default)
+    python bench.py ... --dump-outputs DIR                      # also write the last timed step's results as .npy
     python bench.py --impl reference --gpus 1 --steps 3 ...     # the reference's CPU path
     torchrun ... bench.py --gpus N ...                          # one rank per GPU, the 1 Gnt split N ways
 
@@ -40,6 +41,7 @@ SS_BG = {"B": 0.0163181097311479, "E": 0.272087789050946, "H": 0.153012079123538
 ALGO_BYTES = {"c4": 29.0, "c2": 1.0, "c3": 5.0, "c5": 29.0}     # SURVEY.md section 8(d), per scored position
 N_MOTIFS_C5 = 256
 OTHERS_N = 125_000_000          # symbols per GPU of the side runs (configs 2, 3, 5) and of weak-scaling shards
+DUMP_ENTRY_BYTES = 48 << 20     # --dump-outputs: per-hit / per-window arrays beyond this are sampled (64 MB in all)
 
 
 # ----------------------------------------------------------------------------- helpers
@@ -160,6 +162,33 @@ def record_layout(n_symbols, seed):
 
 def scored_positions(lengths, W):
     return int(np.maximum(lengths - W + 1, 0).sum())
+
+
+def dump_outputs(directory, entries, fixed, seed=0):
+    """Write every array as <directory>/<name>.npy: float32 stays float32, anything else becomes float64.
+    `entries` holds arrays of one length (one element per hit or per window).  When they would take more than
+    DUMP_ENTRY_BYTES, each is cut to the same seeded sample of elements, in ascending order, and the sampled
+    indices are written as `sample_index`.  The `fixed` arrays are small and are written whole.  Arrays may be
+    numpy arrays or tensors; a device tensor is sampled on the device and only the sample is copied to the host."""
+    def as_float(a):
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        return a.astype(np.float32 if a.dtype == np.float32 else np.float64, copy=False)
+
+    def take(a, idx):
+        if not hasattr(a, "cpu"):
+            return np.asarray(a)[idx]
+        import torch
+        return a[torch.from_numpy(idx).to(a.device)]
+    n = len(next(iter(entries.values())))
+    per_entry = sum(4 if str(a.dtype).endswith("float32") else 8 for a in entries.values())
+    if n * per_entry > DUMP_ENTRY_BYTES:
+        idx = np.sort(np.random.default_rng(seed).choice(n, DUMP_ENTRY_BYTES // (per_entry + 8), replace=False))
+        entries = {name: take(a, idx) for name, a in entries.items()}
+        entries["sample_index"] = idx
+    out = {name: as_float(a) for name, a in list(entries.items()) + list(fixed.items())}
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def make_device_shard(n_symbols, seed, workload, device):
@@ -531,6 +560,29 @@ def measure(args, wl, steps, ctx, full, n_target):
         raise SystemExit("candidate buffer overflowed: %d > %d" % (int(hb.cand_counters[0].item()), hb.capacity))
     if wl == "c5":
         hits = int(c5_bases[-1].item())
+    if full and rank == 0 and args.dump_outputs:
+        # the last timed step's results as a caller of the path receives them, before the legs below reuse the buffers
+        found = None if wl == "c3" else (int(c5_bases[-1].item()) if wl == "c5" else int(hb.counters[0].item()))
+        if found is not None and found > hb.capacity:
+            raise SystemExit("hit buffer overflowed: %d > %d" % (found, hb.capacity))
+        if bgscan is not None:
+            pos, sq, sb = bgscan.results()
+            entries, counts8 = {"position": pos, "seq_score": sq, "struct_score": sb}, bgscan.counts_host.numpy()
+        elif ohscan is not None:
+            pos, sq, _ = ohscan.results()
+            entries, counts8 = {"position": pos, "seq_score": sq}, ohscan.counts_host.numpy()[:8]
+        elif wl == "c3":
+            entries, counts8 = {"score": dense_out[:max(0, n - W_MOTIF + 1)]}, counts_host.numpy()
+        else:
+            entries, counts8 = {"position": hb.pos[:found], "seq_score": hb.seq[:found]}, counts_host.numpy()
+            if wl != "c2":
+                entries["struct_score"] = hb.struct[:found]
+            if wl == "c5":
+                entries["motif"] = c5_motif[:found]
+        fixed = {"background_counts": counts8}
+        if wl == "c5":
+            fixed["motif_bases"] = c5_bases
+        dump_outputs(args.dump_outputs, entries, fixed)
 
     # ---- optional device timeline of a few more steps (CUPTI through torch.profiler; never part of a bench value)
     if full and args.trace and rank == 0:
@@ -1099,7 +1151,12 @@ def main():
     ap.add_argument("--no-others", action="store_true", dest="no_others",
                     help="skip the brief runs of the other configurations (other_workloads)")
     ap.add_argument("--c5-path", default="auto", choices=["auto", "cuda", "tensor"], dest="c5_path")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", dest="dump_outputs",
+                    help="after the timed steps, write what the last one computed on rank 0's shard as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB: larger per-hit or per-window outputs are a seeded sample)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,40 +1,39 @@
-"""Differential test against the REFERENCE ITSELF on randomly generated inputs (build container only).
+"""Differential test against the REFERENCE ITSELF on randomly generated inputs.
 
 For every seed a small input set is drawn -- FASTA records with DNA letters, lower case, N runs, empty and
 too-short records; matching one-hot structure contexts; averaged-profile files for some of the records; PFMs
-with zero cells; thresholds from -inf upwards; pseudocounts; background options -- and BOTH programs are run
-on it: the reference's own ``rnascan.rnascan.main()`` (unmodified code under /root/reference, with
-oracle/bio_shim standing in for Biopython and the reference's compiled ``_pwm.c``, exactly as
-tests/golden/make_golden.py runs it) and ``rnascan_b200.rnascan.main()`` with the device entry points swapped
-for the CPU oracle (tests/oracle_backend.py).  stdout must be byte-identical (averaged-profile runs under
-``--reference-compat``, see INTEGRATION.md section 0), exit codes equal.  A reference crash (it has a few:
-merging with an empty structure frame raises KeyError) makes the case skip itself -- there is nothing to be
+with zero cells; thresholds from -inf upwards; pseudocounts; background options.  The reference's own
+``rnascan.rnascan.main()`` (unmodified, with oracle/bio_shim standing in for Biopython and the reference's
+compiled ``_pwm.c``) was run on each of them by tests/golden/make_golden_fuzz.py; its stdout, exit code and
+argv are stored in tests/golden/fuzz.  Here the inputs are drawn again from the seed and
+``rnascan_b200.rnascan.main()`` runs on them with the device entry points swapped for the CPU oracle
+(tests/oracle_backend.py).  stdout must be byte-identical (averaged-profile runs under ``--reference-compat``,
+see INTEGRATION.md section 0), exit codes equal.  A seed the reference crashed on (it has a few: merging with an
+empty structure frame raises KeyError) has no stored output and skips itself -- there is nothing to be
 identical to.
 
 This pins the HOST logic -- record handling, background arithmetic, PFM preprocessing, frame assembly with all
 the pandas dtype artefacts, TSV text -- far beyond the fixed golden files; the kernels are pinned to the same
-oracle by the -m gpu tests.  Skipped when /root/reference is not mounted (the GPU box).
+oracle, and to the same stored outputs, by the -m gpu tests.
 """
 import contextlib
 import io
+import json
 import os
-import sys
 import warnings
 
 import numpy as np
 import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HAVE_REFERENCE = os.path.exists("/root/reference/rnascan/rnascan.py") and \
-    os.path.exists(os.path.join(REPO, "oracle", "_ref", "_pwm.so"))
-pytestmark = pytest.mark.skipif(not HAVE_REFERENCE, reason="needs the reference tree and oracle/_ref/_pwm.so")
+FUZZ = os.path.join(REPO, "tests", "golden", "fuzz")
 
 
 @pytest.fixture(scope="module")
 def reference():
-    sys.path.insert(0, os.path.join(REPO, "tests", "golden"))
-    import make_golden as mg          # sets up bio_shim, the compiled _pwm and the pandas compat wrapper
-    return mg
+    """{seed: {"argv", "exit", "mode"}} of the reference's runs; its stdout is FUZZ/<seed>.stdout."""
+    with open(os.path.join(FUZZ, "cases.json")) as fh:
+        return json.load(fh)
 
 
 def run_ours(argv):
@@ -179,13 +178,14 @@ def test_reference_and_rnascan_b200_print_the_same_bytes(seed, reference, tmp_pa
     rng = np.random.default_rng(9000 + seed)
     paths = draw_inputs(rng, str(tmp_path / "case"))
     mode, argv, compat = draw_argv(rng, paths)
-    try:
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            want, _, want_code = reference.run_cli(argv)
-    except Exception as exc:                       # the reference crashed on this input
-        pytest.skip("reference raised %s: %s" % (type(exc).__name__, exc))
+    case = reference.get(str(seed))
+    if case is None:
+        pytest.skip("the reference raised on this input")
+    placeholders = {v: "{%s}" % k for k, v in paths.items()}
+    assert [placeholders.get(a, a) for a in argv] + compat == case["argv"], "the seed no longer draws the stored case"
+    with open(os.path.join(FUZZ, "%d.stdout" % seed)) as fh:
+        want = fh.read()
     install(monkeypatch)
     got, got_code = run_ours(argv + compat)
-    assert got_code == want_code, (mode, argv)
+    assert got_code == case["exit"], (mode, argv)
     assert got == want, (mode, argv)

@@ -343,11 +343,12 @@ def test_structure_annotation_matches_the_reference_tool():
 
 
 def test_structure_annotation_fuzz_against_the_reference_binary(tmp_path):
+    """tests/golden/dotbracket_fuzz.txt.gz holds the output of the reference's own C++ program for the seeded
+    structures below; when the program is built (oracle/Makefile, `make ref`) it is also run on them here."""
+    import gzip
     import random
     from rnascan_b200 import structure
     binary = os.path.join(REPO, "oracle", "_ref", "parse_secondary_structure")
-    if not os.path.exists(binary):
-        pytest.skip("oracle/_ref/parse_secondary_structure not built")
     rnd = random.Random(5)
 
     def rand_struct(n):
@@ -368,12 +369,16 @@ def test_structure_annotation_fuzz_against_the_reference_binary(tmp_path):
     structs = [s for s in (rand_struct(rnd.randint(1, 300)) for _ in range(3000)) if "." in s]
     fi, fo = tmp_path / "in.txt", tmp_path / "out.txt"
     fi.write_text("\n".join(structs) + "\n")
-    subprocess.check_call([binary, str(fi), str(fo)])
-    assert fo.read_text().split("\n")[:-1] == structure.parse_many(structs)
+    with gzip.open(os.path.join(REPO, "tests", "golden", "dotbracket_fuzz.txt.gz"), "rt") as fh:
+        want = fh.read()
+    if os.path.exists(binary):
+        subprocess.check_call([binary, str(fi), str(fo)])
+        assert fo.read_text() == want
+    assert len(structs) == 2989 and want.split("\n")[:-1] == structure.parse_many(structs)
     # file interface of the tool
     out2 = tmp_path / "out2.txt"
     structure.parse_file(str(fi), str(out2))
-    assert out2.read_text() == fo.read_text()
+    assert out2.read_text() == want
 
 
 def test_structure_annotation_is_linear_time():
@@ -698,6 +703,31 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert out["cpu_baseline"]["kind"] in ("reference", "port") and out["cpu_baseline"]["cores"] >= 1
     assert out["e2e"]["h2d_bytes_per_step"] == 0 and out["e2e"]["value"] == out["value"]
     assert "workload" in out["config"]
+
+
+def test_bench_dump_outputs_keeps_float32_and_samples_large_outputs(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 stays float32, anything else is written as float64; per-hit arrays above
+    the cap are cut to one seeded, ascending sample (written as sample_index), the same on every run and for
+    numpy arrays and tensors alike -- so that the dumps of two builds can be compared."""
+    import torch
+    import bench
+    load = lambda d: {f[:-4]: np.load(os.path.join(d, f)) for f in os.listdir(d)}
+    bench.dump_outputs(str(tmp_path / "small"), {"position": np.arange(10), "seq_score": np.ones(10, np.float32)},
+                       {"counts": np.arange(8)})
+    got = load(tmp_path / "small")
+    assert sorted(got) == ["counts", "position", "seq_score"] and got["position"].tolist() == list(range(10))
+    assert got["seq_score"].dtype == np.float32 and got["position"].dtype == got["counts"].dtype == np.float64
+    monkeypatch.setattr(bench, "DUMP_ENTRY_BYTES", 12000)
+    pos, sc = np.arange(5000) * 3, np.arange(5000, dtype=np.float32)      # 5000 entries of 12 bytes
+    bench.dump_outputs(str(tmp_path / "a"), {"position": pos, "seq_score": sc}, {"counts": np.arange(8)})
+    bench.dump_outputs(str(tmp_path / "b"), {"position": torch.from_numpy(pos), "seq_score": torch.from_numpy(sc)},
+                       {"counts": torch.arange(8)})
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    idx = a["sample_index"]
+    assert idx.dtype == np.float64 and len(idx) == 12000 // (12 + 8) and (np.diff(idx) > 0).all()
+    assert np.array_equal(a["position"], idx * 3) and np.array_equal(a["seq_score"], idx.astype(np.float32))
+    assert a["position"].nbytes + a["seq_score"].nbytes + idx.nbytes <= 12000
+    assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) and a[k].dtype == b[k].dtype for k in a)
 
 
 def test_pfm_reader_without_pandas_equals_pandas_or_declines(tmp_path):
