@@ -391,7 +391,6 @@ class _Batch(object):
         self.piece_start = np.zeros(n, np.int64) if piece_start is None else np.asarray(piece_start, np.int64)
         self.own = None if own is None else np.asarray(own, np.int64)
         self.stream = device.SymbolStream.from_texts(texts, kind)
-        self._raw = None
 
     @classmethod
     def from_pieces(cls, ids, descriptions, text, codes, offsets, lengths, kind, pieces):
@@ -421,7 +420,6 @@ class _Batch(object):
         self.record, self.piece_start = rec, a
         self.own = np.where(o >= b, b, o) - a
         self.stream = device.SymbolStream(pcodes, poff, ln, kind=kind)
-        self._raw = ptext
         return self
 
     def overlap_counts(self):
@@ -449,14 +447,6 @@ class _Batch(object):
     def __len__(self):
         return len(self.texts)
 
-    def raw(self):
-        """The record texts joined by newlines as a uint8 array: byte i is the letter of
-        stream position i (used to cut hit fragments without a Python loop)."""
-        if self._raw is None:
-            joined = ("\n".join(self.texts) + "\n") if self.texts else ""
-            self._raw = np.frombuffer(joined.encode("latin-1", "replace"), dtype=np.uint8)
-        return self._raw
-
 
 class _LazyTexts(object):
     """List-like view of the records of a packed text buffer; strings are made on demand."""
@@ -475,6 +465,20 @@ class _LazyTexts(object):
 
     def __iter__(self):
         return (self[k] for k in range(len(self)))
+
+
+def _record_text(batches):
+    """(uint8 text, offsets) of the whole records of `batches` (under torchrun: of the whole input, which every
+    rank holds) laid out one after the other with one separator each: byte offsets[r] + i is letter i of
+    record r.  Hit fragments are cut from it without a Python loop."""
+    if len(batches) == 1 and isinstance(batches[0].full_texts, _LazyTexts):
+        return batches[0].full_texts.raw, batches[0].full_texts.offsets
+    texts = [t for b in batches for t in b.full_texts]
+    offsets = np.zeros(len(texts), np.int64)
+    if len(texts) > 1:
+        np.cumsum([len(t) + 1 for t in texts[:-1]], out=offsets[1:])
+    joined = ("\n".join(texts) + "\n") if texts else ""
+    return np.frombuffer(joined.encode("latin-1", "replace"), dtype=np.uint8), offsets
 
 
 def _read_fasta_bytes(fasta_file):
@@ -509,7 +513,6 @@ def _native_batch(fasta_file, alphabet):
     batch.own = None
     batch.stream = device.SymbolStream(codes, off if n_rec else None, ln if n_rec else None, kind=kind) \
         if n_rec else device.SymbolStream(np.zeros(0, np.uint8), np.zeros(0, np.int64), np.zeros(0, np.int64), kind=kind)
-    batch._raw = text
     return batch
 
 
@@ -830,153 +833,113 @@ def _scan_batch(batch, pm, kind, minscore):
             pos, scores = every if every is not None else device.scan_struct_onehot(batch.stream, table, minscore)
     STATS.add("scored_positions", int(np.maximum(batch.stream.lengths - table.shape[0] + 1, 0).sum()))
     keep, rec, start0 = batch.locate(pos)
-    return pos[keep], rec[keep], start0[keep], scores[keep]
+    return rec[keep], start0[keep], scores[keep]
 
 
-def _gather_parts(parts, n_records, ids, descs):
-    """Under torchrun: concatenate every rank's hit arrays on rank 0 in rank order (= record
-    order, shard.plan_shards); other ranks get None."""
+def _gather(parts):
+    """The hit arrays of a scan -- one (rec, start0, scores, ...) tuple per device batch -- concatenated column
+    by column.  Under torchrun every rank's columns are gathered on rank 0 and concatenated in rank order
+    (= record order, shard.plan_shards); the other ranks get None."""
     from . import shard
+    columns = [_concat(col) for col in zip(*parts)]
     if _world_size() == 1:
-        return parts
-    rec = np.concatenate([p[0] for p in parts]) if parts else np.zeros(0, np.int64)
-    start0 = np.concatenate([p[1] for p in parts]) if parts else np.zeros(0, np.int64)
-    scores = np.concatenate([p[2] for p in parts]) if parts else np.zeros(0)
-    frags = [f for p in parts for f in p[3]]
-    width = len(frags[0]) if frags else 1
-    # the fragments travel as one (hits, width) byte matrix, the rest as plain arrays: no pickled Python objects
-    frag_bytes = np.frombuffer("".join(frags).encode("latin-1"), np.uint8).reshape(len(frags), width) if frags \
-        else np.zeros((0, width), np.uint8)
-    gathered = shard.gather_arrays([rec, start0, scores, frag_bytes])
-    if gathered is None:
-        return None
-    out = []
-    for g_rec, g_start, g_scores, g_frag in gathered:
-        texts = [] if not len(g_frag) else \
-            np.ascontiguousarray(g_frag).view("S%d" % g_frag.shape[1]).ravel().astype("U%d" % g_frag.shape[1]).tolist()
-        out.append((g_rec, g_start, g_scores, texts, ids, descs))
-    return out
+        return columns
+    ranks = shard.gather_arrays(columns)
+    return None if ranks is None else [_concat(col) for col in zip(*ranks)]
 
 
-def _scan_fasta(fasta_file, pssm, alphabet, minscore, restrict=None):
-    """All records of a FASTA input in one (or a few) kernel launches; returns the assembled
-    frame and the number of records.  `restrict(batch_index, batch, pos)` may drop hits."""
-    motif_id, pm = _first_motif(pssm)
-    kind = _kind_of(alphabet)
-    if kind == "struct" and not pm._is_structure():
-        raise NotImplementedError("GPU scoring supports the nucleotide and BEHLMRT structure alphabets")
-    width = pm.length
-    if _world_size() == 1 and restrict is None:
-        hits = _scan_fasta_hits(fasta_file, pssm, alphabet, minscore)
-        return hits.frame(), hits.n_records
-    parts, n_records = [], 0
-    for b, batch in enumerate(_cached_batches(fasta_file, alphabet)):
-        pos, rec, start0, scores = _scan_batch(batch, pm, kind, minscore)
-        if restrict is not None:
-            keep = restrict(b, batch, pos)
-            pos, rec, start0, scores = pos[keep], rec[keep], start0[keep], scores[keep]
-        parts.append((rec + n_records, start0, scores, _fragments(batch.raw(), pos, width),
-                      batch.ids, batch.descriptions))
-        n_records += len(batch.ids)
-    if _world_size() > 1:
-        ids0 = parts[0][4] if parts else []
-        descs0 = parts[0][5] if parts else []
-        parts = _gather_parts(parts, n_records, ids0, descs0)
-        if parts is None:
-            return pd.DataFrame(), n_records          # not rank 0: nothing to assemble or print
-        parts = [parts[0]] + [(p[0], p[1], p[2], p[3], [], []) for p in parts[1:]]
-    if n_records == 0:
-        return pd.DataFrame(), 0
-    rec = np.concatenate([p[0] for p in parts])
-    start0 = np.concatenate([p[1] for p in parts])
-    scores = np.concatenate([p[2] for p in parts])
-    fragments = [f for p in parts for f in p[3]]
-    ids = [i for p in parts for i in p[4]]
-    descs = [d for p in parts for d in p[5]]
-    logodds = _round3_f32(scores) if kind == "rna" else _round3_f64(scores)
-    return _assemble_fasta_frame(n_records, rec, ids, descs, motif_id, start0, width, fragments,
-                                 logodds), n_records
+def _concat(arrays):
+    """np.concatenate keeping the dtype of the scores: the device-rounded thousandths (int32) of the
+    every-position structure scan turn into floats only next to the float scores of a batch or rank where that
+    form did not apply."""
+    if len(arrays) == 1:
+        return arrays[0]
+    if len({a.dtype for a in arrays}) > 1:
+        arrays = [np.array(_round3_f64(a), np.float64) if a.dtype == np.int32 else a for a in arrays]
+    return np.concatenate(arrays)
 
 
-NATIVE_WRITER_MIN_ROWS = 1           # from this many rows on main() formats hits.tab natively (no DataFrame)
+NATIVE_WRITER_MIN_ROWS = 1           # from this many rows on, a table with arrays is printed natively (no DataFrame)
+NATIVE_CHUNK_ROWS = 4_000_000        # rows formatted per call (bounds the text buffer to ~0.5 GB)
+_HEADER = ["Sequence_ID", "Description", "Motif_ID", "Start", "End", "Sequence", "LogOdds", "Match_ID"]
+_COMBINED_HEADER = ["Sequence_ID", "Description.Seq", "Motif_ID.Seq", "Start", "End", "Sequence.Seq", "LogOdds.Seq",
+                    "Description.Struct", "Motif_ID.Struct", "Sequence.Struct", "LogOdds.Struct",
+                    "LogOdds.SeqStruct", "Match_ID"]
 
 
-class _Hits(object):
-    """Hits of one FASTA input as plain arrays, one part per device batch (single process).
-    `frame()` gives the DataFrame the reference builds; `write_native()` the same text without
-    creating a Python object per row (rs_host_format_hits)."""
+class _HitTable(object):
+    """The rows of one hits.tab.  `frame()` builds the DataFrame the reference prints for them.  A table with
+    arrays can also be printed without one (rs_host_format_hits*): row r is the hit at 0-based `start0[r]` of
+    record `rec[r]` (`ids` / `descs` per record), its fragment is `width` letters of `text` from `text_pos[r]`
+    (no text: "."), its score `scores[r]`, printed as score_kind `kind` says.  Combined rows (`motif_b` set)
+    add the structure side: `text_b` (None: "."), `kind_b` / `scores_b` and per-record `sdescs` (None: empty).
+    A result only pandas can print (-t, the merge fallback, some directory shapes) has the frame only."""
 
-    def __init__(self, motif_id, width, kind):
-        self.motif_id, self.width, self.kind = motif_id, width, kind
-        self.ids, self.descs, self.parts = [], [], []        # parts: (batch, pos, rec_global, start0, scores)
+    def __init__(self, frame, rec=None, start0=None, ids=(), descs=(), motif=None, width=0, text=None,
+                 text_pos=None, kind=0, scores=None, motif_b=None, text_b=None, kind_b=0, scores_b=None,
+                 sdescs=None):
+        self.frame, self.rec, self.start0, self.ids, self.descs = frame, rec, start0, ids, descs
+        self.motif, self.width, self.text, self.text_pos = motif, width, text, text_pos
+        self.kind, self.scores = kind, scores
+        self.motif_b, self.text_b, self.kind_b, self.scores_b, self.sdescs = motif_b, text_b, kind_b, scores_b, sdescs
 
-    def add(self, batch, pos, rec, start0, scores):
-        self.parts.append((batch, pos, rec + len(self.ids), start0, scores))
-        self.ids.extend(batch.ids)
-        self.descs.extend(batch.descriptions)
+    def write(self, out):
+        """hits.tab on `out`: natively when the table has arrays, at least max(1, NATIVE_WRITER_MIN_ROWS) rows and
+        only values the native formatter covers; through pandas otherwise."""
+        if self.rec is None or len(self.rec) < max(1, NATIVE_WRITER_MIN_ROWS) or not self._write_native(out):
+            frame = self.frame()
+            _add_match_id(frame)
+            frame.to_csv(out, sep="\t", index=False)
 
-    @property
-    def n_records(self):
-        return len(self.ids)
-
-    def total(self):
-        return int(sum(len(p[1]) for p in self.parts))
-
-    def per_record(self):
-        rec = np.concatenate([p[2] for p in self.parts]) if self.parts else np.zeros(0, np.int64)
-        return np.bincount(rec, minlength=self.n_records) if self.n_records else np.zeros(0, np.int64)
-
-    def any_record_without_hits(self):
-        return self.n_records > 1 and bool((self.per_record() == 0).any())
-
-    def frame(self):
-        if self.n_records == 0:
-            return pd.DataFrame()
-        rec = np.concatenate([p[2] for p in self.parts])
-        start0 = np.concatenate([p[3] for p in self.parts])
-        scores = np.concatenate([p[4] for p in self.parts])
-        fragments = [f for p in self.parts for f in _fragments(p[0].raw(), p[1], self.width)]
-        logodds = _round3_f32(scores) if self.kind == "rna" else _round3_f64(scores)
-        return _assemble_fasta_frame(self.n_records, rec, self.ids, self.descs, self.motif_id, start0,
-                                     self.width, fragments, logodds)
-
-    def write_native(self, out):
-        """hits.tab of modes RNA / SS.  Returns False (nothing written) when a value falls outside
-        the formats the native writer covers; the caller then uses frame().to_csv()."""
+    def _write_native(self, out):
+        """False (nothing written) when the formatter declines the first chunk; a later chunk it declines raises."""
         blobs = _StringBlobs(self.ids, self.descs)
-        if self.kind == "rna":                     # float32 text unless a record has no hit (H8, a17)
-            kind = 1 if self.any_record_without_hits() else 0
-        elif all(np.asarray(p[4]).dtype == np.int32 for p in self.parts):
-            kind = 4                               # thousandths rounded on the device
-        else:
-            kind = 2
-        header = "\t".join(["Sequence_ID", "Description", "Motif_ID", "Start", "End", "Sequence", "LogOdds",
-                            "Match_ID"]) + "\n"
-        first, started = 1, False
-        for batch, pos, rec, start0, scores in self.parts:
-            if self.kind == "rna":
-                sc = _round3_f32(scores)
-            elif kind == 4:
-                sc = np.ascontiguousarray(scores, np.int32)
-            else:
-                sc = np.ascontiguousarray(_round3_f64(scores) if np.asarray(scores).dtype == np.int32 else scores,
-                                          np.float64)
-            for a in range(0, len(pos), NATIVE_CHUNK_ROWS):
-                b = min(len(pos), a + NATIVE_CHUNK_ROWS)
-                text = _native_rows(b - a, first, rec[a:b], blobs, None, self.motif_id, None, start0[a:b],
-                                    self.width, batch.raw(), None, pos[a:b], kind, sc[a:b], None, None)
-                if text is None:
-                    if started:
-                        raise ValueError("hit score outside the text formats of the native hits.tab writer")
-                    return False
-                if not started:
-                    _emit(out, header)
-                    started = True
-                _emit(out, text)
-                first += b - a
-        if not started:
-            _emit(out, header)
+        sblobs = None if self.sdescs is None else _StringBlobs(self.ids, self.sdescs)
+        scores = _writer_scores(self.kind, self.scores)
+        scores_b = None if self.motif_b is None else _writer_scores(self.kind_b, self.scores_b)
+        for a in range(0, len(self.rec), NATIVE_CHUNK_ROWS):
+            b = min(len(self.rec), a + NATIVE_CHUNK_ROWS)
+            text = _native_rows(b - a, 1 + a, self.rec[a:b], blobs, sblobs, self.motif, self.motif_b, self.start0[a:b],
+                                self.width, self.text, self.text_b, self.text_pos[a:b], self.kind, scores[a:b],
+                                self.kind_b, None if scores_b is None else scores_b[a:b])
+            if text is None:
+                if a:
+                    raise ValueError("hit score outside the text formats of the native hits.tab writer")
+                return False
+            if not a:
+                _emit(out, "\t".join(_HEADER if self.motif_b is None else _COMBINED_HEADER) + "\n")
+            _emit(out, text)
         return True
+
+
+def _writer_scores(kind, scores):
+    """`scores` in the dtype rs_host_format_hits* reads for score_kind `kind`: 0 / 1 float32 rounded to three
+    decimals, 4 int32 thousandths, 2 / 3 float64."""
+    kind &= 0xFF
+    if kind <= 1:
+        return _round3_f32(scores)
+    return np.ascontiguousarray(scores, np.int32 if kind == 4 else np.float64)
+
+
+def _fasta_table(motif_id, width, kind, batches, rec, start0, scores):
+    """The _HitTable of a single-modality FASTA scan (modes RNA / SS) from its hits: record index over all
+    `batches`, 0-based start, scores as the device returned them."""
+    ids = [i for b in batches for i in b.ids]
+    descs = [d for b in batches for d in b.descriptions]
+    text, offsets = _record_text(batches)
+    text_pos = offsets[rec] + start0
+
+    def frame():
+        if not ids:
+            return pd.DataFrame()
+        logodds = _round3_f32(scores) if kind == "rna" else _round3_f64(scores)
+        return _assemble_fasta_frame(len(ids), rec, ids, descs, motif_id, start0, width,
+                                     _fragments(text, text_pos, width), logodds)
+    if kind == "rna":                      # float32 text unless a record has no hit (H8, a17)
+        score_kind = 1 if (np.bincount(rec, minlength=len(ids)) == 0).any() else 0
+    else:                                  # 4: thousandths rounded on the device
+        score_kind = 4 if scores.dtype == np.int32 else 2
+    return _HitTable(frame, rec, start0, ids, descs, motif_id, width, text, text_pos, score_kind, scores)
 
 
 class _StringBlobs(object):
@@ -1033,9 +996,6 @@ def _native_rows(n_rows, match_first, rec, blobs, sblobs, motif_a, motif_b, star
         return out[:int(written[0])].tobytes().decode("utf-8", "replace")
 
 
-NATIVE_CHUNK_ROWS = 4_000_000        # rows formatted per call (bounds the text buffer to ~0.5 GB)
-
-
 def _emit(out, text):
     """Write to a text stream, through its binary buffer when it has one (sys.stdout)."""
     if hasattr(out, "buffer"):
@@ -1046,16 +1006,22 @@ def _emit(out, text):
 
 
 def _scan_fasta_hits(fasta_file, pssm, alphabet, minscore):
-    """Single-process scan of a FASTA input as a _Hits object."""
+    """All records of a FASTA input in one (or a few) kernel launches, as a _HitTable (None on ranks other than
+    0 under torchrun)."""
+    eprint("Scanning sequences ")
     motif_id, pm = _first_motif(pssm)
     kind = _kind_of(alphabet)
     if kind == "struct" and not pm._is_structure():
         raise NotImplementedError("GPU scoring supports the nucleotide and BEHLMRT structure alphabets")
-    hits = _Hits(motif_id, pm.length, kind)
-    for batch in _cached_batches(fasta_file, alphabet):
-        pos, rec, start0, scores = _scan_batch(batch, pm, kind, minscore)
-        hits.add(batch, pos, rec, start0, scores)
-    return hits
+    batches = _cached_batches(fasta_file, alphabet)
+    parts, n_records = [], 0
+    for batch in batches:
+        rec, start0, scores = _scan_batch(batch, pm, kind, minscore)
+        parts.append((rec + n_records, start0, scores))
+        n_records += len(batch.ids)
+    eprint("Processed %d sequences" % n_records)
+    hits = _gather(parts or [(np.zeros(0, np.int64),) * 3])
+    return None if hits is None else _fasta_table(motif_id, pm.length, kind, batches, *hits)
 
 
 def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, minscore):
@@ -1064,7 +1030,7 @@ def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, mi
     a provisional table the device derives from its own counts while the counts travel to the host, the
     exact log-odds are built there (Python's math.log, as Biopython does) and the finish pass decides every
     candidate with them (device.BackgroundOneHotScan; results identical to the serial order).
-    Returns (bg, pssm, _Hits), or None when this shape of run takes the serial path."""
+    Returns (bg, pssm, _HitTable), or None when this shape of run takes the serial path."""
     from . import device
     kind = _kind_of(alphabet)
     columns = device.RNA_COLUMNS if kind == "rna" else device.CHANNELS
@@ -1096,11 +1062,10 @@ def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, mi
     STATS.add("scored_positions", int(np.maximum(batch.stream.lengths - prob.shape[0] + 1, 0).sum()))
     motif_id, pm = _first_motif(state["pssm"])
     eprint("Scanning sequences ")
-    hits = _Hits(motif_id, pm.length, kind)
     keep, rec, start0 = batch.locate(pos)
-    hits.add(batch, pos[keep], rec[keep], start0[keep], scores[keep])
-    eprint("Processed %d sequences" % hits.n_records)
-    return state["bg"], state["pssm"], hits
+    table = _fasta_table(motif_id, pm.length, kind, batches, rec[keep], start0[keep], scores[keep])
+    eprint("Processed %d sequences" % len(table.ids))
+    return state["bg"], state["pssm"], table
 
 
 # one parsed + uploaded input is reused by compute_background and the scan that follows it
@@ -1249,16 +1214,19 @@ def _profile_dir_streams(directory, debug, seq_batches, write_pack):
     return out
 
 
-def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm=None, want_arrays=False,
-                      write_pack=False, seq_table_fn=None):
-    """All ``structure.<id>.txt`` profiles of a directory in one pass (rnascan.py:348-375).
+def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm=None, seq_hits=None,
+                      write_pack=False, precomputed=None):
+    """All ``structure.<id>.txt`` profiles of a directory in one pass (rnascan.py:348-375), as a _HitTable (None
+    on ranks other than 0 under torchrun).
     With `seq_batches`/`seq_pm` (combined mode) the sequence PSSM is evaluated on the same windows and only
-    those passing BOTH thresholds come back (`seq_table_fn(counts)`: the sequence table when its background
-    is computed from the data -- the counts are then taken on the device in the same pass).  The float64
-    rows stay on the host: the device filters a float32 shadow or the pack's 8-byte quantised rows and
-    re-scores the few windows near the threshold from the exact rows (device.scan_profile_host).  Under
-    torchrun every rank takes a contiguous range of files balanced by size; rank 0 assembles the frame."""
+    those passing BOTH thresholds come back: the rows of the combined hits.tab, whose sequence side is the
+    table `seq_hits` of the sequence scan.  The float64 rows stay on the host: the device filters a float32
+    shadow or the pack's 8-byte quantised rows and re-scores the few windows near the threshold from the exact
+    rows (device.scan_profile_host).  `precomputed`: the hits of this motif (pair) found by the batched scan of
+    a motif collection (_batched_profile_hits).  Under torchrun every rank takes a contiguous range of files
+    balanced by size and rank 0 gathers the hits."""
     from . import device, shard
+    eprint("Scanning averaged secondary structures ")
     motif_id, pm = _first_motif(pssm)
     tq = _structure_table(pm)
     width = tq.shape[0]
@@ -1266,10 +1234,7 @@ def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm
     files, all_names, hp, lengths, names, offsets, codes = _profile_dir_streams(directory, debug, seq_batches,
                                                                                 write_pack)
     n_files = len(all_names)
-    seq = None
-    if seq_batches is not None:
-        seq = seq_table_fn if seq_table_fn is not None else _table_for(seq_pm, "rna")
-    precomputed, _PRECOMPUTED[0] = _PRECOMPUTED[0], None
+    seq = None if seq_batches is None else _table_for(seq_pm, "rna")
     if precomputed is not None:           # this motif pair was scanned in the collection's batched pass
         pos, seq_scores, scores = precomputed
         STATS.add("scored_positions", int(np.maximum(lengths - width + 1, 0).sum()))
@@ -1289,50 +1254,57 @@ def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm
     else:
         rec = start0 = np.zeros(0, np.int64)
         scores = np.zeros(0, np.float64)
-        seq_scores = None
-    hit_names = [names[r] for r in rec.tolist()]
-    arrays = None
-    if want_arrays and size == 1 and seq is not None:
-        arrays = (list(hit_names), start0.copy(), np.zeros(0, np.float32) if seq_scores is None else seq_scores,
-                  np.asarray(scores, np.float64))
-    elif want_arrays and size == 1:       # structure only: what the native writer needs (_DirHits)
-        arrays = _DirHits(motif_id, width, list(names), np.asarray(rec, np.int64), np.asarray(start0, np.int64),
-                          np.asarray(scores, np.float64), _dir_frame_shape(all_names, hit_names))
-    if size > 1:
-        first = all_names.index(names[0]) if names else 0          # this rank's files are a contiguous range
-        gathered = shard.gather_arrays([rec + first, start0, np.asarray(scores, np.float64)])
-        if gathered is not None:
-            hit_names = [all_names[r] for g in gathered for r in g[0].tolist()]
-            start0 = np.concatenate([g[1] for g in gathered])
-            scores = np.concatenate([g[2] for g in gathered])
+        seq_scores = np.zeros(0, np.float32)
+    first = all_names.index(names[0]) if names else 0          # this rank's files are a contiguous range
+    hits = _gather([(rec + first, start0, np.asarray(scores, np.float64)) + (() if seq is None else (seq_scores,))])
     # Combined mode without a single joint hit: the reference's merge still needs the STRUCTURE frame's columns,
     # which exist iff some window passes the structure threshold on its own (else its merge raises KeyError, and
     # so does ours): one structure-only pass settles it -- only in this corner, on every rank when sharded.
     any_struct_hits = None
     if seq is not None:
-        need = len(hit_names) == 0 if rank == 0 else None
+        need = len(hits[0]) == 0 if rank == 0 else None
         if size > 1:
             need = shard.broadcast_object(need)
         if need:
             local = bool(len(codes)) and len(device.scan_profile_host(codes, hp, None, tq, minscore)[0]) > 0
             found = shard.gather_objects(local) if size > 1 else [local]
             any_struct_hits = bool(found and any(found))
-    if size > 1 and rank != 0:            # only rank 0 assembles and prints
-        return (_Deferred(lambda: pd.DataFrame()), n_files, None) if want_arrays else (pd.DataFrame(), n_files)
+    eprint("Processed %d sequences" % n_files)
+    if hits is None:                      # only rank 0 prints
+        return None
+    rec, start0, scores = hits[:3]
+    if seq is None:
+        frame = lambda: _averaged_dir_frame(all_names, rec, motif_id, start0, width, scores)
+        shape = _dir_frame_shape(np.bincount(rec, minlength=n_files))
+        if shape not in ("hit", "hit,empty"):       # first file without hits (another column order), or no hit
+            return _HitTable(frame)
+        # Start / End print as floats when some file has no hit; the scores unrounded
+        return _HitTable(frame, rec, start0, all_names, [""] * n_files, motif_id, width, None, start0,
+                         3 | (0x100 if shape == "hit,empty" else 0), scores)
     first_has_hits = None
-    if seq is not None and n_files > 1 and rank == 0 and len(lengths):
-        # combined mode: `hit_names` only knows the windows where BOTH scores pass, but the column order of the
+    if n_files > 1 and len(lengths):
+        # combined mode: `rec` only knows the windows where BOTH scores pass, but the column order of the
         # reference's structure frame -- and with it that of the merged output -- follows the first file's own
         # structure hits: one small structure-only scan of that file settles it
-        first = device.HostProfile(np.ascontiguousarray(hp.rows[:int(lengths[0])]))
-        first_has_hits = len(device.scan_profile_host(None, first, None, tq, minscore)[0]) > 0
-    build = lambda: _averaged_dir_frame(all_names, hit_names, motif_id, start0, width, scores, first_has_hits,
-                                        any_struct_hits)
-    if not want_arrays:
-        return build(), n_files
-    if arrays is not None and first_has_hits is False:
-        arrays = None                     # unusual column order: the DataFrame path prints it
-    return _Deferred(build), n_files, arrays      # the frame only if the native writer cannot print the result
+        head = device.HostProfile(np.ascontiguousarray(hp.rows[:int(lengths[0])]))
+        first_has_hits = len(device.scan_profile_host(None, head, None, tq, minscore)[0]) > 0
+
+    def frame():
+        return combine(seq_hits.frame(), _averaged_dir_frame(all_names, rec, motif_id, start0, width, scores,
+                                                             first_has_hits, any_struct_hits))
+    if first_has_hits is False:           # unusual column order: pandas prints it
+        return _HitTable(frame)
+    # the joint windows in the order of the inner join, whose left side is the sequence frame: sequence record,
+    # then Start
+    text, text_offsets = _record_text(seq_batches)
+    index = {rid: k for k, rid in enumerate(seq_hits.ids)}
+    seq_rec = np.array([index.get(nm, -1) for nm in all_names], np.int64)[rec]
+    keep = seq_rec >= 0
+    order = np.lexsort((start0[keep], seq_rec[keep]))
+    seq_rec, seq_start0 = seq_rec[keep][order], start0[keep][order]
+    return _HitTable(frame, seq_rec, seq_start0, seq_hits.ids, seq_hits.descs, seq_hits.motif, width, text,
+                     text_offsets[seq_rec] + seq_start0, seq_hits.kind, hits[3][keep][order], motif_id, None, 3,
+                     scores[keep][order])
 
 
 _DIR_PROTOTYPES = {}
@@ -1357,51 +1329,37 @@ def _dir_frame_prototype(shape):
     return proto
 
 
-def _dir_frame_shape(all_names, hit_names, first_has_hits=None, any_struct_hits=None):
+def _dir_frame_shape(hits_per_file, first_has_hits=None, any_struct_hits=None):
     """Which per-file frames the reference concatenates, as far as the result's columns and dtypes go: "hit" (every
     file has one), "hit,empty" / "empty,hit" (some file has none; the first file's frame decides the column order),
-    "empty" (no hit anywhere), "" (no file)."""
-    if not all_names:
+    "empty" (no hit anywhere), "" (no file).  `hits_per_file`: the number of hits of each file, in file order."""
+    if not len(hits_per_file):
         return ""
-    n = len(hit_names)
-    with_hits = set(hit_names)
-    any_empty = any(name not in with_hits for name in all_names)
-    if first_has_hits is True and all_names[0] not in with_hits:
-        any_empty = True                  # (combined mode) its structure hits exist, none of them joint
+    n = int(hits_per_file.sum())
+    any_empty = bool((hits_per_file == 0).any())
     if n == 0 and any_struct_hits and first_has_hits is None:
-        first_has_hits = len(all_names) == 1       # a single file: it is the one with the structure hits
+        first_has_hits = len(hits_per_file) == 1   # a single file: it is the one with the structure hits
     if n == 0 and not first_has_hits and not any_struct_hits:
         return "empty"
     if not any_empty:
         return "hit"
     if first_has_hits is None:
-        first_has_hits = all_names[0] in with_hits
+        first_has_hits = hits_per_file[0] > 0
     return "hit,empty" if first_has_hits else "empty,hit"
 
 
-class _Deferred(object):
-    """A value worked out when (and if) somebody asks for it."""
-
-    def __init__(self, fn):
-        self._fn, self._done, self._value = fn, False, None
-
-    def __call__(self):
-        if not self._done:
-            self._value, self._done, self._fn = self._fn(), True, None
-        return self._value
-
-
-def _averaged_dir_frame(all_names, hit_names, motif_id, start0, width, scores, first_has_hits=None,
-                        any_struct_hits=None):
+def _averaged_dir_frame(all_names, rec, motif_id, start0, width, scores, first_has_hits=None, any_struct_hits=None):
     """The frame the reference gets for a directory (rnascan.py:348-375, 408-413): one frame per file built
     by pd.DataFrame(list of Series) -- or, for a file without hits, pd.DataFrame([]) with only the two id
     columns -- then pd.concat and the last two columns moved to the front.  What pandas makes of that mix
     (column order follows the first file's frame; Start/End turn float when any file had no hit; only the id
     columns remain when no file had one) is learnt from one-row prototypes run through the same calls, then
-    applied to the whole result at once."""
-    n = len(hit_names)
-    proto = _dir_frame_prototype(_dir_frame_shape(all_names, hit_names, first_has_hits, any_struct_hits))
-    data = {"Sequence_ID": np.array(hit_names, dtype=object), "Description": np.array([""] * n, dtype=object),
+    applied to the whole result at once.  Hit i is in file `all_names[rec[i]]`."""
+    rec = np.asarray(rec, np.int64)
+    n = len(rec)
+    proto = _dir_frame_prototype(_dir_frame_shape(np.bincount(rec, minlength=len(all_names)), first_has_hits,
+                                                  any_struct_hits))
+    data = {"Sequence_ID": np.array(all_names, dtype=object)[rec], "Description": np.array([""] * n, dtype=object),
             "Motif_ID": np.array([motif_id] * n, dtype=object), "Start": np.asarray(start0, np.int64) + 1,
             "End": np.asarray(start0, np.int64) + width, "Sequence": np.array(["."] * n, dtype=object),
             "LogOdds": np.asarray(scores, dtype=np.float64)}
@@ -1415,22 +1373,23 @@ def _averaged_dir_frame(all_names, hit_names, motif_id, start0, width, scores, f
 def scan_main(fasta_file, pssm, alphabet, bg, args):
     """Scan one input -- a SeqRecord, a directory of averaged profiles or a FASTA file -- and
     return the hit frame with Sequence_ID and Description in front (rnascan.py:335-413)."""
-    count = 0
+    table = _scan_table(fasta_file, pssm, alphabet, args)
+    return pd.DataFrame() if table is None else table.frame()
+
+
+def _scan_table(fasta_file, pssm, alphabet, args, precomputed=None):
+    """scan_main's scan as a _HitTable (None on ranks other than 0 under torchrun)."""
     if _seq.is_seqrecord(fasta_file):
         final = scan_all(fasta_file, pssm, alphabet, args.minscore)
         _add_sequence_id(final, "testseq", "")
-        count += 1
         cols = final.columns.tolist()
         final = final[cols[-2:] + cols[:-2]]
-    elif os.path.isdir(fasta_file):
-        eprint("Scanning averaged secondary structures ")
-        final, count = _scan_profile_dir(fasta_file, pssm, args.minscore, args.debug,
-                                         write_pack=getattr(args, "pack", False))
-    else:
-        eprint("Scanning sequences ")
-        final, count = _scan_fasta(fasta_file, pssm, alphabet, args.minscore)
-    eprint("Processed %d sequences" % count)
-    return final
+        eprint("Processed 1 sequences")
+        return _HitTable(lambda: final)
+    if os.path.isdir(fasta_file):
+        return _scan_profile_dir(fasta_file, pssm, args.minscore, args.debug, write_pack=getattr(args, "pack", False),
+                                 precomputed=precomputed)
+    return _scan_fasta_hits(fasta_file, pssm, alphabet, args.minscore)
 
 
 def combine(seq_results, struct_results):
@@ -1522,124 +1481,36 @@ def load_background(bg_file, uniform, *args):
 ###############################################################################
 # Main
 ###############################################################################
-class _DirHits(object):
-    """Hits of a structure-only scan of a profile directory as arrays (single process), for the native writer:
-    the text pandas prints for the reference's concatenated per-file frames when the first file has a hit --
-    Start / End as integers when every file has one ("hit"), as floats when some file has none ("hit,empty").
-    Other shapes (first file without hits: another column order; no hit at all) are left to the DataFrame path."""
-
-    def __init__(self, motif_id, width, names, rec, start0, scores, shape):
-        self.motif_id, self.width, self.names = motif_id, width, names
-        self.rec, self.start0, self.scores, self.shape = rec, start0, scores, shape
-
-    def write_native(self, out):
-        if self.shape not in ("hit", "hit,empty") or len(self.rec) < max(1, NATIVE_WRITER_MIN_ROWS):
-            return False
-        blobs = _StringBlobs(self.names, [""] * len(self.names))
-        kind = 3 | (0x100 if self.shape == "hit,empty" else 0)
-        header = "\t".join(["Sequence_ID", "Description", "Motif_ID", "Start", "End", "Sequence", "LogOdds",
-                            "Match_ID"]) + "\n"
-        sc = np.ascontiguousarray(self.scores, np.float64)
-        pieces = []
-        for a in range(0, len(self.rec), NATIVE_CHUNK_ROWS):
-            b = min(len(self.rec), a + NATIVE_CHUNK_ROWS)
-            text = _native_rows(b - a, 1 + a, self.rec[a:b], blobs, None, self.motif_id, None, self.start0[a:b],
-                                self.width, None, None, self.start0[a:b], kind, sc[a:b], None, None)
-            if text is None:
-                if pieces:
-                    raise ValueError("hit score outside the text formats of the native hits.tab writer")
-                return False
-            if not pieces:
-                _emit(out, header)
-            _emit(out, text)
-            pieces.append(b - a)
-        return True
-
-
-class _Joint(object):
-    """Windows where BOTH scores pass, as arrays in the order of the sequence input (= the order of
-    the reference's inner join, whose left side is the sequence frame)."""
-
-    def __init__(self):
-        self.rec = self.start0 = self.text_pos = np.zeros(0, np.int64)
-        self.seq_scores = np.zeros(0, np.float32)
-        self.struct_scores = np.zeros(0, np.float64)
-        self.struct_kind = 2               # 2 one-hot (rounded when printed), 3 averaged (unrounded)
-        self.seq_raw = self.struct_raw = None
-        self.struct_descs = None           # per seq record, or None: empty Description.Struct
-        self.struct_frame = None           # callable -> the restricted structure frame (DataFrame path)
-
-    def write_native(self, out, seq_hits, motif_struct, width):
-        blobs = _StringBlobs(seq_hits.ids, seq_hits.descs)
-        sblobs = None if self.struct_descs is None else _StringBlobs(seq_hits.ids, self.struct_descs)
-        seq_kind = 1 if seq_hits.any_record_without_hits() else 0
-        header = "\t".join(["Sequence_ID", "Description.Seq", "Motif_ID.Seq", "Start", "End", "Sequence.Seq",
-                            "LogOdds.Seq", "Description.Struct", "Motif_ID.Struct", "Sequence.Struct",
-                            "LogOdds.Struct", "LogOdds.SeqStruct", "Match_ID"]) + "\n"
-        seq_sc = _round3_f32(self.seq_scores)
-        str_sc = np.ascontiguousarray(self.struct_scores, np.float64)
-        started = False
-        for a in range(0, max(len(self.rec), 1), NATIVE_CHUNK_ROWS):
-            b = min(len(self.rec), a + NATIVE_CHUNK_ROWS)
-            text = _native_rows(b - a, 1 + a, self.rec[a:b], blobs, sblobs, seq_hits.motif_id, motif_struct,
-                                self.start0[a:b], width, self.seq_raw, self.struct_raw, self.text_pos[a:b],
-                                seq_kind, seq_sc[a:b], self.struct_kind, str_sc[a:b])
-            if text is None:
-                if started:
-                    raise ValueError("hit score outside the text formats of the native hits.tab writer")
-                return False
-            if not started:
-                _emit(out, header)
-                started = True
-            _emit(out, text)
-        return True
-
-
-def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, args):
-    """Structure side of the combined mode, restricted ON THE DEVICE to windows whose sequence
-    score also passes (the inner join of rnascan.py:422 keeps nothing else): one fused launch
-    instead of a second full scan + merge.  Returns a _Joint, or None when the restriction cannot
-    be applied (different motif widths, duplicate ids, inputs that do not line up) -- the caller
-    then scans the structure input on its own and merges as the reference does."""
+def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, precomputed=None):
+    """The table of the combined mode (rnascan.py:416-434) on top of `seq_hits`, the sequence scan's table; None
+    on ranks other than 0 under torchrun.  The structure side is scanned ON THE DEVICE only where the sequence
+    score also passes (the inner join keeps nothing else): one fused launch instead of a second full scan +
+    merge.  Where the two inputs cannot be scanned together (-t, different motif widths, duplicate ids, inputs
+    that do not line up) the structure input is scanned on its own and merged as the reference does."""
     from . import device
     _, seq_pm = _first_motif(seq_pssm)
     motif_id, pm = _first_motif(struct_pssm)
-    if seq_pm.length != pm.length:
-        return None
-    rna = IUPAC.IUPACUnambiguousRNA()
-    seq_batches = _cached_batches(seq_file, rna)
+    width = pm.length
+    structure = ContextualSecondaryStructure()
+
+    def merged():
+        struct_hits = _scan_table(struct_file, struct_pssm, structure, args)
+        return None if struct_hits is None else _HitTable(lambda: combine(seq_hits.frame(), struct_hits.frame()))
+    if _seq.is_seqrecord(struct_file) or seq_pm.length != width:
+        return merged()
+    seq_batches = _cached_batches(seq_file, IUPAC.IUPACUnambiguousRNA())
     ids = [i for b in seq_batches for i in b.ids]
     if len(set(ids)) != len(ids):
-        return None                       # duplicate ids join across records: keep the plain path
-    width = pm.length
-    joint = _Joint()
+        return merged()                   # duplicate ids join across records: keep the plain path
     if os.path.isdir(struct_file):
-        eprint("Scanning averaged secondary structures ")
-        frame, count, arrays = _scan_profile_dir(struct_file, struct_pssm, args.minscore, args.debug,
-                                                 seq_batches=seq_batches, seq_pm=seq_pm, want_arrays=True,
-                                                 write_pack=getattr(args, "pack", False))
-        eprint("Processed %d sequences" % count)
-        joint.struct_frame = frame        # deferred: built only when the DataFrame path prints
-        if arrays is None or len(seq_batches) != 1 or _world_size() > 1:
-            joint.rec = None              # frames only
-            return joint
-        names, start0, seq_sc, str_sc = arrays
-        index = {rid: k for k, rid in enumerate(seq_batches[0].ids)}
-        rec = np.array([index.get(nm, -1) for nm in names], dtype=np.int64)
-        keep = rec >= 0
-        order = np.lexsort((start0[keep], rec[keep]))            # sequence-record order, then Start
-        joint.rec, joint.start0 = rec[keep][order], start0[keep][order]
-        joint.seq_scores, joint.struct_scores = seq_sc[keep][order], str_sc[keep][order]
-        joint.struct_kind = 3
-        joint.seq_raw = seq_batches[0].raw()
-        joint.text_pos = seq_batches[0].stream.offsets[joint.rec] + joint.start0
-        return joint
-    alphabet = ContextualSecondaryStructure()
-    struct_batches = _cached_batches(struct_file, alphabet)
-    if len(struct_batches) != len(seq_batches) or any(
-            a.ids != b.ids or not np.array_equal(a.stream.lengths, b.stream.lengths)
-            for a, b in zip(seq_batches, struct_batches)):
-        return None
+        return _scan_profile_dir(struct_file, struct_pssm, args.minscore, args.debug, seq_batches, seq_pm, seq_hits,
+                                 getattr(args, "pack", False), precomputed)
+    struct_batches = _cached_batches(struct_file, structure)
+    seq_text, offsets = _record_text(seq_batches)
+    struct_text, struct_offsets = _record_text(struct_batches)
+    if ([i for b in struct_batches for i in b.ids] != ids or len(struct_text) != len(seq_text)
+            or not np.array_equal(struct_offsets, offsets)):
+        return merged()                   # records of different lengths: windows do not line up
     eprint("Scanning sequences ")
     ts, tq = _table_for(seq_pm, "rna"), _table_for(pm, "struct")
     parts, n_records = [], 0
@@ -1648,43 +1519,25 @@ def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, args):
             pos, seq_sc, scores = device.scan_pair_onehot(sb.stream, qb.stream, ts, tq, args.minscore)
         STATS.add("scored_positions", int(np.maximum(qb.stream.lengths - width + 1, 0).sum()))
         keep, rec, start0 = qb.locate(pos)
-        pos = pos[keep]
-        parts.append((rec[keep] + n_records, start0[keep], scores[keep], _fragments(qb.raw(), pos, width)
-                      if (_world_size() > 1 or len(seq_batches) > 1) else None, qb.ids, qb.descriptions,
-                      pos, seq_sc[keep]))
+        parts.append((rec[keep] + n_records, start0[keep], seq_sc[keep], scores[keep]))
         n_records += len(qb.ids)
     eprint("Processed %d sequences" % n_records)
-    single = _world_size() == 1 and len(seq_batches) == 1
+    hits = _gather(parts or [(np.zeros(0, np.int64),) * 4])
+    if hits is None:
+        return None
+    rec, start0, seq_scores, scores = hits
+    text_pos = offsets[rec] + start0
+    struct_descs = [d for b in struct_batches for d in b.descriptions]
 
-    def struct_frame():
-        ps = parts
-        if _world_size() > 1:
-            ps = _gather_parts([p[:6] for p in parts], n_records, parts[0][4] if parts else [],
-                               parts[0][5] if parts else [])
-            if ps is None:
-                return pd.DataFrame()
-            ps = [ps[0]] + [(p[0], p[1], p[2], p[3], [], []) for p in ps[1:]]
-        if n_records == 0:
-            return pd.DataFrame()
-        frags = [f for k, p in enumerate(ps)
-                 for f in (p[3] if p[3] is not None else _fragments(struct_batches[k].raw(), parts[k][6], width))]
-        return _assemble_fasta_frame(n_records, np.concatenate([p[0] for p in ps]),
-                                     [i for p in ps for i in p[4]], [d for p in ps for d in p[5]], motif_id,
-                                     np.concatenate([p[1] for p in ps]), width, frags,
-                                     _round3_f64(np.concatenate([p[2] for p in ps])))
-    joint.struct_frame = struct_frame
-    if not single:
-        joint.rec = None
-        return joint
-    p = parts[0]
-    joint.rec, joint.start0, joint.struct_scores, joint.seq_scores = p[0], p[1], p[2], p[7]
-    joint.text_pos = p[6]
-    joint.seq_raw, joint.struct_raw = seq_batches[0].raw(), struct_batches[0].raw()
-    joint.struct_descs = struct_batches[0].descriptions
-    return joint
+    def frame():                          # the structure frame of the joint windows: the join keeps the same rows
+        struct = pd.DataFrame() if not ids else _assemble_fasta_frame(
+            len(ids), rec, ids, struct_descs, motif_id, start0, width, _fragments(struct_text, text_pos, width),
+            _round3_f64(scores))
+        return combine(seq_hits.frame(), struct)
+    return _HitTable(frame, rec, start0, seq_hits.ids, seq_hits.descs, seq_hits.motif, width, seq_text, text_pos,
+                     seq_hits.kind, seq_scores, motif_id, struct_text, 2, scores, struct_descs)
 
 
-_PRECOMPUTED = [None]                # hits of the current motif pair found by the batched scan (_run_multi)
 _PROFILE_DIR_CACHE = {}              # directory -> _profile_dir_streams result while a motif collection is scanned
 _PROFILE_DIR_CACHE_ON = [False]
 
@@ -1794,7 +1647,7 @@ def scan_many(struct_dir, struct_pssms, minscore, seq_file=None, seq_pssms=None,
 
     struct_pssms (and seq_pssms, for the combined mode) are lists of ``{motif_id: PSSM}`` as load_motif
     returns them.  Returns one DataFrame per motif (pair): what scan_main(struct_dir, ...) returns for that
-    structure motif alone -- restricted, with seq_pssms, to the windows whose sequence score passes too, with
+    structure motif alone -- limited, with seq_pssms, to the windows whose sequence score passes too, with
     an extra ``LogOdds.Seq`` column."""
     from . import device
     if seq_pssms is not None and len(seq_pssms) != len(struct_pssms):
@@ -1814,8 +1667,7 @@ def scan_many(struct_dir, struct_pssms, minscore, seq_file=None, seq_pssms=None,
         a, b = int(bases[k]), int(bases[k + 1])
         rec = np.searchsorted(offsets, pos[a:b], side="right") - 1
         start0 = pos[a:b] - offsets[rec]
-        frame = _averaged_dir_frame(all_names, [names[r] for r in rec.tolist()], motif_id, start0, tqs[k].shape[0],
-                                    st[a:b])
+        frame = _averaged_dir_frame(all_names, rec, motif_id, start0, tqs[k].shape[0], st[a:b])
         if sq is not None and len(frame.columns) > 2:
             frame["LogOdds.Seq"] = _round3_f32(sq[a:b])
         frames.append(frame)
@@ -1903,118 +1755,66 @@ def _run(args, seq_type, rank, precomputed=None):
     """One reference run (rnascan.py:490-567): backgrounds, motifs, scans, hits.tab on STDOUT.
     `precomputed`: hits of this motif pair on the profile directory, already found by the batched scan."""
     bg = None
-    _PRECOMPUTED[0] = precomputed
     seq_file = struct_file = None
-    seq_pssm = None
-    seq_hits = struct_hits = joint = None          # array-level results (single process, FASTA inputs)
-    dir_hits = dir_frame = None                    # structure-only scan of a profile directory
-    seq_results = struct_results = None
-    arrays_ok = _world_size() == 1 and not args.testseq
+    seq_pssm = seq_hits = table = None
+    fusable = _world_size() == 1 and not args.testseq and not args.bgonly and not args.uniform_background
 
     if args.testseq:
         testseq_stack = args.testseq.split(",")[::-1]
 
     if seq_type in ["RNA", "RNASS"]:
         rna = IUPAC.IUPACUnambiguousRNA()
+        fused = None
         if args.testseq:
             seq_file = SeqRecord(Seq(testseq_stack.pop()))
         else:
             seq_file = args.fastafiles[0]
-            if (arrays_ok and not args.bgonly and not args.bg_seq and not args.uniform_background
-                    and not os.path.isdir(seq_file)):
+            if fusable and not args.bg_seq and not os.path.isdir(seq_file):
                 fused = _scan_fasta_hits_computed_bg(seq_file, args.pfm_seq, args.pseudocount, rna, args.minscore)
-                if fused is not None:
-                    bg, seq_pssm, seq_hits = fused
-            if seq_hits is None:
+            if fused is not None:
+                bg, seq_pssm, seq_hits = fused
+            else:
                 bg = load_background(args.bg_seq, args.uniform_background, seq_file, rna, not args.bgonly)
         if args.bgonly:
             if rank == 0:
                 print(dict(bg))
             sys.exit()
-        if seq_hits is None:              # else: background, motif and scan were done in one overlapped pass
+        if fused is None:                 # else: background, motif and scan were done in one overlapped pass
             seq_pssm = load_motif(args.pfm_seq, args.pseudocount, rna, bg)
-            if arrays_ok and not os.path.isdir(seq_file):
-                eprint("Scanning sequences ")
-                seq_hits = _scan_fasta_hits(seq_file, seq_pssm, rna, args.minscore)
-                eprint("Processed %d sequences" % seq_hits.n_records)
-            else:
-                seq_results = scan_main(seq_file, seq_pssm, rna, bg, args)
+            seq_hits = _scan_table(seq_file, seq_pssm, rna, args)
+        table = seq_hits
 
     if seq_type in ["SS", "RNASS"]:
         structure = ContextualSecondaryStructure()
+        fused = None
         if args.testseq:
             struct_file = SeqRecord(Seq(testseq_stack.pop()))
         elif seq_type == "SS":
             struct_file = args.fastafiles[0]
         else:
             struct_file = args.fastafiles[1]
-        if (seq_type == "SS" and arrays_ok and not args.bgonly and not args.bg_struct
-                and not args.uniform_background and not os.path.isdir(struct_file)):
+        if seq_type == "SS" and fusable and not args.bg_struct and not os.path.isdir(struct_file):
             fused = _scan_fasta_hits_computed_bg(struct_file, args.pfm_struct, args.pseudocount, structure,
                                                  args.minscore)
-            if fused is not None:
-                bg, struct_pssm, struct_hits = fused
-        if not args.testseq and struct_hits is None:
+        if fused is not None:
+            bg, struct_pssm, table = fused
+        elif not args.testseq:
             bg = load_background(args.bg_struct, args.uniform_background, struct_file, structure,
                                  not args.bgonly)
         if args.bgonly:
             if rank == 0:
                 print(dict(bg))
             sys.exit()
-        if struct_hits is None:
+        if fused is None:
             struct_pssm = load_motif(args.pfm_struct, args.pseudocount, structure, bg)
-        if seq_type == "RNASS" and not args.testseq:
-            joint = _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, args)
-        if joint is None and struct_hits is None:
-            if seq_type == "SS" and arrays_ok and not os.path.isdir(struct_file):
-                eprint("Scanning sequences ")
-                struct_hits = _scan_fasta_hits(struct_file, struct_pssm, structure, args.minscore)
-                eprint("Processed %d sequences" % struct_hits.n_records)
-            elif seq_type == "SS" and arrays_ok and os.path.isdir(struct_file):
-                # scan_main's directory branch (same messages), keeping the hit arrays for the native writer; the
-                # DataFrame is only built if that writer cannot print the result
-                eprint("Scanning averaged secondary structures ")
-                dir_frame, count, dir_hits = _scan_profile_dir(struct_file, struct_pssm, args.minscore, args.debug,
-                                                               want_arrays=True,
-                                                               write_pack=getattr(args, "pack", False))
-                eprint("Processed %d sequences" % count)
+            if seq_type == "RNASS":
+                table = _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, precomputed)
             else:
-                struct_results = scan_main(struct_file, struct_pssm, structure, bg, args)
+                table = _scan_table(struct_file, struct_pssm, structure, args, precomputed)
 
     t_out = time.perf_counter()
-    _PRECOMPUTED[0] = None
     if rank == 0:
-        written = False
-        if seq_type == "RNASS":
-            if (joint is not None and joint.rec is not None and seq_hits is not None
-                    and len(joint.rec) >= NATIVE_WRITER_MIN_ROWS):
-                written = joint.write_native(sys.stdout, seq_hits, _first_motif(struct_pssm)[0],
-                                             _first_motif(struct_pssm)[1].length)
-        else:
-            hits = seq_hits if seq_type == "RNA" else struct_hits
-            if hits is not None and hits.n_records > 0 and hits.total() >= NATIVE_WRITER_MIN_ROWS:
-                written = hits.write_native(sys.stdout)
-            elif seq_type == "SS" and dir_hits is not None:
-                written = dir_hits.write_native(sys.stdout)
-        if not written:
-            if seq_type == "SS" and struct_results is None and struct_hits is None and dir_frame is not None:
-                struct_results = dir_frame()
-            if seq_results is None and seq_hits is not None:
-                seq_results = seq_hits.frame()
-            if struct_results is None and struct_hits is not None:
-                struct_results = struct_hits.frame()
-            if struct_results is None and joint is not None:
-                struct_results = joint.struct_frame()
-            if seq_type == "RNASS":
-                final = combine(seq_results, struct_results)
-            elif seq_type == "RNA":
-                final = seq_results
-            else:
-                final = struct_results
-            _add_match_id(final)
-            final.to_csv(sys.stdout, sep="\t", index=False)
-    elif joint is not None and joint.struct_frame is not None:
-        joint.struct_frame()              # other ranks take part in the gather
+        table.write(sys.stdout)
     STATS.phases["output_s"] += time.perf_counter() - t_out
 
 
