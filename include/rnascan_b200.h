@@ -32,6 +32,10 @@
  *    RNA   : A=0 C=1 G=2 U/T=3 (either case), anything else 0x0C (window -> NaN)
  *    struct: B=0 E=1 H=2 L=3 M=4 R=5 T=6 ; lower case = index|8 (scored, not counted:
  *            rnascan.py:196-197 + :450-453 count case-sensitively) ; anything else 0x0F
+ *    alpha : any other alphabet of 1..31 distinct ASCII letters, none of them lower case a-z
+ *            (rs_host_encode_alpha): bits 0-4 index of the UPPER-CASED byte in the caller's
+ *            letters, bit 5 set for a lower-case byte (scored, not counted), anything else
+ *            0x1F.  0xFF & 31 = 31 >= A, so a separator invalidates a window without a test.
  *    A window that contains a separator is not a window of any record; hit scans never
  *    report it, dense outputs hold NaN there.
  *  Device arrays read by the scan kernels must be allocated with rs_padded_count(n)
@@ -57,6 +61,8 @@ extern "C" {
 #define RS_SEP        0xFF
 #define RS_RNA_OTHER  0x0C
 #define RS_SS_OTHER   0x0F
+#define RS_ALPHA_OTHER 0x1F  /* alphabet layout: byte that is no letter of the alphabet      */
+#define RS_ALPHA_LOWER 0x20  /* alphabet layout: lower-case letter (scored, not counted)     */
 #define RS_MAX_W      64     /* widest motif the scan kernels accept                    */
 
 #define RS_F32 0
@@ -118,6 +124,11 @@ int rs_host_parse_doubles(const char *text, int64_t n_bytes, double *out, int64_
  *      switch of _pwm.c:41-63 and the dict lookup of matrix.py:36-41) ---------------- */
 int rs_host_encode_rna(const uint8_t *text, int64_t n, uint8_t *codes);
 int rs_host_encode_struct(const uint8_t *text, int64_t n, uint8_t *codes);
+/* The alphabet layout for `letters` (n_letters of them, 1..31; RS_ERR_INVALID with a message when a
+ * letter is repeated, lower case a-z or not ASCII).  Replaces str.upper() + the dict lookup of
+ * matrix.py:36-41 for alphabets other than GAUC and BEHLMRT.                                   */
+int rs_host_encode_alpha(const uint8_t *text, int64_t n, const uint8_t *letters, int n_letters,
+                         uint8_t *codes);
 
 /* log2(p / b) tables in the arithmetic of Python's math.log(p / b, 2) as Biopython's log_odds
  * uses it (called at rnascan.py:248): prob, out [W][A] row-major, bg [A] normalised.        */
@@ -164,6 +175,9 @@ int rs_hist(const uint8_t *d_codes, int64_t n, uint64_t *d_counts8, void *stream
 /* Same for NUCLEOTIDE streams only (codes 0-3, RS_RNA_OTHER, RS_SEP as rs_host_encode_rna
  * writes them): two index bit-planes instead of three, half the arithmetic; bins 4..7 stay 0.  */
 int rs_hist_rna(const uint8_t *d_codes, int64_t n, uint64_t *d_counts8, void *stream);
+/* Same for ALPHABET-layout streams (rs_host_encode_alpha): d_counts32[k] += symbols with index k and
+ * bit 5 clear (k = 0..31; bin 31 counts the non-letters 0x1F, bins >= A stay 0 otherwise).      */
+int rs_hist_alpha(const uint8_t *d_codes, int64_t n, uint64_t *d_counts32, void *stream);
 
 /* ---- dense scores: the calculate() semantics, every window, NaN in band ------------
  * seq    : _pwm.c:34-68   out[i] = (float)(sum_j table[j][code]) double accumulation
@@ -188,6 +202,11 @@ int rs_scores_dense_struct_milli(const uint8_t *d_codes, int64_t n, const double
 int rs_scores_dense_profile(const void *d_profile, int profile_dtype, int64_t n_rows,
                             const uint8_t *d_codes /* may be NULL: no separators */,
                             const double *table_Wx7, int W, double *d_out, void *stream);
+/* alpha  : matrix.py:25-43 for any alphabet of A = 1..31 letters (rs_host_encode_alpha codes),
+ *          table [W][A] in the caller's letter order; out[i] = sum_j table[j][code] in double.
+ *          A <= 7 runs the structure kernels, 8..31 kernels with a 32-column table row.   */
+int rs_scores_dense_alpha(const uint8_t *d_codes, int64_t n, const double *table_WxA, int W, int A,
+                          double *d_out, void *stream);
 
 /* ---- profile statistics, once per uploaded profile ---------------------------------
  * d_stats[0] = max over rows of sum_c |p[r][c]| ; d_stats[1] = number of non-finite
@@ -220,6 +239,12 @@ int rs_scan_struct_onehot(const uint8_t *d_codes, int64_t n, const double *table
                           double threshold, int64_t hit_capacity, int64_t *d_hit_pos,
                           double *d_hit_score, uint64_t *d_counters2, void *d_work,
                           int64_t work_bytes, void *stream);
+/* rs_scan_alpha         : rs_scan_struct_onehot for an alphabet-layout stream of A = 1..31 letters,
+ *                         table [W][A] (as rs_scores_dense_alpha; replaces search() over
+ *                         matrix.py:25-43, rnascan.py:263, for alphabets other than BEHLMRT).    */
+int rs_scan_alpha(const uint8_t *d_codes, int64_t n, const double *table_WxA, int W, int A,
+                  double threshold, int64_t hit_capacity, int64_t *d_hit_pos, double *d_hit_score,
+                  uint64_t *d_counters2, void *d_work, int64_t work_bytes, void *stream);
 int rs_scan_pair_onehot(const uint8_t *d_seq_codes, const uint8_t *d_struct_codes, int64_t n,
                         const double *seq_table_Wx4, const double *struct_table_Wx7, int W,
                         double threshold, int64_t hit_capacity, int64_t *d_hit_pos,

@@ -55,15 +55,18 @@ class ExtendedPositionSpecificScoringMatrix(dict):
         return sorted(self.alphabet.letters) == sorted(device.CHANNELS)
 
     def _py_calculate(self, sequence, m, n):
-        """Generic-alphabet scores as a list of Python floats (matrix.py:25-43); runs on
-        the GPU for the structure-context alphabet."""
+        """Generic-alphabet scores as a list of Python floats (matrix.py:25-43), on the GPU:
+        the structure-context kernels for BEHLMRT, the alphabet kernels for any other
+        alphabet device.AlphaKind accepts (NotImplementedError otherwise)."""
         if n - m + 1 <= 0:
             return []
-        if not self._is_structure():
-            raise NotImplementedError(
-                "GPU scoring supports the nucleotide and BEHLMRT structure alphabets")
-        stream = device.SymbolStream.from_texts([sequence], "struct")
-        out = device.dense_struct(stream, self.table(device.CHANNELS)).cpu().numpy()
+        if self._is_structure():
+            stream = device.SymbolStream.from_texts([sequence], "struct")
+            out = device.dense_struct(stream, self.table(device.CHANNELS)).cpu().numpy()
+        else:
+            kind = device.AlphaKind(self.alphabet.letters)
+            stream = device.SymbolStream.from_texts([sequence], kind)
+            out = device.dense_alpha(stream, self.table(kind.letters)).cpu().numpy()
         return [float(v) for v in out[:n - m + 1]]
 
     def _calculate(self, sequence, m, n):
@@ -99,10 +102,12 @@ class ExtendedPositionSpecificScoringMatrix(dict):
             for p, s in zip(pos.tolist(), score):
                 yield (p, s)                       # s is numpy.float32, as in the reference
         else:
-            if not self._is_structure():
-                raise NotImplementedError(
-                    "GPU scoring supports the nucleotide and BEHLMRT structure alphabets")
-            stream = device.SymbolStream.from_texts([text], "struct")
-            pos, score = device.scan_struct_onehot(stream, self.table(device.CHANNELS), threshold)
+            if self._is_structure():
+                stream = device.SymbolStream.from_texts([text], "struct")
+                pos, score = device.scan_struct_onehot(stream, self.table(device.CHANNELS), threshold)
+            else:
+                kind = device.AlphaKind(self.alphabet.letters)
+                stream = device.SymbolStream.from_texts([text], kind)
+                pos, score = device.scan_alpha(stream, self.table(kind.letters), threshold)
             for p, s in zip(pos.tolist(), score.tolist()):
                 yield (p, s)                       # Python float

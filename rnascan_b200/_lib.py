@@ -15,6 +15,7 @@ RS_F32, RS_F64 = 0, 1
 RS_MODE_STRUCT, RS_MODE_AND = 0, 1
 RS_ROWS_F32, RS_ROWS_F32_SHADOW, RS_ROWS_Q8, RS_ROWS_Q4 = 0, 1, 2, 3
 RS_SEP, RS_RNA_OTHER, RS_SS_OTHER, RS_MAX_W = 0xFF, 0x0C, 0x0F, 64
+RS_ALPHA_OTHER, RS_ALPHA_LOWER = 0x1F, 0x20
 RS_MILLI_NAN, RS_MILLI_NINF, RS_MILLI_NEG0, RS_MILLI_RANGE = -2147483648, -2147483647, -2147483646, -2147483645
 
 
@@ -51,6 +52,7 @@ _SIGS = {
     "rs_host_parse_doubles": ([ctypes.c_char_p, _i64, _vp, _i64, _vp, _vp], _int),
     "rs_host_encode_rna": ([_vp, _i64, _vp], _int),
     "rs_host_encode_struct": ([_vp, _i64, _vp], _int),
+    "rs_host_encode_alpha": ([_vp, _i64, ctypes.c_char_p, _int, _vp], _int),
     "rs_host_log_odds": ([_vp, _vp, _int, _int, _vp], _int),
     "rs_host_annotate_structures": ([_vp, _vp, _vp, _i64, _vp, _vp], _int),
     "rs_host_format_hits": ([_i64, _i64, _vp, ctypes.c_char_p, _vp, ctypes.c_char_p, _vp, ctypes.c_char_p, _vp, _i64,
@@ -60,13 +62,16 @@ _SIGS = {
                                       _int, _vp, _vp, _i64, _vp], _int),
     "rs_hist": ([_vp, _i64, _vp, _vp], _int),
     "rs_hist_rna": ([_vp, _i64, _vp, _vp], _int),
+    "rs_hist_alpha": ([_vp, _i64, _vp, _vp], _int),
     "rs_scores_dense_seq": ([_vp, _i64, _vp, _int, _vp, _vp], _int),
     "rs_scores_dense_struct": ([_vp, _i64, _vp, _int, _vp, _vp], _int),
     "rs_scores_dense_struct_milli": ([_vp, _i64, _vp, _int, _vp, _vp], _int),
+    "rs_scores_dense_alpha": ([_vp, _i64, _vp, _int, _int, _vp, _vp], _int),
     "rs_scores_dense_profile": ([_vp, _int, _i64, _vp, _vp, _int, _vp, _vp], _int),
     "rs_profile_stats": ([_vp, _int, _i64, _vp, _vp], _int),
     "rs_scan_seq": ([_vp, _i64, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _i64, _vp], _int),
     "rs_scan_struct_onehot": ([_vp, _i64, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _i64, _vp], _int),
+    "rs_scan_alpha": ([_vp, _i64, _vp, _int, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _i64, _vp], _int),
     "rs_scan_pair_onehot": ([_vp, _vp, _i64, _vp, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _vp, _i64,
                              _vp], _int),
     "rs_scan_fused": ([_vp, _vp, _int, _i64, _vp, _vp, _int, _dbl, _dbl, _int, _i64, _vp, _vp, _vp, _vp,

@@ -128,16 +128,19 @@ __device__ __forceinline__ double rs_exact_profile_window(const PT *rows /* firs
 
 // One window of a one-hot PSSM score: sequential double adds in j order (_pwm.c:36-60,
 // matrix.py:34-38).  A = number of valid letters (4 or 7), table row stride TS doubles.
+// The letter index is code & 7 for TS <= 8 (RNA and structure layouts) and code & 31 for TS = 32
+// (alphabet layout, whose letter count is only known at run time: pass it as n_letters).
 // Returns false when the window holds an invalid symbol (score is NaN in the reference).
 template <int A, int TS>
 __device__ __forceinline__ bool rs_exact_onehot_window(const uint8_t *codes, const double *tab, int W,
-                                                       double &score)
+                                                       double &score, int n_letters = A)
 {
+    constexpr int MASK = TS > 8 ? TS - 1 : 7;
     double s = 0.0;
     bool ok = true;
     for (int j = 0; j < W; j++) {
-        int idx = codes[j] & 7;
-        if (idx >= A) { ok = false; break; }
+        int idx = codes[j] & MASK;
+        if (idx >= n_letters) { ok = false; break; }
         s = __dadd_rn(s, tab[j * TS + idx]);
     }
     score = s;

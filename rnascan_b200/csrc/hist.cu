@@ -155,3 +155,74 @@ extern "C" int rs_hist(const uint8_t *d_codes, int64_t n, uint64_t *d_counts8, v
 {
     return hist_launch<3>(d_codes, n, d_counts8, stream);
 }
+
+// ---- alphabet layout (rs_host_encode_alpha): 32 bins, bin = code & 31, counted iff bit 5 is clear ----------------
+// Replaces the same Seq.count() loop (rnascan.py:450-453) for alphabets of up to 31 letters.  Lower-case letters
+// (bit 5) and separators (0xFF) are not counted; bin 31 collects the layout's "other" symbol 0x1F, which is no letter.
+// Each lane owns one column of its warp's 32 x 32 counter block in shared memory (no bank conflicts, no contention):
+// the increments are fire-and-forget shared atomics, so consecutive symbols of one lane do not wait for each other.
+// A lane counts at most n / (threads of the grid) symbols: 32-bit counters hold any stream that fits on a device.
+__global__ void __launch_bounds__(HI_THREADS) hist32_kernel(const uint8_t *__restrict__ codes, int64_t n,
+                                                            unsigned long long *__restrict__ counts)
+{
+    __shared__ unsigned s_cnt[HI_THREADS / 32][32][32];       // [warp][bin][lane]
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned (*mine)[32] = s_cnt[warp];
+#pragma unroll
+    for (int b = 0; b < 32; b++) mine[b][lane] = 0;
+    auto count_word = [&](unsigned w) {
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const unsigned c = (w >> (8 * k)) & 0xFFu;
+            if (!(c & 0x20u)) atomicAdd(&mine[c & 31u][lane], 1u);
+        }
+    };
+    const int64_t nvec = n / 16;
+    const uint4 *v = reinterpret_cast<const uint4 *>(codes);
+    const int64_t gstride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nvec; i += HI_UNROLL * gstride) {
+        uint4 q[HI_UNROLL];
+#pragma unroll
+        for (int u = 0; u < HI_UNROLL; u++) {
+            const int64_t j = i + u * gstride;
+            q[u] = j < nvec ? __ldg(v + j) : make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
+        }
+#pragma unroll
+        for (int u = 0; u < HI_UNROLL; u++) {
+            count_word(q[u].x); count_word(q[u].y); count_word(q[u].z); count_word(q[u].w);
+        }
+    }
+    if (blockIdx.x == 0 && threadIdx.x < (n & 15)) {           // tail symbols (n % 16)
+        const unsigned c = codes[nvec * 16 + threadIdx.x];
+        if (!(c & 0x20u)) atomicAdd(&mine[c & 31u][lane], 1u);
+    }
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        unsigned long long sum = 0;
+        for (int w = 0; w < HI_THREADS / 32; w++)
+            for (int l = 0; l < 32; l++) sum += s_cnt[w][threadIdx.x][(l + threadIdx.x) & 31];
+        if (sum) atomicAdd(&counts[threadIdx.x], sum);
+    }
+}
+
+extern "C" int rs_hist_alpha(const uint8_t *d_codes, int64_t n, uint64_t *d_counts32, void *stream)
+{
+    if (!d_codes || !d_counts32 || n < 0) { rs_set_error("rs_hist_alpha: bad argument"); return RS_ERR_INVALID; }
+    if ((uintptr_t)d_codes & 15) { rs_set_error("codes pointer must be 16-byte aligned"); return RS_ERR_INVALID; }
+    if (n == 0) return RS_OK;
+    int64_t blocks = (n / 64 + HI_THREADS - 1) / HI_THREADS;
+    static int per_sm[RS_MAX_DEVICES] = {};                   // one resident wave, as hist_launch
+    const int dev = rs_current_device();
+    if (!per_sm[dev]) {
+        int v = 0;
+        RS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, hist32_kernel, HI_THREADS, 0));
+        per_sm[dev] = v > 0 ? v : 4;
+    }
+    const int64_t cap = (int64_t)rs_sm_count() * per_sm[dev];
+    if (blocks > cap) blocks = cap;
+    if (blocks < 1) blocks = 1;
+    hist32_kernel<<<(unsigned)blocks, HI_THREADS, 0, (cudaStream_t)stream>>>(d_codes, n,
+                                                                           (unsigned long long *)d_counts32);
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
+}

@@ -9,6 +9,8 @@
 #include <cmath>
 #include "../../include/rnascan_b200.h"
 
+void rs_set_error(const char *fmt, ...);        // capi.cu
+
 namespace {
 struct Luts {
     uint8_t rna[256], ss[256];
@@ -48,6 +50,34 @@ extern "C" int rs_host_encode_struct(const uint8_t *text, int64_t n, uint8_t *co
 {
     if (n < 0 || (n > 0 && (!text || !codes))) return RS_ERR_INVALID;
     run(text, n, codes, g_luts.ss);
+    return RS_OK;
+}
+
+// The alphabet layout: index of the upper-cased byte in `letters` (bits 0-4), bit 5 for a lower-case byte (scored,
+// not counted: str.upper() before scoring, matrix.py:36-41, but a case-sensitive Seq.count, rnascan.py:450-453),
+// 0x1F for any other byte.  Letters: 1..31 distinct ASCII characters, none of them lower-case a-z (a lower-case
+// letter would need two indices in one code).
+extern "C" int rs_host_encode_alpha(const uint8_t *text, int64_t n, const uint8_t *letters, int n_letters,
+                                    uint8_t *codes)
+{
+    if (n < 0 || (n > 0 && (!text || !codes))) return RS_ERR_INVALID;
+    if (!letters || n_letters < 1 || n_letters > 31) {
+        rs_set_error("alphabet of %d letters: 1..31 are supported", n_letters);
+        return RS_ERR_INVALID;
+    }
+    uint8_t lut[256];
+    std::fill(lut, lut + 256, (uint8_t)RS_ALPHA_OTHER);
+    for (int k = 0; k < n_letters; k++) {
+        const uint8_t c = letters[k];
+        if (c >= 128 || (c >= 'a' && c <= 'z') || lut[c] != RS_ALPHA_OTHER) {
+            rs_set_error("alphabet letter %d (byte %d) is not a distinct ASCII character outside a-z", k, (int)c);
+            return RS_ERR_INVALID;
+        }
+        lut[c] = (uint8_t)k;
+    }
+    for (int c = 'a'; c <= 'z'; c++)
+        if (lut[c - 32] != RS_ALPHA_OTHER) lut[c] = (uint8_t)(lut[c - 32] | RS_ALPHA_LOWER);
+    run(text, n, codes, lut);
     return RS_OK;
 }
 

@@ -44,14 +44,52 @@ def padded_count(n):
     return int(lib.rs_padded_count(int(n)))
 
 
+MAX_ALPHA_LETTERS = 31
+
+
+class AlphaKind(object):
+    """Stream kind of any other alphabet: the "alphabet" layout of rnascan_b200.h, letter k of `letters` (in
+    the caller's column order) has index k.  Supported: 1..31 distinct single ASCII characters, none of them a
+    lower-case a-z (text is scored upper-cased but counted case-sensitively, so a lower-case letter would need
+    two indices in one code); NotImplementedError names the rule otherwise."""
+
+    def __init__(self, letters):
+        letters = "".join(letters) if letters is not None else ""
+        if not (1 <= len(letters) <= MAX_ALPHA_LETTERS and len(set(letters)) == len(letters)
+                and all(ord(c) < 128 and not "a" <= c <= "z" for c in letters)):
+            raise NotImplementedError(
+                "GPU scoring supports GAUC, BEHLMRT and alphabets of 1 to %d distinct single ASCII characters "
+                "without lower-case a-z (got %r)" % (MAX_ALPHA_LETTERS, letters))
+        self.letters = letters
+
+    def __eq__(self, other):
+        return isinstance(other, AlphaKind) and other.letters == self.letters
+
+    def __ne__(self, other):
+        return not self == other
+
+    def __hash__(self):
+        return hash(("alpha", self.letters))
+
+    def __repr__(self):
+        return "AlphaKind(%r)" % self.letters
+
+
 # --------------------------------------------------------------------------- packing (host)
 def pack_texts(texts, kind):
-    """Encode a list of record strings into one symbol stream (host, numpy).
+    """Encode a list of record strings into one symbol stream (host, numpy).  `kind`: "rna", "struct" or an
+    AlphaKind.
 
     Returns (codes uint8[n_total], offsets int64[R], lengths int64[R]); record r occupies
     codes[offsets[r] : offsets[r]+lengths[r]] and is followed by one separator.
     """
-    enc = lib.rs_host_encode_rna if kind == "rna" else lib.rs_host_encode_struct
+    if isinstance(kind, AlphaKind):
+        letters = kind.letters.encode("ascii")
+
+        def enc(src, n, dst):
+            return lib.rs_host_encode_alpha(src, n, letters, len(letters), dst)
+    else:
+        enc = lib.rs_host_encode_rna if kind == "rna" else lib.rs_host_encode_struct
     lengths = np.fromiter((len(t) for t in texts), dtype=np.int64, count=len(texts))
     offsets = np.zeros(len(texts), dtype=np.int64)
     if len(texts) > 1:
@@ -85,7 +123,7 @@ class SymbolStream(object):
     def __init__(self, codes, offsets=None, lengths=None, device=None, kind=None):
         require_cuda()
         codes = np.ascontiguousarray(codes, dtype=np.uint8)
-        self.kind = kind                 # "rna" | "struct" | None (unknown: generic kernels)
+        self.kind = kind                 # "rna" | "struct" | AlphaKind | None (unknown: generic kernels)
         self.n = int(codes.shape[0])
         self.offsets = np.zeros(1, np.int64) if offsets is None else np.asarray(offsets, np.int64)
         self.lengths = np.array([self.n], np.int64) if lengths is None else np.asarray(lengths, np.int64)
@@ -185,7 +223,13 @@ def _table(table, cols):
 
 
 def histogram(stream):
-    """int64[8] exact counts of symbols 0..7 whose 'not counted' bit is clear."""
+    """int64[8] exact counts of symbols 0..7 whose 'not counted' bit is clear; for an AlphaKind stream
+    int64[A], the counts of its A letters in upper case."""
+    kind = getattr(stream, "kind", None)
+    if isinstance(kind, AlphaKind):
+        counts = torch.zeros(32, dtype=torch.int64, device=stream.codes.device)
+        check(lib.rs_hist_alpha(_ptr(stream.codes), stream.n, _ptr(counts), _stream()))
+        return counts[:len(kind.letters)]
     counts = torch.zeros(8, dtype=torch.int64, device=stream.codes.device)
     fn = lib.rs_hist_rna if getattr(stream, "kind", None) == "rna" else lib.rs_hist
     check(fn(_ptr(stream.codes), stream.n, _ptr(counts), _stream()))
@@ -207,6 +251,24 @@ def dense_struct(stream, table):
     nout = max(0, stream.n - W + 1)
     out = torch.empty(max(nout, 1), dtype=torch.float64, device=stream.codes.device)
     check(lib.rs_scores_dense_struct(_ptr(stream.codes), stream.n, t.ctypes.data, W, _ptr(out), _stream()))
+    return out[:nout]
+
+
+def _alpha_table(table):
+    t = np.ascontiguousarray(table, dtype=np.float64)
+    if t.ndim != 2 or not 1 <= t.shape[1] <= MAX_ALPHA_LETTERS:
+        raise ValueError("position-weight matrix must be (width, 1..%d letters)" % MAX_ALPHA_LETTERS)
+    return _table(t, t.shape[1])
+
+
+def dense_alpha(stream, table):
+    """float64 score of every window of an alphabet-layout stream (rs_scores_dense_alpha); table (W, A), column k
+    = letter index k of the stream's codes."""
+    t = _alpha_table(table)
+    W, A = t.shape
+    nout = max(0, stream.n - W + 1)
+    out = torch.empty(max(nout, 1), dtype=torch.float64, device=stream.codes.device)
+    check(lib.rs_scores_dense_alpha(_ptr(stream.codes), stream.n, t.ctypes.data, W, A, _ptr(out), _stream()))
     return out[:nout]
 
 
@@ -313,6 +375,26 @@ def scan_struct_onehot(stream, table, threshold, capacity=None):
         check(lib.rs_scan_struct_onehot(_ptr(stream.codes), stream.n, t.ctypes.data, W, threshold,
                                         hb.capacity, _ptr(hb.pos), _ptr(hb.struct), _ptr(hb.counters),
                                         _ptr(hb.work), hb.work_bytes, _stream()))
+    pos, _, st, _ = _run_thresholded(stream.n, stream.codes.device, launch, False, True, capacity)
+    return pos, st
+
+
+def scan_alpha(stream, table, threshold, capacity=None):
+    """Ordered (pos int64[], score float64[]) of the windows of an alphabet-layout stream with score > threshold
+    (rs_scan_alpha); table as for dense_alpha."""
+    t = _alpha_table(table)
+    W, A = t.shape
+    threshold = float(threshold)
+    if threshold == float("-inf"):
+        sc = dense_alpha(stream, t).cpu().numpy()
+        with np.errstate(invalid="ignore"):
+            pos = np.nonzero(sc > threshold)[0].astype(np.int64)
+        return pos, sc[pos]
+
+    def launch(hb):
+        check(lib.rs_scan_alpha(_ptr(stream.codes), stream.n, t.ctypes.data, W, A, threshold, hb.capacity,
+                                _ptr(hb.pos), _ptr(hb.struct), _ptr(hb.counters), _ptr(hb.work), hb.work_bytes,
+                                _stream()))
     pos, _, st, _ = _run_thresholded(stream.n, stream.codes.device, launch, False, True, capacity)
     return pos, st
 

@@ -164,21 +164,26 @@ def pwm_scan_fwd(pwm, seq):
     seq = str(seq)
     if len(seq) - length + 1 <= 0:
         return []
-    if len(letters) > 7 or any(len(letter) != 1 or ord(letter) > 255 for letter in letters):
-        raise NotImplementedError("GPU scoring supports alphabets of up to 7 single-byte letters")
-    lut = np.full(256, device._lib.RS_SS_OTHER, np.uint8)
+    if len(letters) > device.MAX_ALPHA_LETTERS or any(len(letter) != 1 or ord(letter) > 255 for letter in letters):
+        raise NotImplementedError("GPU scoring supports alphabets of up to %d single-byte letters"
+                                  % device.MAX_ALPHA_LETTERS)
+    lut = np.full(256, device._lib.RS_ALPHA_OTHER, np.uint8)      # case-sensitive: each key has its own index
     for k, letter in enumerate(letters):
         lut[ord(letter)] = k
     raw = np.frombuffer(seq.encode("latin-1", "replace"), np.uint8)
     codes = lut[raw]
-    bad = np.nonzero(codes == device._lib.RS_SS_OTHER)[0]
+    bad = np.nonzero(codes == device._lib.RS_ALPHA_OTHER)[0]
     if len(bad):
         raise KeyError(seq[int(bad[0])])
-    table = np.zeros((length, 7), np.float64)
-    for k, letter in enumerate(letters):
-        table[:, k] = pwm[letter]
     stream = device.SymbolStream(codes)
-    scores = device.dense_struct(stream, table).cpu().numpy()
+    if len(letters) <= 7:                                         # the structure kernels, table padded to 7 columns
+        table = np.zeros((length, 7), np.float64)
+        for k, letter in enumerate(letters):
+            table[:, k] = pwm[letter]
+        scores = device.dense_struct(stream, table).cpu().numpy()
+    else:
+        table = np.array([pwm[letter] for letter in letters], np.float64).T
+        scores = device.dense_alpha(stream, table).cpu().numpy()
     return [float(v) for v in scores]
 
 

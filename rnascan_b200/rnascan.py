@@ -423,16 +423,18 @@ class _Batch(object):
         return self
 
     def overlap_counts(self):
-        """Counts (int64[8]) of the symbols this rank holds but does not own (the overlap
-        tails of split records); the device histogram minus these is the owned count."""
-        counts = np.zeros(8, np.int64)
+        """Counts (int64[8], int64[A] for an alphabet kind: the bins of device.histogram) of the symbols this rank
+        holds but does not own (the overlap tails of split records); the device histogram minus these is the
+        owned count."""
+        bins = 8 if self.kind in ("rna", "struct") else len(self.kind.letters)
+        counts = np.zeros(bins, np.int64)
         if self.own is None:
             return counts
         host = self.stream.host_codes()
         for k in np.nonzero(self.own < self.stream.lengths)[0]:
             a = self.stream.offsets[k] + self.own[k]
             tail = host[a:self.stream.offsets[k] + self.stream.lengths[k]]
-            counts += np.bincount(tail[tail < 8], minlength=8)[:8]
+            counts += np.bincount(tail[tail < bins], minlength=bins)[:bins]
         return counts
 
     def locate(self, pos):
@@ -519,12 +521,15 @@ def _native_batch(fasta_file, alphabet):
 def _native_parse(fasta_file, alphabet, max_symbols=None):
     """(text uint8[], codes uint8[], offsets, lengths, ids, descriptions, kind) of a FASTA input from the native
     two-pass parser, records laid out one after the other with one separator each; None when it does not
-    apply (non-ASCII input, DNA target alphabet, unreadable file, more than `max_symbols`)."""
+    apply (non-ASCII input, DNA target alphabet, an alphabet other than GAUC and BEHLMRT, unreadable file, more
+    than `max_symbols`)."""
     from . import _lib
     rna_target = _seq.is_ambiguous_rna_alphabet(alphabet)
     kind = _kind_of(alphabet)
     if kind == "rna" and not rna_target:
         return None                                   # DNA target alphabets: no transcription (not a CLI path)
+    if kind not in ("rna", "struct"):
+        return None                                   # other alphabets: the Python parser (not a CLI path)
     try:
         data = _read_fasta_bytes(fasta_file)
     except (OSError, EOFError):
@@ -558,7 +563,14 @@ NATIVE_INGEST = True                 # tests switch it off to exercise the Pytho
 
 
 def _kind_of(alphabet):
-    return "rna" if _seq.is_nucleotide_alphabet(alphabet) else "struct"
+    """Stream kind of a target alphabet: "rna" (nucleotides), "struct" (BEHLMRT) or a device.AlphaKind for any
+    other alphabet (NotImplementedError, naming the rule, for one the device layouts cannot hold)."""
+    from . import device
+    if _seq.is_nucleotide_alphabet(alphabet):
+        return "rna"
+    if sorted(alphabet.letters or "") == sorted(device.CHANNELS):
+        return "struct"
+    return device.AlphaKind(alphabet.letters)
 
 
 def _sharded_batch(fasta_file, alphabet, rank, size):
@@ -614,9 +626,16 @@ def _record_batches(fasta_file, alphabet, max_symbols=None):
         yield _Batch(ids, descs, texts, _kind_of(alphabet))
 
 
-def _table_for(pm, kind):
+def _columns(kind):
+    """Device column order of a stream kind: the order of tables and histogram bins."""
     from . import device
-    return pm.table(device.RNA_COLUMNS if kind == "rna" else device.CHANNELS)
+    if kind == "rna":
+        return device.RNA_COLUMNS
+    return device.CHANNELS if kind == "struct" else kind.letters
+
+
+def _table_for(pm, kind):
+    return pm.table(_columns(kind))
 
 
 def _first_motif(pssm):
@@ -826,6 +845,8 @@ def _scan_batch(batch, pm, kind, minscore):
     with STATS.phase("scan_s"):
         if kind == "rna":
             pos, scores = device.scan_seq(batch.stream, table, minscore)
+        elif kind != "struct":
+            pos, scores = device.scan_alpha(batch.stream, table, minscore)
         else:
             every = None
             if minscore == float("-inf"):               # every position: the device rounds, 4 B per window come back
@@ -1011,8 +1032,6 @@ def _scan_fasta_hits(fasta_file, pssm, alphabet, minscore):
     eprint("Scanning sequences ")
     motif_id, pm = _first_motif(pssm)
     kind = _kind_of(alphabet)
-    if kind == "struct" and not pm._is_structure():
-        raise NotImplementedError("GPU scoring supports the nucleotide and BEHLMRT structure alphabets")
     batches = _cached_batches(fasta_file, alphabet)
     parts, n_records = [], 0
     for batch in batches:
@@ -1033,7 +1052,9 @@ def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, mi
     Returns (bg, pssm, _HitTable), or None when this shape of run takes the serial path."""
     from . import device
     kind = _kind_of(alphabet)
-    columns = device.RNA_COLUMNS if kind == "rna" else device.CHANNELS
+    if kind not in ("rna", "struct"):
+        return None
+    columns = _columns(kind)
     if not np.isfinite(minscore) or any(letter not in columns for letter in alphabet.letters):
         return None
     batches = _cached_batches(fasta_file, alphabet)
@@ -1421,10 +1442,10 @@ def compute_background(fastas, alphabet, verbose=True):
     from . import device
     eprint("Calculating background probabilities...")
     kind = _kind_of(alphabet)
-    columns = device.RNA_COLUMNS if kind == "rna" else device.CHANNELS
-    if any(letter not in columns for letter in alphabet.letters):
-        raise NotImplementedError("GPU background counting supports GAUC and EHTBLRM alphabets")
-    counts = np.zeros(8, dtype=np.int64)
+    if any(letter not in _columns(kind) for letter in alphabet.letters):
+        raise NotImplementedError("GPU background counting of nucleotides supports the letters A, C, G, U only "
+                                  "(alphabet %r)" % (alphabet.letters,))
+    counts = np.zeros(8 if kind in ("rna", "struct") else len(kind.letters), dtype=np.int64)
     n_records = 0
     for batch in _cached_batches(fastas, alphabet):
         counts += device.histogram(batch.stream).cpu().numpy() - batch.overlap_counts()
@@ -1435,8 +1456,7 @@ def compute_background(fastas, alphabet, verbose=True):
 
 def _background_from_counts(counts, n_records, alphabet, verbose=True):
     """(count + 1) / (total + |alphabet|) per letter, messages and checks of rnascan.py:454-465."""
-    from . import device
-    columns = device.RNA_COLUMNS if _kind_of(alphabet) == "rna" else device.CHANNELS
+    columns = _columns(_kind_of(alphabet))
     content = defaultdict(int)
     total = len(alphabet.letters)
     if n_records:
