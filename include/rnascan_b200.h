@@ -458,6 +458,23 @@ int rs_scan_batched_shadow(const uint8_t *d_codes, const float *d_shadow_f32, co
                            uint64_t *d_motif_counters2, uint64_t *d_bases, void *d_work, int64_t work_bytes,
                            void *stream);
 
+/* ---- many one-hot PSSMs over ONE symbol stream (a motif collection over a FASTA input) -----------
+ * The reference scans one PFM per process run (rnascan.py:490-576); here M motifs are scanned over the
+ * same resident stream in one call.  alphabet 4: RNA-layout codes, scores as rs_scan_seq (float32, into
+ * d_hit_f32); alphabet 7: structure-layout codes, scores as rs_scan_struct_onehot (float64, d_hit_f64).
+ * Motif m has width widths[m] (1..16, <= table_stride_rows <= 16) and table tables[m][table_stride_rows]
+ * [alphabet] (rows >= widths[m] are ignored); the threshold must be finite.  n < 2^32.
+ * Hits come back grouped by motif (ascending), sorted by position inside a motif: d_hit_motif[k],
+ * d_hit_pos[k], score[k].  After syncing the stream, d_bases[m] .. d_bases[m+1] is motif m's slice and
+ * d_bases[n_motifs] the total (if it exceeds hit_capacity nothing beyond the capacity was stored: re-run
+ * with a larger buffer).  Per motif the hits and scores are exactly rs_scan_seq's / rs_scan_struct_onehot's.
+ * Motifs are processed in groups of 256 (one k-mer decision table of 2 MB / 1 MB each).                  */
+int64_t rs_scan_onehot_many_workspace_bytes(int alphabet, int64_t n, int n_motifs, int table_stride_rows);
+int rs_scan_onehot_many(int alphabet, const uint8_t *d_codes, int64_t n, int n_motifs, const int *widths,
+                        const double *tables, int table_stride_rows, double threshold, int64_t hit_capacity,
+                        int32_t *d_hit_motif, int64_t *d_hit_pos, float *d_hit_f32, double *d_hit_f64,
+                        uint64_t *d_bases, void *d_work, int64_t work_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -105,6 +105,9 @@ _SIGS = {
     "rs_last_batched_path": ([], _int),
     "rs_scan_batched": ([_vp, _vp, _int, _i64, _int, _vp, _vp, _vp, _int, _dbl, _dbl, _int, _i64, _vp, _vp,
                          _vp, _vp, _vp, _vp, _vp, _i64, _vp], _int),
+    "rs_scan_onehot_many_workspace_bytes": ([_int, _i64, _int, _int], _i64),
+    "rs_scan_onehot_many": ([_int, _vp, _i64, _int, _vp, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64,
+                             _vp], _int),
     "rs_scan_batched_shadow": ([_vp, _vp, _vp, _i64, _int, _vp, _vp, _vp, _int, _dbl, _dbl, _int, _i64, _vp, _vp,
                                 _vp, _vp, _vp, _vp, _vp, _i64, _vp], _int),
 }

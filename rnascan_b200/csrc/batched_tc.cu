@@ -28,7 +28,7 @@
 //               candidates staged per warp in shared memory, flushed with one atomic per ~1000
 //   warps 8-11  converters: fp32 rows -> bf16 x 8 rows (the A operand), fence.proxy.async; in RS_MODE_AND also
 //               the SEQUENCE MASK of every position of the tile (one thread per position): the 8-mer the window
-//               starts with indexes a 65536 x 256-bit table (seqmask_build_kernel: which motifs' sequence score can
+//               starts with indexes a 65536 x 256-bit table (kmer_mask_build_kernel: which motifs' sequence score can
 //               pass), restricted to the motifs no wider than the distance to the first invalid symbol; 32 B per
 //               position into an 8-stage shared-memory ring that the epilogue ANDs into its sign masks, so only
 //               (position, motif) pairs that can be combined hits are ever staged
@@ -427,40 +427,45 @@ __global__ void __launch_bounds__(TC_THREADS, 1) batched_tc_kernel(const __grid_
     }
 }
 
-// ------------------------------------------------------------------------------------------------ sequence mask
-// seqmask[kmer][word]: for the 8 symbols a window starts with, which motifs' SEQUENCE score can exceed the threshold.
-// W <= 8: the decision itself -- the reference's arithmetic (_pwm.c:36-65: float64 adds in j order, one cast to
-// float32; compared widened, SURVEY.md N1) over the first W symbols.  W > 8: the exact prefix sum plus the largest
-// the remaining rows can add (a superset; the exact pass decides).  Bit (31 - k) of word c stands for motif 32 c + k,
-// the order in which the epilogue's sign masks come out.
-__global__ void __launch_bounds__(256) seqmask_build_kernel(uint32_t *mask, int mask_words, const double *seq_tables,
-                                                            const int *widths, int n_motifs, int stride_rows,
-                                                            double threshold)
+// ------------------------------------------------------------------------------------------------ k-mer decision masks
+// mask[kmer][word]: for the K symbols a window starts with, which motifs' one-hot score can exceed the threshold.
+// A = 4: 8-mers of 2-bit codes (symbol j in bits 2j, 2j+1); A = 7: 5-mers of 3-bit codes (bits 3j .. 3j+2; index 7,
+// an invalid symbol, passes nothing -- the callers mask motifs wider than the distance to it anyway).
+// W <= K: the decision itself -- the reference's arithmetic (float64 adds in j order; A = 4 casts to float32 once
+// and compares widened, _pwm.c:36-65 and SURVEY.md N1; A = 7 compares the float64 sum, matrix.py:34-38).
+// W > K: the prefix sum, then the largest entry of every remaining row added in the same order.  Rounded addition
+// is monotone, so that is >= the exact score of every window with this prefix: a superset, the exact pass decides
+// (NaN: no bound, the window is a candidate).  Bit (31 - k) of word c stands for motif 32 c + k, the order in
+// which the tensor-core epilogue's sign masks come out.
+template <int A, int K>
+__global__ void __launch_bounds__(256) kmer_mask_build_kernel(uint32_t *mask, int mask_words, const double *tables,
+                                                              const int *widths, int n_motifs, int stride_rows,
+                                                              double threshold)
 {
-    // block (word, slab): the 32 motifs of one mask word, 1024 consecutive 8-mers; their tables sit in shared memory
-    __shared__ double s_tab[32 * 8 * 4];          // first 8 rows of each motif
-    __shared__ double s_rest[32];                 // W > 8: the most the rows beyond the 8th can add (NaN: no bound)
+    constexpr int BITS = A == 4 ? 2 : 3;
+    constexpr int REST = RS_KMER_WMAX - K;
+    // block (word, slab): the 32 motifs of one mask word, 1024 consecutive k-mers; their tables sit in shared memory
+    __shared__ double s_tab[32 * K * A];          // first K rows of each motif
+    __shared__ double s_rest[32][REST];           // W > K: the largest entry of each row beyond the K-th
     __shared__ int s_w[32];
     const int word = blockIdx.x, slab = blockIdx.y;
-    for (int k = threadIdx.x; k < 32 * 32; k += blockDim.x) {
-        const int m = word * 32 + (k >> 5), e = k & 31;                // e = row * 4 + letter
-        s_tab[k] = (m < n_motifs && (e >> 2) < stride_rows) ? seq_tables[(size_t)m * stride_rows * 4 + e] : 0.0;
+    for (int k = threadIdx.x; k < 32 * K * A; k += blockDim.x) {
+        const int m = word * 32 + k / (K * A), e = k % (K * A);                // e = row * A + letter
+        s_tab[k] = (m < n_motifs && e / A < stride_rows) ? tables[(size_t)m * stride_rows * A + e] : 0.0;
     }
     if (threadIdx.x < 32) {
         const int m = word * 32 + threadIdx.x;
         int W = 0;
-        double rest = 0.0;
         if (m < n_motifs) {
             W = widths[m];
-            const double *tab = seq_tables + (size_t)m * stride_rows * 4;
-            for (int j = 8; j < W; j++) {
-                const double mx = fmax(fmax(tab[j * 4], tab[j * 4 + 1]), fmax(tab[j * 4 + 2], tab[j * 4 + 3]));
-                if (mx != mx || mx == INFINITY) rest = nan("");         // NaN / +inf entries: let the exact pass decide
-                else rest += mx;
+            const double *tab = tables + (size_t)m * stride_rows * A;
+            for (int j = K; j < W; j++) {
+                double mx = tab[j * A];
+                for (int c = 1; c < A; c++) mx = fmax(mx, tab[j * A + c]);
+                s_rest[threadIdx.x][j - K] = mx;
             }
         }
         s_w[threadIdx.x] = W;
-        s_rest[threadIdx.x] = rest;
     }
     __syncthreads();
     for (int q = threadIdx.x; q < 1024; q += blockDim.x) {
@@ -469,23 +474,38 @@ __global__ void __launch_bounds__(256) seqmask_build_kernel(uint32_t *mask, int 
         for (int k = 0; k < 32; k++) {
             const int W = s_w[k];
             if (W == 0) break;
-            const double *tab = s_tab + k * 32;
-            const int wp = W < 8 ? W : 8;
+            const double *tab = s_tab + k * K * A;
+            const int wp = W < K ? W : K;
             double sum = 0.0;
-            for (int j = 0; j < wp; j++) sum = __dadd_rn(sum, tab[j * 4 + ((kmer >> (2 * j)) & 3u)]);
-            bool pass;
-            if (W <= 8) {
-                pass = (double)(float)sum > threshold;
-            } else {
-                // the sequential float64 adds of the real score differ from this sum by a few ulps at most
-                const double total = sum + s_rest[k];
-                const double bound = total + fabs(total) * 1e-12 + 1e-300;
-                pass = total != total || (double)(float)bound > threshold;
+            bool valid = true;
+            for (int j = 0; j < wp; j++) {
+                const uint32_t d = (kmer >> (BITS * j)) & ((1u << BITS) - 1u);
+                if (d >= (uint32_t)A) { valid = false; break; }
+                sum = __dadd_rn(sum, tab[j * A + d]);
             }
-            if (pass) bits |= 1u << (31 - k);
+            if (!valid) continue;
+            for (int j = K; j < W; j++) sum = __dadd_rn(sum, s_rest[k][j - K]);
+            const double cmp = A == 4 ? (double)(float)sum : sum;
+            if (cmp > threshold || (W > K && sum != sum)) bits |= 1u << (31 - k);
         }
         mask[(size_t)kmer * mask_words + word] = bits;
     }
+}
+
+// Builds mask[rows][mask_words] for n_motifs device-resident tables [n_motifs][stride_rows][alphabet] (W <= 16).
+int rs_kmer_mask_build(int alphabet, uint32_t *d_mask, int mask_words, const double *d_tables, const int *d_widths,
+                       int n_motifs, int stride_rows, double threshold, cudaStream_t st)
+{
+    if (alphabet == 4)
+        kmer_mask_build_kernel<4, 8><<<dim3((unsigned)mask_words, 64), 256, 0, st>>>(d_mask, mask_words, d_tables,
+                                                                                     d_widths, n_motifs, stride_rows,
+                                                                                     threshold);
+    else
+        kmer_mask_build_kernel<7, 5><<<dim3((unsigned)mask_words, 32), 256, 0, st>>>(d_mask, mask_words, d_tables,
+                                                                                     d_widths, n_motifs, stride_rows,
+                                                                                     threshold);
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ exact re-score
@@ -830,9 +850,8 @@ int rs_scan_batched_tc(const uint8_t *d_codes, const void *d_profile, int64_t n,
     }
     const bool use_mask = mode == RS_MODE_AND && seq_tables != nullptr && g_tc_seqmask;
     if (use_mask) {
-        seqmask_build_kernel<<<dim3((unsigned)mask_words, 64), 256, 0, st>>>(d_seqmask, mask_words, d_ts, d_w, n_motifs,
-                                                                            stride_rows, threshold);
-        RS_CUDA(cudaGetLastError());
+        int rc = rs_kmer_mask_build(4, d_seqmask, mask_words, d_ts, d_w, n_motifs, stride_rows, threshold, st);
+        if (rc) return rc;
     }
     TcParams tp = {};
     tp.codes = use_mask ? d_codes : nullptr; tp.seqmask = d_seqmask; tp.mask_words = mask_words;

@@ -246,6 +246,11 @@ int rs_scan_pair_masks(const uint8_t *d_seq_codes, const uint8_t *d_struct_codes
                        const double *struct_table, int W, double threshold, int64_t cap, int64_t *d_hit_pos,
                        float *d_hit_seq, double *d_hit_str, uint64_t *d_counters2, void *d_work, cudaStream_t st);
 int64_t rs_kmer_work_bytes(int64_t n);   // workspace of the W <= 8 sequence scan (kmer_scan.cu)
+#define RS_KMER_WMAX 16          // widest motif the k-mer decision masks take
+// k-mer decision masks of one-hot motifs (batched_tc.cu): mask[kmer][word], bit (31 - k) of word c = motif 32 c + k
+// may pass; alphabet 4: 8-mers (65536 rows), 7: 5-mers (32768 rows); device tables [n_motifs][stride_rows][alphabet].
+int rs_kmer_mask_build(int alphabet, uint32_t *d_mask, int mask_words, const double *d_tables, const int *d_widths,
+                       int n_motifs, int stride_rows, double threshold, cudaStream_t st);
 
 int rs_scan_seq_kmer(const uint8_t *d_codes, int64_t n, const double *table, int W, double threshold, int64_t cap,
                      int64_t *d_hit_pos, float *d_hit_score, uint64_t *d_counters2, void *d_work, cudaStream_t st);

@@ -847,6 +847,56 @@ def scan_batched(stream, profile, seq_tables, struct_tables, threshold, capacity
         cap = total
 
 
+MANY_MAX_W = 16                 # widest motif scan_onehot_many takes
+
+
+def scan_onehot_many(stream, tables, threshold, capacity=None):
+    """Many one-hot PSSMs over one FASTA symbol stream in one call (rs_scan_onehot_many).
+
+    stream.kind "rna": tables (W_m, 4) in ACGU order, float32 scores as scan_seq; "struct": (W_m, 7) in
+    BEHLMRT order, float64 scores as scan_struct_onehot.  Widths 1..16, finite threshold.  Returns
+    (motif int32[], pos int64[], scores, bases int64[M+1]) with hits grouped by motif, ordered by position:
+    bases[m] .. bases[m+1] is motif m's slice, identical to the per-motif scan."""
+    if stream.kind not in ("rna", "struct"):
+        raise ValueError("scan_onehot_many takes RNA or structure streams (kind %r)" % (stream.kind,))
+    A = 4 if stream.kind == "rna" else 7
+    M = len(tables)
+    if M == 0:
+        raise ValueError("no motifs")
+    ts = [_table(t, A) for t in tables]
+    widths = np.array([t.shape[0] for t in ts], dtype=np.int32)
+    if widths.max() > MANY_MAX_W:
+        raise ValueError("scan_onehot_many takes motifs up to %d wide (%d found)" % (MANY_MAX_W, widths.max()))
+    stride = int(widths.max())
+    packed = np.zeros((M, stride, A), np.float64)
+    for m, t in enumerate(ts):
+        packed[m, :t.shape[0]] = t
+    threshold = float(threshold)
+    if not np.isfinite(threshold):
+        raise ValueError("scan_onehot_many needs a finite threshold")
+    dev = stream.codes.device
+    work_bytes = int(lib.rs_scan_onehot_many_workspace_bytes(A, stream.n, M, stride))
+    if work_bytes < 0:
+        check(_lib.RS_ERR_INVALID)
+    work = torch.empty(max(work_bytes, 1), dtype=torch.uint8, device=dev)
+    bases = torch.zeros(M + 1, dtype=torch.int64, device=dev)
+    sdt = torch.float32 if A == 4 else torch.float64
+    cap = int(capacity) if capacity else max(1 << 16, stream.n // 16)
+    while True:
+        motif = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+        pos = torch.empty(max(cap, 1), dtype=torch.int64, device=dev)
+        scores = torch.empty(max(cap, 1), dtype=sdt, device=dev)
+        check(lib.rs_scan_onehot_many(A, _ptr(stream.codes), stream.n, M, widths.ctypes.data, packed.ctypes.data,
+                                      stride, threshold, cap, _ptr(motif), _ptr(pos),
+                                      _ptr(scores) if A == 4 else 0, 0 if A == 4 else _ptr(scores), _ptr(bases),
+                                      _ptr(work), work_bytes, _stream()))
+        b = bases.cpu().numpy()
+        total = int(b[-1])
+        if total <= cap:
+            return motif[:total].cpu().numpy(), pos[:total].cpu().numpy(), scores[:total].cpu().numpy(), b
+        cap = total
+
+
 # --------------------------------------------------------------------------- host-buffer pipeline
 class _HitOverflow(Exception):
     def __init__(self, found):

@@ -1026,21 +1026,60 @@ def _emit(out, text):
         out.write(text)
 
 
-def _scan_fasta_hits(fasta_file, pssm, alphabet, minscore):
+def _scan_fasta_hits(fasta_file, pssm, alphabet, minscore, precomputed=None):
     """All records of a FASTA input in one (or a few) kernel launches, as a _HitTable (None on ranks other than
-    0 under torchrun)."""
+    0 under torchrun).  `precomputed`: this motif's hits from the batched scan of its motif collection
+    (_batched_fasta_hits); the input is then not scanned again."""
     eprint("Scanning sequences ")
     motif_id, pm = _first_motif(pssm)
     kind = _kind_of(alphabet)
     batches = _cached_batches(fasta_file, alphabet)
+    if precomputed is not None:
+        eprint("Processed %d sequences" % sum(len(b.ids) for b in batches))
+        hits = precomputed.hits
+    else:
+        parts, n_records = [], 0
+        for batch in batches:
+            rec, start0, scores = _scan_batch(batch, pm, kind, minscore)
+            parts.append((rec + n_records, start0, scores))
+            n_records += len(batch.ids)
+        eprint("Processed %d sequences" % n_records)
+        hits = _gather(parts or [(np.zeros(0, np.int64),) * 3])
+    return None if hits is None else _fasta_table(motif_id, pm.length, kind, batches, *hits)
+
+
+class _FastaHits(object):
+    """One motif's hits from the batched scan of a FASTA input: (record index, 0-based start, scores) on rank 0,
+    None on the other ranks under torchrun."""
+
+    def __init__(self, hits):
+        self.hits = hits
+
+
+def _fasta_many_hits(batches, kind, tables, minscore):
+    """Hits of every table on the FASTA input `batches` from one device.scan_onehot_many call per batch: one
+    (record index, 0-based start, scores) tuple per table, or None per table on ranks other than 0.  Under
+    torchrun each rank scans its own pieces and the whole collection makes ONE _gather."""
+    from . import device
     parts, n_records = [], 0
     for batch in batches:
-        rec, start0, scores = _scan_batch(batch, pm, kind, minscore)
-        parts.append((rec + n_records, start0, scores))
+        with STATS.phase("scan_s"):
+            motif, pos, scores, _ = device.scan_onehot_many(batch.stream, tables, minscore)
+        lengths = batch.stream.lengths
+        STATS.add("scored_positions", sum(int(np.maximum(lengths - t.shape[0] + 1, 0).sum()) for t in tables))
+        keep, rec, start0 = batch.locate(pos)
+        parts.append((motif[keep], rec[keep] + n_records, start0[keep], scores[keep]))
         n_records += len(batch.ids)
-    eprint("Processed %d sequences" % n_records)
-    hits = _gather(parts or [(np.zeros(0, np.int64),) * 3])
-    return None if hits is None else _fasta_table(motif_id, pm.length, kind, batches, *hits)
+    empty = (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64),
+             np.zeros(0, np.float32 if kind == "rna" else np.float64))
+    hits = _gather(parts or [empty])
+    if hits is None:
+        return [None] * len(tables)
+    motif, rec, start0, scores = hits
+    order = np.argsort(motif, kind="stable")          # rank order (= record order) within each motif
+    motif, rec, start0, scores = motif[order], rec[order], start0[order], scores[order]
+    cut = np.searchsorted(motif, np.arange(len(tables) + 1))
+    return [(rec[a:b], start0[a:b], scores[a:b]) for a, b in zip(cut[:-1], cut[1:])]
 
 
 def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, minscore):
@@ -1410,7 +1449,7 @@ def _scan_table(fasta_file, pssm, alphabet, args, precomputed=None):
     if os.path.isdir(fasta_file):
         return _scan_profile_dir(fasta_file, pssm, args.minscore, args.debug, write_pack=getattr(args, "pack", False),
                                  precomputed=precomputed)
-    return _scan_fasta_hits(fasta_file, pssm, alphabet, args.minscore)
+    return _scan_fasta_hits(fasta_file, pssm, alphabet, args.minscore, precomputed)
 
 
 def combine(seq_results, struct_results):
@@ -1588,7 +1627,7 @@ def _run_multi(args, seq_type, rank, pairs):
     try:
         pre = None
         if not args.bgonly:
-            pre = _batched_profile_hits(args, seq_type, pairs)
+            pre = _batched_profile_hits(args, seq_type, pairs) or _batched_fasta_hits(args, seq_type, pairs)
         for k, (seq_pfm, struct_pfm) in enumerate(pairs):
             one = copy.copy(args)
             one.pfm_seq, one.pfm_struct = seq_pfm, struct_pfm
@@ -1660,6 +1699,69 @@ def _batched_profile_hits(args, seq_type, pairs):
         a, b = int(bases[k]), int(bases[k + 1])
         out.append((pos[a:b], None if sq is None else sq[a:b], st[a:b]))
     return out
+
+
+MULTI_FASTA_MIN_MOTIFS = 2           # motif collections from this size on are scanned over a FASTA input in one pass
+
+
+def _on_device(batches):
+    """True when every batch's stream is resident on a CUDA device (what the batched kernel reads)."""
+    return all(b.stream.codes.is_cuda for b in batches)
+
+
+def _batched_fasta_hits(args, seq_type, pairs):
+    """Hits of every motif of a collection scanned over one FASTA input (modes RNA / SS) by
+    device.scan_onehot_many: a list of _FastaHits per motif, or None when this run does not have that shape (the
+    per-motif scans then run one after the other).  The background is taken once, quietly; every _run still
+    prints its own messages."""
+    if seq_type not in ("RNA", "SS") or args.testseq or args.bgonly or len(pairs) < MULTI_FASTA_MIN_MOTIFS:
+        return None
+    if not np.isfinite(args.minscore) or not args.fastafiles or os.path.isdir(args.fastafiles[0]):
+        return None
+    fasta = args.fastafiles[0]
+    if seq_type == "RNA":
+        alphabet, kind, bg_file, pfms = IUPAC.IUPACUnambiguousRNA(), "rna", args.bg_seq, [p for p, _ in pairs]
+    else:
+        alphabet, kind, bg_file, pfms = ContextualSecondaryStructure(), "struct", args.bg_struct, [q for _, q in pairs]
+    batches = _cached_batches(fasta, alphabet)
+    if not _on_device(batches):
+        return None
+    try:
+        bg = _quiet(load_background, bg_file, args.uniform_background, fasta, alphabet, False)
+        pms = [_first_motif(_quiet(load_motif, pfm, args.pseudocount, alphabet, bg))[1] for pfm in pfms]
+    except Exception:
+        return None                       # the per-motif run reports what is wrong
+    tables = [_table_for(pm, kind) for pm in pms]
+    if max(t.shape[0] for t in tables) > 16:
+        return None
+    hits = _fasta_many_hits(batches, kind, tables, args.minscore)
+    STATS.notes["batched_motifs"] = len(pairs)
+    return [_FastaHits(h) for h in hits]
+
+
+def scan_many_fasta(fasta_file, pssms, alphabet, minscore):
+    """Scan a FASTA file with MANY motifs in one batched pass per device batch.
+
+    pssms: a list of ``{motif_id: PSSM}`` as load_motif returns them, for the RNA or the
+    ContextualSecondaryStructure alphabet.  Returns one DataFrame per motif, equal to what
+    scan_main(fasta_file, pssm, alphabet, bg, args) returns for that motif (empty frames on ranks other than 0
+    under torchrun).  Motifs wider than 16 and a threshold of -inf are scanned one motif at a time."""
+    kind = _kind_of(alphabet)
+    if kind not in ("rna", "struct"):
+        raise NotImplementedError("scan_many_fasta takes the RNA or the ContextualSecondaryStructure alphabet")
+    pms = [_first_motif(p) for p in pssms]
+    tables = [_table_for(pm, kind) for _, pm in pms]
+    batches = _cached_batches(fasta_file, alphabet)
+    many = [k for k, t in enumerate(tables) if t.shape[0] <= 16] if np.isfinite(minscore) else []
+    hits = dict(zip(many, _fasta_many_hits(batches, kind, [tables[k] for k in many], minscore))) if many else {}
+    frames = []
+    for k, (motif_id, pm) in enumerate(pms):
+        if k in hits:
+            table = None if hits[k] is None else _fasta_table(motif_id, pm.length, kind, batches, *hits[k])
+        else:
+            table = _quiet(_scan_fasta_hits, fasta_file, pssms[k], alphabet, minscore)
+        frames.append(pd.DataFrame() if table is None else table.frame())
+    return frames
 
 
 def scan_many(struct_dir, struct_pssms, minscore, seq_file=None, seq_pssms=None, debug=False):
@@ -1773,11 +1875,13 @@ def _main(argv=None):
 
 def _run(args, seq_type, rank, precomputed=None):
     """One reference run (rnascan.py:490-567): backgrounds, motifs, scans, hits.tab on STDOUT.
-    `precomputed`: hits of this motif pair on the profile directory, already found by the batched scan."""
+    `precomputed`: hits of this motif pair on the profile directory, or of this motif on the FASTA input,
+    already found by the batched scan of its collection."""
     bg = None
     seq_file = struct_file = None
     seq_pssm = seq_hits = table = None
-    fusable = _world_size() == 1 and not args.testseq and not args.bgonly and not args.uniform_background
+    fusable = (_world_size() == 1 and not args.testseq and not args.bgonly and not args.uniform_background
+               and precomputed is None)
 
     if args.testseq:
         testseq_stack = args.testseq.split(",")[::-1]
@@ -1801,7 +1905,7 @@ def _run(args, seq_type, rank, precomputed=None):
             sys.exit()
         if fused is None:                 # else: background, motif and scan were done in one overlapped pass
             seq_pssm = load_motif(args.pfm_seq, args.pseudocount, rna, bg)
-            seq_hits = _scan_table(seq_file, seq_pssm, rna, args)
+            seq_hits = _scan_table(seq_file, seq_pssm, rna, args, precomputed if seq_type == "RNA" else None)
         table = seq_hits
 
     if seq_type in ["SS", "RNASS"]:
