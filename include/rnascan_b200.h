@@ -474,6 +474,26 @@ int rs_scan_onehot_many(int alphabet, const uint8_t *d_codes, int64_t n, int n_m
                         const double *tables, int table_stride_rows, double threshold, int64_t hit_capacity,
                         int32_t *d_hit_motif, int64_t *d_hit_pos, float *d_hit_f32, double *d_hit_f64,
                         uint64_t *d_bases, void *d_work, int64_t work_bytes, void *stream);
+/* ---- many (sequence, structure) motif pairs over two aligned symbol streams ---------------------------
+ * Replaces, for a collection of M pairs in the combined two-FASTA mode, the per-pair search() of both inputs
+ * (rnascan.py:263, run once per motif on each input) and the combine() inner join (rnascan.py:416-434).
+ * d_seq_codes (RNA layout) and d_struct_codes (structure layout) are n symbols each, separators at the same
+ * places.  Pair m has one width widths[m] (1..16, <= table_stride_rows <= 16) for its sequence table
+ * seq_tables[m][table_stride_rows][4] (ACGU) and its structure table struct_tables[m][table_stride_rows][7]
+ * (BEHLMRT).  A window is a hit when its float32 sequence score > threshold AND its float64 structure
+ * score > threshold; both scores are stored (d_hit_seq, d_hit_struct).  Everything else is
+ * rs_scan_onehot_many's contract: finite threshold, n < 2^32, 16-byte aligned code pointers, hits grouped by
+ * pair and in position order inside a pair, d_bases[M+1], re-run on overflow.  Per pair, positions and both
+ * scores are exactly rs_scan_pair_onehot's with that pair's two tables.                                   */
+int64_t rs_scan_pair_onehot_many_workspace_bytes(int64_t n, int n_motifs, int table_stride_rows);
+int rs_scan_pair_onehot_many(const uint8_t *d_seq_codes, const uint8_t *d_struct_codes, int64_t n,
+                             int n_motifs, const int *widths,
+                             const double *seq_tables,    /* [M][stride][4], ACGU   */
+                             const double *struct_tables, /* [M][stride][7], BEHLMRT */
+                             int table_stride_rows, double threshold, int64_t hit_capacity,
+                             int32_t *d_hit_motif, int64_t *d_hit_pos, float *d_hit_seq,
+                             double *d_hit_struct, uint64_t *d_bases, void *d_work, int64_t work_bytes,
+                             void *stream);
 
 #ifdef __cplusplus
 }

@@ -108,6 +108,9 @@ _SIGS = {
     "rs_scan_onehot_many_workspace_bytes": ([_int, _i64, _int, _int], _i64),
     "rs_scan_onehot_many": ([_int, _vp, _i64, _int, _vp, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64,
                              _vp], _int),
+    "rs_scan_pair_onehot_many_workspace_bytes": ([_i64, _int, _int], _i64),
+    "rs_scan_pair_onehot_many": ([_vp, _vp, _i64, _int, _vp, _vp, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _vp,
+                                  _vp, _i64, _vp], _int),
     "rs_scan_batched_shadow": ([_vp, _vp, _vp, _i64, _int, _vp, _vp, _vp, _int, _dbl, _dbl, _int, _i64, _vp, _vp,
                                 _vp, _vp, _vp, _vp, _vp, _i64, _vp], _int),
 }

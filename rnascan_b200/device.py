@@ -897,6 +897,64 @@ def scan_onehot_many(stream, tables, threshold, capacity=None):
         cap = total
 
 
+def scan_pair_onehot_many(seq_stream, struct_stream, seq_tables, struct_tables, threshold, capacity=None):
+    """Many (sequence, structure) motif pairs over an RNA stream and the structure stream that lines up with it,
+    in one call (rs_scan_pair_onehot_many).
+
+    seq_tables[m] (W_m, 4) in ACGU order and struct_tables[m] (W_m, 7) in BEHLMRT order share one width, 1..16;
+    the threshold is finite.  Returns (motif int32[], pos int64[], seq_scores float32[], struct_scores float64[],
+    bases int64[M+1]): pair m's slice bases[m] .. bases[m+1], in position order, is exactly what
+    scan_pair_onehot returns for that pair."""
+    if seq_stream.kind != "rna" or struct_stream.kind != "struct":
+        raise ValueError("scan_pair_onehot_many takes an RNA stream and a structure stream (kinds %r, %r)"
+                         % (seq_stream.kind, struct_stream.kind))
+    if seq_stream.n != struct_stream.n:
+        raise ValueError("sequence and structure streams differ in length")
+    M = len(seq_tables)
+    if M == 0 or len(struct_tables) != M:
+        raise ValueError("need as many structure tables as sequence tables (%d, %d), at least one"
+                         % (M, len(struct_tables)))
+    ts = [_table(t, 4) for t in seq_tables]
+    tq = [_table(t, 7) for t in struct_tables]
+    widths = np.array([t.shape[0] for t in ts], dtype=np.int32)
+    if any(a.shape[0] != b.shape[0] for a, b in zip(ts, tq)):
+        raise ValueError("sequence and structure motifs of a pair must have the same width")
+    if widths.max() > MANY_MAX_W:
+        raise ValueError("scan_pair_onehot_many takes motifs up to %d wide (%d found)" % (MANY_MAX_W, widths.max()))
+    stride = int(widths.max())
+    packed_s = np.zeros((M, stride, 4), np.float64)
+    packed_q = np.zeros((M, stride, 7), np.float64)
+    for m in range(M):
+        packed_s[m, :widths[m]] = ts[m]
+        packed_q[m, :widths[m]] = tq[m]
+    threshold = float(threshold)
+    if not np.isfinite(threshold):
+        raise ValueError("scan_pair_onehot_many needs a finite threshold")
+    dev = seq_stream.codes.device
+    n = seq_stream.n
+    work_bytes = int(lib.rs_scan_pair_onehot_many_workspace_bytes(n, M, stride))
+    if work_bytes < 0:
+        check(_lib.RS_ERR_INVALID)
+    work = torch.empty(max(work_bytes, 1), dtype=torch.uint8, device=dev)
+    bases = torch.zeros(M + 1, dtype=torch.int64, device=dev)
+    cap = int(capacity) if capacity else max(1 << 16, n // 16)
+    while True:
+        motif = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+        pos = torch.empty(max(cap, 1), dtype=torch.int64, device=dev)
+        seq = torch.empty(max(cap, 1), dtype=torch.float32, device=dev)
+        struct = torch.empty(max(cap, 1), dtype=torch.float64, device=dev)
+        check(lib.rs_scan_pair_onehot_many(_ptr(seq_stream.codes), _ptr(struct_stream.codes), n, M,
+                                           widths.ctypes.data, packed_s.ctypes.data, packed_q.ctypes.data, stride,
+                                           threshold, cap, _ptr(motif), _ptr(pos), _ptr(seq), _ptr(struct),
+                                           _ptr(bases), _ptr(work), work_bytes, _stream()))
+        b = bases.cpu().numpy()
+        total = int(b[-1])
+        if total <= cap:
+            return (motif[:total].cpu().numpy(), pos[:total].cpu().numpy(), seq[:total].cpu().numpy(),
+                    struct[:total].cpu().numpy(), b)
+        cap = total
+
+
 # --------------------------------------------------------------------------- host-buffer pipeline
 class _HitOverflow(Exception):
     def __init__(self, found):

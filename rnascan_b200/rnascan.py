@@ -379,7 +379,9 @@ class _Batch(object):
 
     ids/descriptions describe ALL records of the batch's input range; `record` maps each
     packed text to its record, `piece_start` is its offset inside that record and `own`
-    the number of leading window starts / symbols this rank owns (shard.plan_shards)."""
+    the number of leading window starts / symbols this rank owns (shard.plan_shards).
+    `counts`: the owned symbol counts (compute_background), taken once per batch."""
+    counts = None
 
     def __init__(self, ids, descriptions, texts, kind, record=None, piece_start=None, own=None,
                  full_texts=None):
@@ -1072,14 +1074,38 @@ def _fasta_many_hits(batches, kind, tables, minscore):
         n_records += len(batch.ids)
     empty = (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64),
              np.zeros(0, np.float32 if kind == "rna" else np.float64))
-    hits = _gather(parts or [empty])
+    return _by_motif(_gather(parts or [empty]), len(tables))
+
+
+def _by_motif(hits, n_motifs):
+    """Gathered (motif, rec, start0, scores...) columns -> one (rec, start0, scores...) tuple per motif, in record
+    order; None per motif on ranks other than 0."""
     if hits is None:
-        return [None] * len(tables)
-    motif, rec, start0, scores = hits
-    order = np.argsort(motif, kind="stable")          # rank order (= record order) within each motif
-    motif, rec, start0, scores = motif[order], rec[order], start0[order], scores[order]
-    cut = np.searchsorted(motif, np.arange(len(tables) + 1))
-    return [(rec[a:b], start0[a:b], scores[a:b]) for a, b in zip(cut[:-1], cut[1:])]
+        return [None] * n_motifs
+    order = np.argsort(hits[0], kind="stable")        # rank order (= record order) within each motif
+    cols = [c[order] for c in hits]
+    cut = np.searchsorted(cols[0], np.arange(n_motifs + 1))
+    return [tuple(c[a:b] for c in cols[1:]) for a, b in zip(cut[:-1], cut[1:])]
+
+
+def _pair_many_hits(seq_batches, struct_batches, seq_tables, struct_tables, minscore):
+    """Joint hits of every (sequence, structure) table pair on two FASTA inputs that line up (_lined_up) from one
+    device.scan_pair_onehot_many call per device batch: one (record index, 0-based start, sequence scores,
+    structure scores) tuple per pair, or None per pair on ranks other than 0; one _gather for the collection."""
+    from . import device
+    parts, n_records = [], 0
+    for sb, qb in zip(seq_batches, struct_batches):
+        with STATS.phase("scan_s"):
+            motif, pos, seq_sc, scores, _ = device.scan_pair_onehot_many(sb.stream, qb.stream, seq_tables,
+                                                                         struct_tables, minscore)
+        lengths = qb.stream.lengths
+        STATS.add("scored_positions", sum(int(np.maximum(lengths - t.shape[0] + 1, 0).sum()) for t in seq_tables))
+        keep, rec, start0 = qb.locate(pos)
+        parts.append((motif[keep], rec[keep] + n_records, start0[keep], seq_sc[keep], scores[keep]))
+        n_records += len(qb.ids)
+    empty = (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64), np.zeros(0, np.float32),
+             np.zeros(0, np.float64))
+    return _by_motif(_gather(parts or [empty]), len(seq_tables))
 
 
 def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, minscore):
@@ -1487,7 +1513,9 @@ def compute_background(fastas, alphabet, verbose=True):
     counts = np.zeros(8 if kind in ("rna", "struct") else len(kind.letters), dtype=np.int64)
     n_records = 0
     for batch in _cached_batches(fastas, alphabet):
-        counts += device.histogram(batch.stream).cpu().numpy() - batch.overlap_counts()
+        if batch.counts is None:
+            batch.counts = device.histogram(batch.stream).cpu().numpy() - batch.overlap_counts()
+        counts += batch.counts
         n_records += len(batch.ids)
     counts = _allreduce_counts(counts)
     return _background_from_counts(counts, n_records, alphabet, verbose)
@@ -1540,12 +1568,28 @@ def load_background(bg_file, uniform, *args):
 ###############################################################################
 # Main
 ###############################################################################
+def _lined_up(seq_batches, struct_batches):
+    """(sequence text, structure text, record offsets) when the two FASTA inputs of the combined mode can be
+    scanned together -- unique ids (duplicate ids join across records), the same ids in the same order and the
+    same whole-record lengths, so that every window lines up -- else None (the inputs are then scanned apart
+    and merged as the reference does)."""
+    ids = [i for b in seq_batches for i in b.ids]
+    if len(set(ids)) != len(ids) or [i for b in struct_batches for i in b.ids] != ids:
+        return None
+    seq_text, offsets = _record_text(seq_batches)
+    struct_text, struct_offsets = _record_text(struct_batches)
+    if len(struct_text) != len(seq_text) or not np.array_equal(struct_offsets, offsets):
+        return None
+    return seq_text, struct_text, offsets
+
+
 def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, precomputed=None):
     """The table of the combined mode (rnascan.py:416-434) on top of `seq_hits`, the sequence scan's table; None
     on ranks other than 0 under torchrun.  The structure side is scanned ON THE DEVICE only where the sequence
     score also passes (the inner join keeps nothing else): one fused launch instead of a second full scan +
     merge.  Where the two inputs cannot be scanned together (-t, different motif widths, duplicate ids, inputs
-    that do not line up) the structure input is scanned on its own and merged as the reference does."""
+    that do not line up) the structure input is scanned on its own and merged as the reference does.
+    `precomputed`: the pair's hits on the profile directory, or its _PairHits on the structure FASTA input."""
     from . import device
     _, seq_pm = _first_motif(seq_pssm)
     motif_id, pm = _first_motif(struct_pssm)
@@ -1565,23 +1609,26 @@ def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args,
         return _scan_profile_dir(struct_file, struct_pssm, args.minscore, args.debug, seq_batches, seq_pm, seq_hits,
                                  getattr(args, "pack", False), precomputed)
     struct_batches = _cached_batches(struct_file, structure)
-    seq_text, offsets = _record_text(seq_batches)
-    struct_text, struct_offsets = _record_text(struct_batches)
-    if ([i for b in struct_batches for i in b.ids] != ids or len(struct_text) != len(seq_text)
-            or not np.array_equal(struct_offsets, offsets)):
-        return merged()                   # records of different lengths: windows do not line up
+    lined = _lined_up(seq_batches, struct_batches)
+    if lined is None:
+        return merged()
+    seq_text, struct_text, offsets = lined
     eprint("Scanning sequences ")
-    ts, tq = _table_for(seq_pm, "rna"), _table_for(pm, "struct")
-    parts, n_records = [], 0
-    for sb, qb in zip(seq_batches, struct_batches):
-        with STATS.phase("scan_s"):
-            pos, seq_sc, scores = device.scan_pair_onehot(sb.stream, qb.stream, ts, tq, args.minscore)
-        STATS.add("scored_positions", int(np.maximum(qb.stream.lengths - width + 1, 0).sum()))
-        keep, rec, start0 = qb.locate(pos)
-        parts.append((rec[keep] + n_records, start0[keep], seq_sc[keep], scores[keep]))
-        n_records += len(qb.ids)
-    eprint("Processed %d sequences" % n_records)
-    hits = _gather(parts or [(np.zeros(0, np.int64),) * 4])
+    if precomputed is not None:
+        eprint("Processed %d sequences" % sum(len(qb.ids) for qb in struct_batches))
+        hits = precomputed.joint
+    else:
+        ts, tq = _table_for(seq_pm, "rna"), _table_for(pm, "struct")
+        parts, n_records = [], 0
+        for sb, qb in zip(seq_batches, struct_batches):
+            with STATS.phase("scan_s"):
+                pos, seq_sc, scores = device.scan_pair_onehot(sb.stream, qb.stream, ts, tq, args.minscore)
+            STATS.add("scored_positions", int(np.maximum(qb.stream.lengths - width + 1, 0).sum()))
+            keep, rec, start0 = qb.locate(pos)
+            parts.append((rec[keep] + n_records, start0[keep], seq_sc[keep], scores[keep]))
+            n_records += len(qb.ids)
+        eprint("Processed %d sequences" % n_records)
+        hits = _gather(parts or [(np.zeros(0, np.int64),) * 4])
     if hits is None:
         return None
     rec, start0, seq_scores, scores = hits
@@ -1627,7 +1674,8 @@ def _run_multi(args, seq_type, rank, pairs):
     try:
         pre = None
         if not args.bgonly:
-            pre = _batched_profile_hits(args, seq_type, pairs) or _batched_fasta_hits(args, seq_type, pairs)
+            pre = (_batched_profile_hits(args, seq_type, pairs) or _batched_fasta_hits(args, seq_type, pairs)
+                   or _batched_pair_hits(args, seq_type, pairs))
         for k, (seq_pfm, struct_pfm) in enumerate(pairs):
             one = copy.copy(args)
             one.pfm_seq, one.pfm_struct = seq_pfm, struct_pfm
@@ -1764,6 +1812,79 @@ def scan_many_fasta(fasta_file, pssms, alphabet, minscore):
     return frames
 
 
+class _PairHits(object):
+    """One motif pair's hits from the batched scans of its collection in the combined mode over two FASTA inputs:
+    `seq`, the sequence motif's _FastaHits, and `joint`, the pair's (record index, 0-based start, sequence scores,
+    structure scores) -- None on ranks other than 0 and for a pair whose two widths differ."""
+
+    def __init__(self, seq, joint):
+        self.seq, self.joint = seq, joint
+
+
+def _pair_on_device(seq_batches, struct_batches):
+    """True when the streams of both inputs are resident on a CUDA device (what the pair kernel reads)."""
+    return all(b.stream.codes.is_cuda for b in list(seq_batches) + list(struct_batches))
+
+
+def _batched_pair_hits(args, seq_type, pairs):
+    """Hits of every motif pair of a collection in the combined mode over two FASTA inputs (RNASS): the sequence
+    motifs' hits from device.scan_onehot_many and the joint hits of the equal-width pairs from
+    device.scan_pair_onehot_many, one call of each per device batch.  A list of _PairHits per pair, or None when
+    this run does not have that shape (the per-pair scans then run one after the other).  Both backgrounds are
+    taken once, quietly; every _run still prints its own messages."""
+    if seq_type != "RNASS" or args.testseq or args.bgonly or len(pairs) < MULTI_FASTA_MIN_MOTIFS:
+        return None
+    if not np.isfinite(args.minscore) or len(args.fastafiles or []) < 2:
+        return None
+    seq_file, struct_file = args.fastafiles[:2]
+    if os.path.isdir(seq_file) or os.path.isdir(struct_file):
+        return None
+    rna, structure = IUPAC.IUPACUnambiguousRNA(), ContextualSecondaryStructure()
+    seq_batches = _cached_batches(seq_file, rna)
+    struct_batches = _cached_batches(struct_file, structure)
+    if not _pair_on_device(seq_batches, struct_batches) or len(seq_batches) != len(struct_batches):
+        return None
+    if _lined_up(seq_batches, struct_batches) is None:
+        return None
+    try:
+        bg_seq = _quiet(load_background, args.bg_seq, args.uniform_background, seq_file, rna, False)
+        bg_struct = _quiet(load_background, args.bg_struct, args.uniform_background, struct_file, structure, False)
+        seq_pssms = [_quiet(load_motif, p_, args.pseudocount, rna, bg_seq) for p_, _ in pairs]
+        struct_pssms = [_quiet(load_motif, q, args.pseudocount, structure, bg_struct) for _, q in pairs]
+    except Exception:
+        return None                       # the per-pair run reports what is wrong
+    ts = [_table_for(_first_motif(p)[1], "rna") for p in seq_pssms]
+    tq = [_table_for(_first_motif(p)[1], "struct") for p in struct_pssms]
+    same = [k for k in range(len(ts)) if ts[k].shape[0] == tq[k].shape[0]]
+    if max(t.shape[0] for t in ts + tq) > 16:
+        return None
+    seq_hits = _fasta_many_hits(seq_batches, "rna", ts, args.minscore)
+    joint = dict(zip(same, _pair_many_hits(seq_batches, struct_batches, [ts[k] for k in same],
+                                           [tq[k] for k in same], args.minscore))) if same else {}
+    STATS.notes["batched_motifs"] = len(pairs)
+    return [_PairHits(_FastaHits(h), joint.get(k)) for k, h in enumerate(seq_hits)]
+
+
+def scan_many_combined(seq_file, struct_file, seq_pssms, struct_pssms, minscore):
+    """The combined mode over two FASTA files for MANY motif pairs.
+
+    seq_pssms / struct_pssms: lists of ``{motif_id: PSSM}`` as load_motif returns them (RNA and
+    ContextualSecondaryStructure alphabets), paired by position.  Returns one DataFrame per pair, equal to
+    combine(scan_main(seq_file, seq_pssm, rna, None, args), scan_main(struct_file, struct_pssm, structure, None,
+    args)) for that pair -- columns, dtypes and values -- (empty frames on ranks other than 0 under torchrun).
+    Each input is scanned with all its motifs in one batched pass per device batch (scan_many_fasta) and the two
+    frames of a pair are joined as the reference joins them: the structure frame's dtypes depend on which records
+    have a structure-only hit, which the joint windows alone do not tell.  Any widths and any two inputs are taken;
+    a threshold of -inf and motifs wider than 16 are scanned one motif at a time."""
+    if len(seq_pssms) != len(struct_pssms):
+        raise ValueError("sequence and structure motif lists differ in length")
+    seq = scan_many_fasta(seq_file, seq_pssms, IUPAC.IUPACUnambiguousRNA(), minscore)
+    struct = scan_many_fasta(struct_file, struct_pssms, ContextualSecondaryStructure(), minscore)
+    if _rank() != 0:
+        return [pd.DataFrame() for _ in seq_pssms]
+    return [combine(a, b) for a, b in zip(seq, struct)]
+
+
 def scan_many(struct_dir, struct_pssms, minscore, seq_file=None, seq_pssms=None, debug=False):
     """Scan a directory of averaged profiles with MANY motifs in one batched pass (BASELINE config 5).
 
@@ -1875,8 +1996,8 @@ def _main(argv=None):
 
 def _run(args, seq_type, rank, precomputed=None):
     """One reference run (rnascan.py:490-567): backgrounds, motifs, scans, hits.tab on STDOUT.
-    `precomputed`: hits of this motif pair on the profile directory, or of this motif on the FASTA input,
-    already found by the batched scan of its collection."""
+    `precomputed`: hits of this motif pair on the profile directory, of this motif on the FASTA input, or of this
+    pair on the two FASTA inputs (_PairHits), already found by the batched scans of its collection."""
     bg = None
     seq_file = struct_file = None
     seq_pssm = seq_hits = table = None
@@ -1905,7 +2026,9 @@ def _run(args, seq_type, rank, precomputed=None):
             sys.exit()
         if fused is None:                 # else: background, motif and scan were done in one overlapped pass
             seq_pssm = load_motif(args.pfm_seq, args.pseudocount, rna, bg)
-            seq_hits = _scan_table(seq_file, seq_pssm, rna, args, precomputed if seq_type == "RNA" else None)
+            seq_pre = precomputed.seq if isinstance(precomputed, _PairHits) else (
+                precomputed if seq_type == "RNA" else None)
+            seq_hits = _scan_table(seq_file, seq_pssm, rna, args, seq_pre)
         table = seq_hits
 
     if seq_type in ["SS", "RNASS"]:
