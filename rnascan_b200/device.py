@@ -792,20 +792,13 @@ def scan_batched(stream, profile, seq_tables, struct_tables, threshold, capacity
         raise ValueError("no motifs")
     if seq_tables is not None and len(seq_tables) != M:
         raise ValueError("sequence and structure motif lists differ in length")
-    tq = [_table(t, 7) for t in struct_tables]
-    widths = np.array([t.shape[0] for t in tq], dtype=np.int32)
-    stride = int(widths.max())
-    qs = np.zeros((M, stride, 7), np.float64)
-    for m, t in enumerate(tq):
-        qs[m, :t.shape[0]] = t
+    widths, qs, stride = _pack_tables(struct_tables, 7)
     ss = None
     if seq_tables is not None:
-        ss = np.zeros((M, stride, 4), np.float64)
-        for m, t in enumerate(seq_tables):
-            t = _table(t, 4)
-            if t.shape[0] != widths[m]:
-                raise ValueError("motif %d: sequence and structure widths differ" % m)
-            ss[m, :t.shape[0]] = t
+        seq_widths, ss, _ = _pack_tables(seq_tables, 4)
+        differ = np.nonzero(seq_widths != widths)[0]
+        if len(differ):
+            raise ValueError("motif %d: sequence and structure widths differ" % differ[0])
     if stream.n != profile.n:
         raise ValueError("symbol stream and profile stream differ in length")
     threshold = float(threshold)
@@ -850,6 +843,36 @@ def scan_batched(stream, profile, seq_tables, struct_tables, threshold, capacity
 MANY_MAX_W = 16                 # widest motif scan_onehot_many takes
 
 
+def _pack_tables(tables, A):
+    """(widths int32[M], packed, stride): the checked (W_m, A) tables zero-padded into one (M, stride, A) float64
+    array, stride = the widest W_m, as the grouped scans read them."""
+    ts = [_table(t, A) for t in tables]
+    widths = np.array([t.shape[0] for t in ts], dtype=np.int32)
+    stride = int(widths.max())
+    packed = np.zeros((len(ts), stride, A), np.float64)
+    for m, t in enumerate(ts):
+        packed[m, :t.shape[0]] = t
+    return widths, packed, stride
+
+
+def _run_many(dev, M, work_bytes, cap, score_dtypes, launch):
+    """Run `launch(cap, work, bases, motif, pos, *scores)` of a grouped one-hot scan with output buffers for `cap`
+    hits (one score buffer per dtype of `score_dtypes`); re-run with the exact capacity if the hits overflowed.
+    Returns (motif, pos, *scores, bases) on the host."""
+    if work_bytes < 0:
+        check(_lib.RS_ERR_INVALID)
+    work = torch.empty(max(work_bytes, 1), dtype=torch.uint8, device=dev)
+    bases = torch.zeros(M + 1, dtype=torch.int64, device=dev)
+    while True:
+        out = [torch.empty(max(cap, 1), dtype=dt, device=dev) for dt in (torch.int32, torch.int64) + score_dtypes]
+        launch(cap, work, bases, *out)
+        b = bases.cpu().numpy()
+        total = int(b[-1])
+        if total <= cap:
+            return tuple(t[:total].cpu().numpy() for t in out) + (b,)
+        cap = total
+
+
 def scan_onehot_many(stream, tables, threshold, capacity=None):
     """Many one-hot PSSMs over one FASTA symbol stream in one call (rs_scan_onehot_many).
 
@@ -863,38 +886,21 @@ def scan_onehot_many(stream, tables, threshold, capacity=None):
     M = len(tables)
     if M == 0:
         raise ValueError("no motifs")
-    ts = [_table(t, A) for t in tables]
-    widths = np.array([t.shape[0] for t in ts], dtype=np.int32)
+    widths, packed, stride = _pack_tables(tables, A)
     if widths.max() > MANY_MAX_W:
         raise ValueError("scan_onehot_many takes motifs up to %d wide (%d found)" % (MANY_MAX_W, widths.max()))
-    stride = int(widths.max())
-    packed = np.zeros((M, stride, A), np.float64)
-    for m, t in enumerate(ts):
-        packed[m, :t.shape[0]] = t
     threshold = float(threshold)
     if not np.isfinite(threshold):
         raise ValueError("scan_onehot_many needs a finite threshold")
-    dev = stream.codes.device
     work_bytes = int(lib.rs_scan_onehot_many_workspace_bytes(A, stream.n, M, stride))
-    if work_bytes < 0:
-        check(_lib.RS_ERR_INVALID)
-    work = torch.empty(max(work_bytes, 1), dtype=torch.uint8, device=dev)
-    bases = torch.zeros(M + 1, dtype=torch.int64, device=dev)
-    sdt = torch.float32 if A == 4 else torch.float64
-    cap = int(capacity) if capacity else max(1 << 16, stream.n // 16)
-    while True:
-        motif = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
-        pos = torch.empty(max(cap, 1), dtype=torch.int64, device=dev)
-        scores = torch.empty(max(cap, 1), dtype=sdt, device=dev)
+
+    def launch(cap, work, bases, motif, pos, scores):
         check(lib.rs_scan_onehot_many(A, _ptr(stream.codes), stream.n, M, widths.ctypes.data, packed.ctypes.data,
                                       stride, threshold, cap, _ptr(motif), _ptr(pos),
                                       _ptr(scores) if A == 4 else 0, 0 if A == 4 else _ptr(scores), _ptr(bases),
                                       _ptr(work), work_bytes, _stream()))
-        b = bases.cpu().numpy()
-        total = int(b[-1])
-        if total <= cap:
-            return motif[:total].cpu().numpy(), pos[:total].cpu().numpy(), scores[:total].cpu().numpy(), b
-        cap = total
+    cap = int(capacity) if capacity else max(1 << 16, stream.n // 16)
+    return _run_many(stream.codes.device, M, work_bytes, cap, (torch.float32 if A == 4 else torch.float64,), launch)
 
 
 def scan_pair_onehot_many(seq_stream, struct_stream, seq_tables, struct_tables, threshold, capacity=None):
@@ -914,45 +920,25 @@ def scan_pair_onehot_many(seq_stream, struct_stream, seq_tables, struct_tables, 
     if M == 0 or len(struct_tables) != M:
         raise ValueError("need as many structure tables as sequence tables (%d, %d), at least one"
                          % (M, len(struct_tables)))
-    ts = [_table(t, 4) for t in seq_tables]
-    tq = [_table(t, 7) for t in struct_tables]
-    widths = np.array([t.shape[0] for t in ts], dtype=np.int32)
-    if any(a.shape[0] != b.shape[0] for a, b in zip(ts, tq)):
+    widths, packed_s, stride = _pack_tables(seq_tables, 4)
+    struct_widths, packed_q, _ = _pack_tables(struct_tables, 7)
+    if not np.array_equal(widths, struct_widths):
         raise ValueError("sequence and structure motifs of a pair must have the same width")
     if widths.max() > MANY_MAX_W:
         raise ValueError("scan_pair_onehot_many takes motifs up to %d wide (%d found)" % (MANY_MAX_W, widths.max()))
-    stride = int(widths.max())
-    packed_s = np.zeros((M, stride, 4), np.float64)
-    packed_q = np.zeros((M, stride, 7), np.float64)
-    for m in range(M):
-        packed_s[m, :widths[m]] = ts[m]
-        packed_q[m, :widths[m]] = tq[m]
     threshold = float(threshold)
     if not np.isfinite(threshold):
         raise ValueError("scan_pair_onehot_many needs a finite threshold")
-    dev = seq_stream.codes.device
     n = seq_stream.n
     work_bytes = int(lib.rs_scan_pair_onehot_many_workspace_bytes(n, M, stride))
-    if work_bytes < 0:
-        check(_lib.RS_ERR_INVALID)
-    work = torch.empty(max(work_bytes, 1), dtype=torch.uint8, device=dev)
-    bases = torch.zeros(M + 1, dtype=torch.int64, device=dev)
-    cap = int(capacity) if capacity else max(1 << 16, n // 16)
-    while True:
-        motif = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
-        pos = torch.empty(max(cap, 1), dtype=torch.int64, device=dev)
-        seq = torch.empty(max(cap, 1), dtype=torch.float32, device=dev)
-        struct = torch.empty(max(cap, 1), dtype=torch.float64, device=dev)
+
+    def launch(cap, work, bases, motif, pos, seq, struct):
         check(lib.rs_scan_pair_onehot_many(_ptr(seq_stream.codes), _ptr(struct_stream.codes), n, M,
                                            widths.ctypes.data, packed_s.ctypes.data, packed_q.ctypes.data, stride,
                                            threshold, cap, _ptr(motif), _ptr(pos), _ptr(seq), _ptr(struct),
                                            _ptr(bases), _ptr(work), work_bytes, _stream()))
-        b = bases.cpu().numpy()
-        total = int(b[-1])
-        if total <= cap:
-            return (motif[:total].cpu().numpy(), pos[:total].cpu().numpy(), seq[:total].cpu().numpy(),
-                    struct[:total].cpu().numpy(), b)
-        cap = total
+    cap = int(capacity) if capacity else max(1 << 16, n // 16)
+    return _run_many(seq_stream.codes.device, M, work_bytes, cap, (torch.float32, torch.float64), launch)
 
 
 # --------------------------------------------------------------------------- host-buffer pipeline

@@ -840,23 +840,37 @@ def _assemble_fasta_frame(n_records, rec, ids, descriptions, motif_id, start0, w
     return frame
 
 
-def _scan_batch(batch, pm, kind, minscore):
-    """(record index, 0-based start, scores) of all hits in a packed batch."""
+def _scan_batch(batch, table, kind, minscore):
+    """(stream positions, scores) of one motif's hits in a packed batch."""
     from . import device
-    table = _table_for(pm, kind)
-    with STATS.phase("scan_s"):
-        if kind == "rna":
-            pos, scores = device.scan_seq(batch.stream, table, minscore)
-        elif kind != "struct":
-            pos, scores = device.scan_alpha(batch.stream, table, minscore)
-        else:
-            every = None
-            if minscore == float("-inf"):               # every position: the device rounds, 4 B per window come back
-                every = device.scan_struct_every_position(batch.stream, table)
-            pos, scores = every if every is not None else device.scan_struct_onehot(batch.stream, table, minscore)
-    STATS.add("scored_positions", int(np.maximum(batch.stream.lengths - table.shape[0] + 1, 0).sum()))
-    keep, rec, start0 = batch.locate(pos)
-    return rec[keep], start0[keep], scores[keep]
+    if kind == "rna":
+        return device.scan_seq(batch.stream, table, minscore)
+    if kind != "struct":
+        return device.scan_alpha(batch.stream, table, minscore)
+    every = None
+    if minscore == float("-inf"):                       # every position: the device rounds, 4 B per window come back
+        every = device.scan_struct_every_position(batch.stream, table)
+    return every if every is not None else device.scan_struct_onehot(batch.stream, table, minscore)
+
+
+def _scan_batches(batches, scan, widths, dtypes):
+    """The hits of `scan` over the device batches of an input, gathered (_gather): the columns (record index over
+    all batches, 0-based start, column...), None on ranks other than 0 under torchrun.  A device batch is a
+    _Batch or a lined-up (sequence, structure) pair of them, located by its structure batch; `scan(batch)`
+    returns (stream positions, column...) of its hits, `dtypes` are the dtypes of those columns and `widths` the
+    widths of the motifs it scores."""
+    parts, n_records = [], 0
+    for batch in batches:
+        where = batch[1] if isinstance(batch, tuple) else batch
+        with STATS.phase("scan_s"):
+            pos, *columns = scan(batch)
+        lengths = where.stream.lengths
+        STATS.add("scored_positions", sum(int(np.maximum(lengths - w + 1, 0).sum()) for w in widths))
+        keep, rec, start0 = where.locate(pos)
+        parts.append((rec[keep] + n_records, start0[keep]) + tuple(c[keep] for c in columns))
+        n_records += len(where.ids)
+    empty = (np.zeros(0, np.int64), np.zeros(0, np.int64)) + tuple(np.zeros(0, dt) for dt in dtypes)
+    return _gather(parts or [empty])
 
 
 def _gather(parts):
@@ -1028,31 +1042,26 @@ def _emit(out, text):
         out.write(text)
 
 
-def _scan_fasta_hits(fasta_file, pssm, alphabet, minscore, precomputed=None):
+def _scan_fasta_hits(fasta_file, pssm, alphabet, minscore, found=None):
     """All records of a FASTA input in one (or a few) kernel launches, as a _HitTable (None on ranks other than
-    0 under torchrun).  `precomputed`: this motif's hits from the batched scan of its motif collection
+    0 under torchrun).  `found`: this motif's _Found hits from the batched scan of its motif collection
     (_batched_fasta_hits); the input is then not scanned again."""
     eprint("Scanning sequences ")
     motif_id, pm = _first_motif(pssm)
     kind = _kind_of(alphabet)
     batches = _cached_batches(fasta_file, alphabet)
-    if precomputed is not None:
-        eprint("Processed %d sequences" % sum(len(b.ids) for b in batches))
-        hits = precomputed.hits
-    else:
-        parts, n_records = [], 0
-        for batch in batches:
-            rec, start0, scores = _scan_batch(batch, pm, kind, minscore)
-            parts.append((rec + n_records, start0, scores))
-            n_records += len(batch.ids)
-        eprint("Processed %d sequences" % n_records)
-        hits = _gather(parts or [(np.zeros(0, np.int64),) * 3])
-    return None if hits is None else _fasta_table(motif_id, pm.length, kind, batches, *hits)
+    if found is None:
+        table = _table_for(pm, kind)
+        found = _Found(_scan_batches(batches, lambda batch: _scan_batch(batch, table, kind, minscore),
+                                     [table.shape[0]], [np.float64]))
+    eprint("Processed %d sequences" % sum(len(b.ids) for b in batches))
+    return None if found.hits is None else _fasta_table(motif_id, pm.length, kind, batches, *found.hits)
 
 
-class _FastaHits(object):
-    """One motif's hits from the batched scan of a FASTA input: (record index, 0-based start, scores) on rank 0,
-    None on the other ranks under torchrun."""
+class _Found(object):
+    """One motif's (pair's) hits from a batched scan, in record coordinates: the columns (record index, 0-based
+    start, scores) -- (record index, 0-based start, sequence scores, structure scores) for joint hits -- on rank
+    0, None on the other ranks under torchrun."""
 
     def __init__(self, hits):
         self.hits = hits
@@ -1063,29 +1072,23 @@ def _fasta_many_hits(batches, kind, tables, minscore):
     (record index, 0-based start, scores) tuple per table, or None per table on ranks other than 0.  Under
     torchrun each rank scans its own pieces and the whole collection makes ONE _gather."""
     from . import device
-    parts, n_records = [], 0
-    for batch in batches:
-        with STATS.phase("scan_s"):
-            motif, pos, scores, _ = device.scan_onehot_many(batch.stream, tables, minscore)
-        lengths = batch.stream.lengths
-        STATS.add("scored_positions", sum(int(np.maximum(lengths - t.shape[0] + 1, 0).sum()) for t in tables))
-        keep, rec, start0 = batch.locate(pos)
-        parts.append((motif[keep], rec[keep] + n_records, start0[keep], scores[keep]))
-        n_records += len(batch.ids)
-    empty = (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64),
-             np.zeros(0, np.float32 if kind == "rna" else np.float64))
-    return _by_motif(_gather(parts or [empty]), len(tables))
+
+    def scan(batch):
+        motif, pos, scores, _ = device.scan_onehot_many(batch.stream, tables, minscore)
+        return pos, scores, motif
+    dtypes = [np.float32 if kind == "rna" else np.float64, np.int32]
+    return _by_motif(_scan_batches(batches, scan, [t.shape[0] for t in tables], dtypes), len(tables))
 
 
 def _by_motif(hits, n_motifs):
-    """Gathered (motif, rec, start0, scores...) columns -> one (rec, start0, scores...) tuple per motif, in record
+    """Gathered (rec, start0, scores..., motif) columns -> one (rec, start0, scores...) tuple per motif, in record
     order; None per motif on ranks other than 0."""
     if hits is None:
         return [None] * n_motifs
-    order = np.argsort(hits[0], kind="stable")        # rank order (= record order) within each motif
+    order = np.argsort(hits[-1], kind="stable")       # rank order (= record order) within each motif
     cols = [c[order] for c in hits]
-    cut = np.searchsorted(cols[0], np.arange(n_motifs + 1))
-    return [tuple(c[a:b] for c in cols[1:]) for a, b in zip(cut[:-1], cut[1:])]
+    cut = np.searchsorted(cols[-1], np.arange(n_motifs + 1))
+    return [tuple(c[a:b] for c in cols[:-1]) for a, b in zip(cut[:-1], cut[1:])]
 
 
 def _pair_many_hits(seq_batches, struct_batches, seq_tables, struct_tables, minscore):
@@ -1093,19 +1096,14 @@ def _pair_many_hits(seq_batches, struct_batches, seq_tables, struct_tables, mins
     device.scan_pair_onehot_many call per device batch: one (record index, 0-based start, sequence scores,
     structure scores) tuple per pair, or None per pair on ranks other than 0; one _gather for the collection."""
     from . import device
-    parts, n_records = [], 0
-    for sb, qb in zip(seq_batches, struct_batches):
-        with STATS.phase("scan_s"):
-            motif, pos, seq_sc, scores, _ = device.scan_pair_onehot_many(sb.stream, qb.stream, seq_tables,
-                                                                         struct_tables, minscore)
-        lengths = qb.stream.lengths
-        STATS.add("scored_positions", sum(int(np.maximum(lengths - t.shape[0] + 1, 0).sum()) for t in seq_tables))
-        keep, rec, start0 = qb.locate(pos)
-        parts.append((motif[keep], rec[keep] + n_records, start0[keep], seq_sc[keep], scores[keep]))
-        n_records += len(qb.ids)
-    empty = (np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(0, np.int64), np.zeros(0, np.float32),
-             np.zeros(0, np.float64))
-    return _by_motif(_gather(parts or [empty]), len(seq_tables))
+
+    def scan(pair):
+        motif, pos, seq_sc, scores, _ = device.scan_pair_onehot_many(pair[0].stream, pair[1].stream, seq_tables,
+                                                                     struct_tables, minscore)
+        return pos, seq_sc, scores, motif
+    hits = _scan_batches(list(zip(seq_batches, struct_batches)), scan, [t.shape[0] for t in seq_tables],
+                         [np.float32, np.float64, np.int32])
+    return _by_motif(hits, len(seq_tables))
 
 
 def _scan_fasta_hits_computed_bg(fasta_file, pfm_file, pseudocount, alphabet, minscore):
@@ -1301,15 +1299,15 @@ def _profile_dir_streams(directory, debug, seq_batches, write_pack):
 
 
 def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm=None, seq_hits=None,
-                      write_pack=False, precomputed=None):
+                      write_pack=False, found=None):
     """All ``structure.<id>.txt`` profiles of a directory in one pass (rnascan.py:348-375), as a _HitTable (None
     on ranks other than 0 under torchrun).
     With `seq_batches`/`seq_pm` (combined mode) the sequence PSSM is evaluated on the same windows and only
     those passing BOTH thresholds come back: the rows of the combined hits.tab, whose sequence side is the
     table `seq_hits` of the sequence scan.  The float64 rows stay on the host: the device filters a float32
     shadow or the pack's 8-byte quantised rows and re-scores the few windows near the threshold from the exact
-    rows (device.scan_profile_host).  `precomputed`: the hits of this motif (pair) found by the batched scan of
-    a motif collection (_batched_profile_hits).  Under torchrun every rank takes a contiguous range of files
+    rows (device.scan_profile_host).  `found`: the _Found hits of this motif (pair) from the batched scan of a
+    motif collection (_batched_profile_hits).  Under torchrun every rank takes a contiguous range of files
     balanced by size and rank 0 gathers the hits."""
     from . import device, shard
     eprint("Scanning averaged secondary structures ")
@@ -1321,28 +1319,25 @@ def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm
                                                                                 write_pack)
     n_files = len(all_names)
     seq = None if seq_batches is None else _table_for(seq_pm, "rna")
-    if precomputed is not None:           # this motif pair was scanned in the collection's batched pass
-        pos, seq_scores, scores = precomputed
-        STATS.add("scored_positions", int(np.maximum(lengths - width + 1, 0).sum()))
-        rec = np.searchsorted(offsets, pos, side="right") - 1
-        start0 = pos - offsets[rec]
-    elif len(codes):
-        with STATS.phase("scan_s"):
-            pos, seq_scores, scores, scanner = device.scan_profile_host(codes, hp, seq, tq, minscore,
-                                                                        return_scanner=True)
-        STATS.add("scored_positions", int(np.maximum(lengths - width + 1, 0).sum()))
-        if scanner is not None:
-            STATS.notes["profile_filter_form"] = scanner.form
-            STATS.add("h2d_bytes", scanner.h2d_bytes)
-            STATS.add("candidates", scanner.n_candidates)
-        rec = np.searchsorted(offsets, pos, side="right") - 1
-        start0 = pos - offsets[rec]
+    STATS.add("scored_positions", int(np.maximum(lengths - width + 1, 0).sum()))
+    if found is not None:                 # this motif (pair) was scanned in the collection's batched pass
+        hits = found.hits
     else:
         rec = start0 = np.zeros(0, np.int64)
-        scores = np.zeros(0, np.float64)
-        seq_scores = np.zeros(0, np.float32)
-    first = all_names.index(names[0]) if names else 0          # this rank's files are a contiguous range
-    hits = _gather([(rec + first, start0, np.asarray(scores, np.float64)) + (() if seq is None else (seq_scores,))])
+        scores, seq_scores = np.zeros(0, np.float64), np.zeros(0, np.float32)
+        if len(codes):
+            with STATS.phase("scan_s"):
+                pos, seq_scores, scores, scanner = device.scan_profile_host(codes, hp, seq, tq, minscore,
+                                                                            return_scanner=True)
+            if scanner is not None:
+                STATS.notes["profile_filter_form"] = scanner.form
+                STATS.add("h2d_bytes", scanner.h2d_bytes)
+                STATS.add("candidates", scanner.n_candidates)
+            rec = np.searchsorted(offsets, pos, side="right") - 1
+            start0 = pos - offsets[rec]
+        first = all_names.index(names[0]) if names else 0      # this rank's files are a contiguous range
+        hits = _gather([(rec + first, start0) + (() if seq is None else (seq_scores,))
+                        + (np.asarray(scores, np.float64),)])
     # Combined mode without a single joint hit: the reference's merge still needs the STRUCTURE frame's columns,
     # which exist iff some window passes the structure threshold on its own (else its merge raises KeyError, and
     # so does ours): one structure-only pass settles it -- only in this corner, on every rank when sharded.
@@ -1353,12 +1348,12 @@ def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm
             need = shard.broadcast_object(need)
         if need:
             local = bool(len(codes)) and len(device.scan_profile_host(codes, hp, None, tq, minscore)[0]) > 0
-            found = shard.gather_objects(local) if size > 1 else [local]
-            any_struct_hits = bool(found and any(found))
+            ranks = shard.gather_objects(local) if size > 1 else [local]
+            any_struct_hits = bool(ranks and any(ranks))
     eprint("Processed %d sequences" % n_files)
     if hits is None:                      # only rank 0 prints
         return None
-    rec, start0, scores = hits[:3]
+    rec, start0, scores = hits[0], hits[1], hits[-1]
     if seq is None:
         frame = lambda: _averaged_dir_frame(all_names, rec, motif_id, start0, width, scores)
         shape = _dir_frame_shape(np.bincount(rec, minlength=n_files))
@@ -1389,7 +1384,7 @@ def _scan_profile_dir(directory, pssm, minscore, debug, seq_batches=None, seq_pm
     order = np.lexsort((start0[keep], seq_rec[keep]))
     seq_rec, seq_start0 = seq_rec[keep][order], start0[keep][order]
     return _HitTable(frame, seq_rec, seq_start0, seq_hits.ids, seq_hits.descs, seq_hits.motif, width, text,
-                     text_offsets[seq_rec] + seq_start0, seq_hits.kind, hits[3][keep][order], motif_id, None, 3,
+                     text_offsets[seq_rec] + seq_start0, seq_hits.kind, hits[2][keep][order], motif_id, None, 3,
                      scores[keep][order])
 
 
@@ -1463,8 +1458,9 @@ def scan_main(fasta_file, pssm, alphabet, bg, args):
     return pd.DataFrame() if table is None else table.frame()
 
 
-def _scan_table(fasta_file, pssm, alphabet, args, precomputed=None):
-    """scan_main's scan as a _HitTable (None on ranks other than 0 under torchrun)."""
+def _scan_table(fasta_file, pssm, alphabet, args, found=None):
+    """scan_main's scan as a _HitTable (None on ranks other than 0 under torchrun); `found`: the _Found hits of
+    this motif from the batched scan of its collection."""
     if _seq.is_seqrecord(fasta_file):
         final = scan_all(fasta_file, pssm, alphabet, args.minscore)
         _add_sequence_id(final, "testseq", "")
@@ -1474,8 +1470,8 @@ def _scan_table(fasta_file, pssm, alphabet, args, precomputed=None):
         return _HitTable(lambda: final)
     if os.path.isdir(fasta_file):
         return _scan_profile_dir(fasta_file, pssm, args.minscore, args.debug, write_pack=getattr(args, "pack", False),
-                                 precomputed=precomputed)
-    return _scan_fasta_hits(fasta_file, pssm, alphabet, args.minscore, precomputed)
+                                 found=found)
+    return _scan_fasta_hits(fasta_file, pssm, alphabet, args.minscore, found)
 
 
 def combine(seq_results, struct_results):
@@ -1568,13 +1564,18 @@ def load_background(bg_file, uniform, *args):
 ###############################################################################
 # Main
 ###############################################################################
+def _unique_ids(batches):
+    """The record ids of an input, or None when an id repeats (duplicate ids join across records)."""
+    ids = [i for b in batches for i in b.ids]
+    return ids if len(set(ids)) == len(ids) else None
+
+
 def _lined_up(seq_batches, struct_batches):
     """(sequence text, structure text, record offsets) when the two FASTA inputs of the combined mode can be
-    scanned together -- unique ids (duplicate ids join across records), the same ids in the same order and the
-    same whole-record lengths, so that every window lines up -- else None (the inputs are then scanned apart
-    and merged as the reference does)."""
-    ids = [i for b in seq_batches for i in b.ids]
-    if len(set(ids)) != len(ids) or [i for b in struct_batches for i in b.ids] != ids:
+    scanned together -- unique ids, the same ids in the same order and the same whole-record lengths, so that
+    every window lines up -- else None (the inputs are then scanned apart and merged as the reference does)."""
+    ids = _unique_ids(seq_batches)
+    if ids is None or [i for b in struct_batches for i in b.ids] != ids:
         return None
     seq_text, offsets = _record_text(seq_batches)
     struct_text, struct_offsets = _record_text(struct_batches)
@@ -1583,13 +1584,13 @@ def _lined_up(seq_batches, struct_batches):
     return seq_text, struct_text, offsets
 
 
-def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, precomputed=None):
+def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, found=None):
     """The table of the combined mode (rnascan.py:416-434) on top of `seq_hits`, the sequence scan's table; None
     on ranks other than 0 under torchrun.  The structure side is scanned ON THE DEVICE only where the sequence
     score also passes (the inner join keeps nothing else): one fused launch instead of a second full scan +
     merge.  Where the two inputs cannot be scanned together (-t, different motif widths, duplicate ids, inputs
     that do not line up) the structure input is scanned on its own and merged as the reference does.
-    `precomputed`: the pair's hits on the profile directory, or its _PairHits on the structure FASTA input."""
+    `found`: the pair's joint _Found hits from the batched scan of its collection."""
     from . import device
     _, seq_pm = _first_motif(seq_pssm)
     motif_id, pm = _first_motif(struct_pssm)
@@ -1602,36 +1603,28 @@ def _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args,
     if _seq.is_seqrecord(struct_file) or seq_pm.length != width:
         return merged()
     seq_batches = _cached_batches(seq_file, IUPAC.IUPACUnambiguousRNA())
-    ids = [i for b in seq_batches for i in b.ids]
-    if len(set(ids)) != len(ids):
-        return merged()                   # duplicate ids join across records: keep the plain path
+    ids = _unique_ids(seq_batches)
+    if ids is None:
+        return merged()
     if os.path.isdir(struct_file):
         return _scan_profile_dir(struct_file, struct_pssm, args.minscore, args.debug, seq_batches, seq_pm, seq_hits,
-                                 getattr(args, "pack", False), precomputed)
+                                 getattr(args, "pack", False), found)
     struct_batches = _cached_batches(struct_file, structure)
     lined = _lined_up(seq_batches, struct_batches)
     if lined is None:
         return merged()
     seq_text, struct_text, offsets = lined
     eprint("Scanning sequences ")
-    if precomputed is not None:
-        eprint("Processed %d sequences" % sum(len(qb.ids) for qb in struct_batches))
-        hits = precomputed.joint
-    else:
+    if found is None:
         ts, tq = _table_for(seq_pm, "rna"), _table_for(pm, "struct")
-        parts, n_records = [], 0
-        for sb, qb in zip(seq_batches, struct_batches):
-            with STATS.phase("scan_s"):
-                pos, seq_sc, scores = device.scan_pair_onehot(sb.stream, qb.stream, ts, tq, args.minscore)
-            STATS.add("scored_positions", int(np.maximum(qb.stream.lengths - width + 1, 0).sum()))
-            keep, rec, start0 = qb.locate(pos)
-            parts.append((rec[keep] + n_records, start0[keep], seq_sc[keep], scores[keep]))
-            n_records += len(qb.ids)
-        eprint("Processed %d sequences" % n_records)
-        hits = _gather(parts or [(np.zeros(0, np.int64),) * 4])
-    if hits is None:
+        found = _Found(_scan_batches(
+            list(zip(seq_batches, struct_batches)),
+            lambda pair: device.scan_pair_onehot(pair[0].stream, pair[1].stream, ts, tq, args.minscore),
+            [width], [np.float32, np.float64]))
+    eprint("Processed %d sequences" % sum(len(qb.ids) for qb in struct_batches))
+    if found.hits is None:
         return None
-    rec, start0, seq_scores, scores = hits
+    rec, start0, seq_scores, scores = found.hits
     text_pos = offsets[rec] + start0
     struct_descs = [d for b in struct_batches for d in b.descriptions]
 
@@ -1699,10 +1692,22 @@ def _quiet(fn, *a, **kw):
         _QUIET -= 1
 
 
+def _side_tables(args, pfms, alphabet, bg_file, table, fasta=None):
+    """`table(pssm)` for the PSSM of every PFM of one side of a motif collection, with that side's background
+    (`bg_file`, uniform, or computed over `fasta`), all loaded quietly; None when anything raises (the per-motif
+    runs then report it)."""
+    bg_input = () if fasta is None else (fasta, alphabet, False)
+    try:
+        bg = _quiet(load_background, bg_file, args.uniform_background, *bg_input)
+        return [table(_first_motif(_quiet(load_motif, pfm, args.pseudocount, alphabet, bg))[1]) for pfm in pfms]
+    except Exception:
+        return None
+
+
 def _batched_profile_hits(args, seq_type, pairs):
-    """Hits of every motif pair on a directory of averaged profiles from one device.scan_batched call:
-    a list of (pos, seq_scores | None, struct_scores) per pair in packed-stream positions, or None when this
-    run does not have that shape (the per-motif scans then run one after the other)."""
+    """Hits of every motif pair on a directory of averaged profiles from one device.scan_batched call: a
+    (None, _Found) per pair, or None when this run does not have that shape (the per-motif scans then run one
+    after the other)."""
     from . import device
     if args.testseq or _world_size() > 1 or len(pairs) < 2 or not np.isfinite(args.minscore):
         return None
@@ -1711,41 +1716,46 @@ def _batched_profile_hits(args, seq_type, pairs):
         return None
     if not (args.bg_struct or args.uniform_background):
         return None                       # an averaged-profile run cannot compute a structure background
-    structure = ContextualSecondaryStructure()
-    try:
-        bg_struct = _quiet(load_background, args.bg_struct, args.uniform_background)
-        struct_pssms = [_quiet(pfm2pssm, q, args.pseudocount, structure, bg_struct) for _, q in pairs]
-        seq_pssms = seq_batches = None
-        if seq_type == "RNASS":
-            rna = IUPAC.IUPACUnambiguousRNA()
-            seq_file = args.fastafiles[0]
-            bg_seq = _quiet(load_background, args.bg_seq, args.uniform_background, seq_file, rna, False)
-            seq_pssms = [_quiet(pfm2pssm, p_, args.pseudocount, rna, bg_seq) for p_, _ in pairs]
-            if any(a.length != b.length for a, b in zip(seq_pssms, struct_pssms)):
-                return None
+    tqs = _side_tables(args, [q for _, q in pairs], ContextualSecondaryStructure(), args.bg_struct, _structure_table)
+    if tqs is None:
+        return None
+    tss = seq_batches = None
+    if seq_type == "RNASS":
+        rna = IUPAC.IUPACUnambiguousRNA()
+        seq_file = args.fastafiles[0]
+        tss = _side_tables(args, [p for p, _ in pairs], rna, args.bg_seq, lambda pm: _table_for(pm, "rna"), seq_file)
+        if tss is None or any(a.shape[0] != b.shape[0] for a, b in zip(tss, tqs)):
+            return None
+        try:
             seq_batches = _cached_batches(seq_file, rna)
-            ids = [i for b in seq_batches for i in b.ids]
-            if len(set(ids)) != len(ids):
-                return None
-    except Exception:
-        return None                       # the per-motif run reports what is wrong
-    tqs = [_structure_table(pm) for pm in struct_pssms]
-    tss = None if seq_pssms is None else [_table_for(pm, "rna") for pm in seq_pssms]
+        except Exception:
+            return None                   # the per-motif run reports what is wrong
+        if _unique_ids(seq_batches) is None:
+            return None
     if max(t.shape[0] for t in tqs) > 24:
         return None
     files, all_names, hp, lengths, names, offsets, codes = _profile_dir_streams(
         struct_file, args.debug, seq_batches, getattr(args, "pack", False))
     if not len(codes) or not device.filter_applies(np.concatenate(tqs), args.minscore, hp.absrow_max()):
         return None
+    hits = _profile_collection_hits(offsets, lengths, codes, hp, tss, tqs, args.minscore)
+    STATS.notes["batched_motifs"] = len(pairs)
+    return [(None, _Found(h)) for h in hits]
+
+
+def _profile_collection_hits(offsets, lengths, codes, hp, seq_tables, struct_tables, minscore):
+    """Hits of every motif (pair) on the streams of a profile directory (_profile_dir_streams) from one
+    device.scan_batched call: per motif (pair), the columns (file index, 0-based start, scores) -- (file index,
+    0-based start, sequence scores, structure scores) with `seq_tables`."""
+    from . import device
     with STATS.phase("scan_s"):
         stream = device.SymbolStream(codes, offsets, lengths)
         profile = device.ProfileStream(hp.rows)
-        motif, pos, sq, st, bases = device.scan_batched(stream, profile, tss, tqs, args.minscore)
-    STATS.notes["batched_motifs"] = len(pairs)
+        motif, pos, sq, st, bases = device.scan_batched(stream, profile, seq_tables, struct_tables, minscore)
     out = []
-    for k in range(len(pairs)):
-        a, b = int(bases[k]), int(bases[k + 1])
-        out.append((pos[a:b], None if sq is None else sq[a:b], st[a:b]))
+    for a, b in zip(bases[:-1].tolist(), bases[1:].tolist()):
+        rec = np.searchsorted(offsets, pos[a:b], side="right") - 1
+        out.append((rec, pos[a:b] - offsets[rec]) + (() if sq is None else (sq[a:b],)) + (st[a:b],))
     return out
 
 
@@ -1757,34 +1767,45 @@ def _on_device(batches):
     return all(b.stream.codes.is_cuda for b in batches)
 
 
+def _pair_on_device(seq_batches, struct_batches):
+    """True when the streams of both inputs are resident on a CUDA device (what the pair kernel reads).  Kept apart
+    from _on_device so that replacing one check (as the CPU tests do) opens only its own route."""
+    return all(b.stream.codes.is_cuda for b in list(seq_batches) + list(struct_batches))
+
+
+def _fasta_inputs(args, pairs, n_inputs):
+    """The `n_inputs` FASTA inputs of a motif collection run that a batched FASTA route can take -- no -t or
+    --bgonly, at least MULTI_FASTA_MIN_MOTIFS motifs, a finite -m, no directory -- else None."""
+    if args.testseq or args.bgonly or len(pairs) < MULTI_FASTA_MIN_MOTIFS or not np.isfinite(args.minscore):
+        return None
+    files = (args.fastafiles or [])[:n_inputs]
+    if len(files) < n_inputs or any(os.path.isdir(f) for f in files):
+        return None
+    return files
+
+
 def _batched_fasta_hits(args, seq_type, pairs):
     """Hits of every motif of a collection scanned over one FASTA input (modes RNA / SS) by
-    device.scan_onehot_many: a list of _FastaHits per motif, or None when this run does not have that shape (the
-    per-motif scans then run one after the other).  The background is taken once, quietly; every _run still
-    prints its own messages."""
-    if seq_type not in ("RNA", "SS") or args.testseq or args.bgonly or len(pairs) < MULTI_FASTA_MIN_MOTIFS:
+    device.scan_onehot_many: a (_Found, None) (RNA) or (None, _Found) (SS) per motif, or None when this run does
+    not have that shape (the per-motif scans then run one after the other).  The background is taken once,
+    quietly; every _run still prints its own messages."""
+    from . import device
+    files = _fasta_inputs(args, pairs, 1)
+    if seq_type not in ("RNA", "SS") or files is None:
         return None
-    if not np.isfinite(args.minscore) or not args.fastafiles or os.path.isdir(args.fastafiles[0]):
-        return None
-    fasta = args.fastafiles[0]
     if seq_type == "RNA":
         alphabet, kind, bg_file, pfms = IUPAC.IUPACUnambiguousRNA(), "rna", args.bg_seq, [p for p, _ in pairs]
     else:
         alphabet, kind, bg_file, pfms = ContextualSecondaryStructure(), "struct", args.bg_struct, [q for _, q in pairs]
-    batches = _cached_batches(fasta, alphabet)
+    batches = _cached_batches(files[0], alphabet)
     if not _on_device(batches):
         return None
-    try:
-        bg = _quiet(load_background, bg_file, args.uniform_background, fasta, alphabet, False)
-        pms = [_first_motif(_quiet(load_motif, pfm, args.pseudocount, alphabet, bg))[1] for pfm in pfms]
-    except Exception:
-        return None                       # the per-motif run reports what is wrong
-    tables = [_table_for(pm, kind) for pm in pms]
-    if max(t.shape[0] for t in tables) > 16:
+    tables = _side_tables(args, pfms, alphabet, bg_file, lambda pm: _table_for(pm, kind), files[0])
+    if tables is None or max(t.shape[0] for t in tables) > device.MANY_MAX_W:
         return None
-    hits = _fasta_many_hits(batches, kind, tables, args.minscore)
+    found = [_Found(h) for h in _fasta_many_hits(batches, kind, tables, args.minscore)]
     STATS.notes["batched_motifs"] = len(pairs)
-    return [_FastaHits(h) for h in hits]
+    return [(f, None) if kind == "rna" else (None, f) for f in found]
 
 
 def scan_many_fasta(fasta_file, pssms, alphabet, minscore):
@@ -1794,13 +1815,14 @@ def scan_many_fasta(fasta_file, pssms, alphabet, minscore):
     ContextualSecondaryStructure alphabet.  Returns one DataFrame per motif, equal to what
     scan_main(fasta_file, pssm, alphabet, bg, args) returns for that motif (empty frames on ranks other than 0
     under torchrun).  Motifs wider than 16 and a threshold of -inf are scanned one motif at a time."""
+    from . import device
     kind = _kind_of(alphabet)
     if kind not in ("rna", "struct"):
         raise NotImplementedError("scan_many_fasta takes the RNA or the ContextualSecondaryStructure alphabet")
     pms = [_first_motif(p) for p in pssms]
     tables = [_table_for(pm, kind) for _, pm in pms]
     batches = _cached_batches(fasta_file, alphabet)
-    many = [k for k, t in enumerate(tables) if t.shape[0] <= 16] if np.isfinite(minscore) else []
+    many = [k for k, t in enumerate(tables) if t.shape[0] <= device.MANY_MAX_W] if np.isfinite(minscore) else []
     hits = dict(zip(many, _fasta_many_hits(batches, kind, [tables[k] for k in many], minscore))) if many else {}
     frames = []
     for k, (motif_id, pm) in enumerate(pms):
@@ -1812,33 +1834,17 @@ def scan_many_fasta(fasta_file, pssms, alphabet, minscore):
     return frames
 
 
-class _PairHits(object):
-    """One motif pair's hits from the batched scans of its collection in the combined mode over two FASTA inputs:
-    `seq`, the sequence motif's _FastaHits, and `joint`, the pair's (record index, 0-based start, sequence scores,
-    structure scores) -- None on ranks other than 0 and for a pair whose two widths differ."""
-
-    def __init__(self, seq, joint):
-        self.seq, self.joint = seq, joint
-
-
-def _pair_on_device(seq_batches, struct_batches):
-    """True when the streams of both inputs are resident on a CUDA device (what the pair kernel reads)."""
-    return all(b.stream.codes.is_cuda for b in list(seq_batches) + list(struct_batches))
-
-
 def _batched_pair_hits(args, seq_type, pairs):
     """Hits of every motif pair of a collection in the combined mode over two FASTA inputs (RNASS): the sequence
     motifs' hits from device.scan_onehot_many and the joint hits of the equal-width pairs from
-    device.scan_pair_onehot_many, one call of each per device batch.  A list of _PairHits per pair, or None when
-    this run does not have that shape (the per-pair scans then run one after the other).  Both backgrounds are
-    taken once, quietly; every _run still prints its own messages."""
-    if seq_type != "RNASS" or args.testseq or args.bgonly or len(pairs) < MULTI_FASTA_MIN_MOTIFS:
+    device.scan_pair_onehot_many, one call of each per device batch.  A (_Found, _Found) per pair -- (_Found, None)
+    for a pair of unequal widths --, or None when this run does not have that shape (the per-pair scans then run
+    one after the other).  Both backgrounds are taken once, quietly; every _run still prints its own messages."""
+    from . import device
+    files = _fasta_inputs(args, pairs, 2)
+    if seq_type != "RNASS" or files is None:
         return None
-    if not np.isfinite(args.minscore) or len(args.fastafiles or []) < 2:
-        return None
-    seq_file, struct_file = args.fastafiles[:2]
-    if os.path.isdir(seq_file) or os.path.isdir(struct_file):
-        return None
+    seq_file, struct_file = files
     rna, structure = IUPAC.IUPACUnambiguousRNA(), ContextualSecondaryStructure()
     seq_batches = _cached_batches(seq_file, rna)
     struct_batches = _cached_batches(struct_file, structure)
@@ -1846,23 +1852,17 @@ def _batched_pair_hits(args, seq_type, pairs):
         return None
     if _lined_up(seq_batches, struct_batches) is None:
         return None
-    try:
-        bg_seq = _quiet(load_background, args.bg_seq, args.uniform_background, seq_file, rna, False)
-        bg_struct = _quiet(load_background, args.bg_struct, args.uniform_background, struct_file, structure, False)
-        seq_pssms = [_quiet(load_motif, p_, args.pseudocount, rna, bg_seq) for p_, _ in pairs]
-        struct_pssms = [_quiet(load_motif, q, args.pseudocount, structure, bg_struct) for _, q in pairs]
-    except Exception:
-        return None                       # the per-pair run reports what is wrong
-    ts = [_table_for(_first_motif(p)[1], "rna") for p in seq_pssms]
-    tq = [_table_for(_first_motif(p)[1], "struct") for p in struct_pssms]
-    same = [k for k in range(len(ts)) if ts[k].shape[0] == tq[k].shape[0]]
-    if max(t.shape[0] for t in ts + tq) > 16:
+    ts = _side_tables(args, [p for p, _ in pairs], rna, args.bg_seq, lambda pm: _table_for(pm, "rna"), seq_file)
+    tq = None if ts is None else _side_tables(args, [q for _, q in pairs], structure, args.bg_struct,
+                                              lambda pm: _table_for(pm, "struct"), struct_file)
+    if tq is None or max(t.shape[0] for t in ts + tq) > device.MANY_MAX_W:
         return None
+    same = [k for k in range(len(ts)) if ts[k].shape[0] == tq[k].shape[0]]
     seq_hits = _fasta_many_hits(seq_batches, "rna", ts, args.minscore)
     joint = dict(zip(same, _pair_many_hits(seq_batches, struct_batches, [ts[k] for k in same],
                                            [tq[k] for k in same], args.minscore))) if same else {}
     STATS.notes["batched_motifs"] = len(pairs)
-    return [_PairHits(_FastaHits(h), joint.get(k)) for k, h in enumerate(seq_hits)]
+    return [(_Found(h), _Found(joint[k]) if k in joint else None) for k, h in enumerate(seq_hits)]
 
 
 def scan_many_combined(seq_file, struct_file, seq_pssms, struct_pssms, minscore):
@@ -1892,7 +1892,6 @@ def scan_many(struct_dir, struct_pssms, minscore, seq_file=None, seq_pssms=None,
     returns them.  Returns one DataFrame per motif (pair): what scan_main(struct_dir, ...) returns for that
     structure motif alone -- limited, with seq_pssms, to the windows whose sequence score passes too, with
     an extra ``LogOdds.Seq`` column."""
-    from . import device
     if seq_pssms is not None and len(seq_pssms) != len(struct_pssms):
         raise ValueError("sequence and structure motif lists differ in length")
     seq_batches = None
@@ -1902,17 +1901,12 @@ def scan_many(struct_dir, struct_pssms, minscore, seq_file=None, seq_pssms=None,
     pms = [_first_motif(p) for p in struct_pssms]
     tqs = [_structure_table(pm) for _, pm in pms]
     tss = None if seq_pssms is None else [_table_for(_first_motif(p)[1], "rna") for p in seq_pssms]
-    stream = device.SymbolStream(codes, offsets, lengths)
-    profile = device.ProfileStream(hp.rows)
-    motif, pos, sq, st, bases = device.scan_batched(stream, profile, tss, tqs, minscore)
     frames = []
-    for k, (motif_id, pm) in enumerate(pms):
-        a, b = int(bases[k]), int(bases[k + 1])
-        rec = np.searchsorted(offsets, pos[a:b], side="right") - 1
-        start0 = pos[a:b] - offsets[rec]
-        frame = _averaged_dir_frame(all_names, rec, motif_id, start0, tqs[k].shape[0], st[a:b])
-        if sq is not None and len(frame.columns) > 2:
-            frame["LogOdds.Seq"] = _round3_f32(sq[a:b])
+    for (motif_id, _), tq, hits in zip(pms, tqs, _profile_collection_hits(offsets, lengths, codes, hp, tss, tqs,
+                                                                          minscore)):
+        frame = _averaged_dir_frame(all_names, hits[0], motif_id, hits[1], tq.shape[0], hits[-1])
+        if tss is not None and len(frame.columns) > 2:
+            frame["LogOdds.Seq"] = _round3_f32(hits[2])
         frames.append(frame)
     return frames
 
@@ -1996,8 +1990,9 @@ def _main(argv=None):
 
 def _run(args, seq_type, rank, precomputed=None):
     """One reference run (rnascan.py:490-567): backgrounds, motifs, scans, hits.tab on STDOUT.
-    `precomputed`: hits of this motif pair on the profile directory, of this motif on the FASTA input, or of this
-    pair on the two FASTA inputs (_PairHits), already found by the batched scans of its collection."""
+    `precomputed`: (sequence side, structure side) of this motif (pair) from the batched scans of its collection,
+    each a _Found or None where that side is scanned here."""
+    seq_found, struct_found = precomputed or (None, None)
     bg = None
     seq_file = struct_file = None
     seq_pssm = seq_hits = table = None
@@ -2026,9 +2021,7 @@ def _run(args, seq_type, rank, precomputed=None):
             sys.exit()
         if fused is None:                 # else: background, motif and scan were done in one overlapped pass
             seq_pssm = load_motif(args.pfm_seq, args.pseudocount, rna, bg)
-            seq_pre = precomputed.seq if isinstance(precomputed, _PairHits) else (
-                precomputed if seq_type == "RNA" else None)
-            seq_hits = _scan_table(seq_file, seq_pssm, rna, args, seq_pre)
+            seq_hits = _scan_table(seq_file, seq_pssm, rna, args, seq_found)
         table = seq_hits
 
     if seq_type in ["SS", "RNASS"]:
@@ -2055,9 +2048,9 @@ def _run(args, seq_type, rank, precomputed=None):
         if fused is None:
             struct_pssm = load_motif(args.pfm_struct, args.pseudocount, structure, bg)
             if seq_type == "RNASS":
-                table = _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, precomputed)
+                table = _combined_hits(seq_file, struct_file, seq_pssm, struct_pssm, seq_hits, args, struct_found)
             else:
-                table = _scan_table(struct_file, struct_pssm, structure, args, precomputed)
+                table = _scan_table(struct_file, struct_pssm, structure, args, struct_found)
 
     t_out = time.perf_counter()
     if rank == 0:
