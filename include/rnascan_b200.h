@@ -257,6 +257,16 @@ int rs_scan_fused(const uint8_t *d_codes, const void *d_profile, int profile_dty
                   int64_t *d_hit_pos, float *d_hit_seq, double *d_hit_struct,
                   uint64_t *d_counters2, void *d_work, int64_t work_bytes, void *stream);
 
+/* rs_scan_fused_seqfirst_counted : rs_scan_fused(RS_MODE_AND) for W <= 16, which rs_scan_fused itself runs
+ *     this way: the sequence scan first (exact table), then only the windows that pass it have their profile
+ *     rows read and scored.  Same hits, scores and order.  d_cand_counters2[0] = sequence candidates (above
+ *     hit_capacity => re-run larger), [1] = structure scores computed; d_counters2[0] = hits.               */
+int rs_scan_fused_seqfirst_counted(const uint8_t *d_codes, const void *d_profile, int profile_dtype, int64_t n,
+                                   const double *seq_table_Wx4, const double *struct_table_Wx7, int W,
+                                   double threshold, int64_t hit_capacity, int64_t *d_hit_pos,
+                                   float *d_hit_seq, double *d_hit_struct, uint64_t *d_cand_counters2,
+                                   uint64_t *d_counters2, void *d_work, int64_t work_bytes, void *stream);
+
 /* ---- one-hot threshold scans without waiting for the host's log-odds ---------------------
  * The exact log-odds need the host's libm (Python's math.log(p / b, 2), called by Biopython's
  * log_odds at rnascan.py:248) and the background counts (rnascan.py:445-457), i.e. a device ->

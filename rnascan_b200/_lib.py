@@ -80,6 +80,8 @@ _SIGS = {
     "rs_scan_onehot_begin": ([_int, _vp, _i64, _vp, _vp, _int, _dbl, _dbl, _i64, _vp, _i64, _vp], _int),
     "rs_scan_onehot_begin_notify": ([_int, _vp, _i64, _vp, _vp, _int, _dbl, _dbl, _i64, _vp, _i64, _vp, _u32, _vp,
                                      _vp], _int),
+    "rs_scan_fused_seqfirst_counted": ([_vp, _vp, _int, _i64, _vp, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _vp,
+                                        _vp, _i64, _vp], _int),
     "rs_scan_onehot_finish": ([_int, _vp, _i64, _vp, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _i64, _vp], _int),
     "rs_refine_hits_seq": ([_vp, _i64, _vp, _int, _dbl, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _vp], _int),
     "rs_scan_fused_candidates": ([_vp, _vp, _int, _i64, _vp, _int, _dbl, _dbl, _i64, _vp, _vp, _i64, _vp, _vp], _int),

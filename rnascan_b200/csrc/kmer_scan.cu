@@ -28,6 +28,7 @@
 // segment) with positions and exact scores written straight to their final, position-sorted place.
 #include "common.cuh"
 #include "provisional.cuh"
+#include <type_traits>
 
 #define KM_CONSUMERS   512                         // consumer threads (16 warps share one table; 2 CTAs per SM)
 #define KM_THREADS     (KM_CONSUMERS + 32)         // + one producer warp
@@ -249,6 +250,13 @@ struct ExpandParams {
     double ta[16 * 8];        // exact table, row stride A_STRIDE
     const uint8_t *codes_b;   // pair mode: structure stream scored with tb (row stride 8) into od.str
     double tb[16 * 8];
+    // profile mode (kmer_finish_kernel<4, PT>): every candidate whose exact sequence score passes gets its W profile
+    // rows scored with sd (row stride 7); od receives every candidate at its candidate index, position -1 unless
+    // both scores pass, and counters[1] counts the structure scores computed.  compact_hits_kernel then keeps the hits.
+    const void *profile;
+    double sd[16 * RS_CHANNELS];
+    unsigned long long *zero;  // compact_hits_kernel's ticket + aggregates, zeroed here
+    int n_zero;
 };
 
 __device__ __forceinline__ unsigned long long fin_block_scan(unsigned long long v, unsigned long long &total)
@@ -280,6 +288,12 @@ __device__ __forceinline__ unsigned long long fin_block_scan(unsigned long long 
     return s_w[warp] + incl - v;
 }
 
+__device__ __forceinline__ void add_warp_count(unsigned long long *counter, unsigned v)
+{
+    v = __reduce_add_sync(0xffffffffu, v);
+    if ((threadIdx.x & 31) == 0 && v) atomicAdd(counter, (unsigned long long)v);
+}
+
 // exact score of the (W <= 16)-symbol window at stream position `pos`: its bytes come from five aligned
 // words fetched together (ONE memory round trip per hit instead of W dependent ones; the padding of the
 // stream covers the over-read), then sequential fp64 adds in j order.
@@ -302,11 +316,14 @@ __device__ __forceinline__ double fin_window_score(const uint8_t *codes, int64_t
     return s;
 }
 
-// A = 4: float32 sequence scores (row stride 4); A = 7: float64 structure scores (row stride 8)
-template <int A>
+// A = 4: float32 sequence scores (row stride 4); A = 7: float64 structure scores (row stride 8).
+// PT = float or double: combined mode over the profile rows (see ExpandParams::profile).
+template <int A, typename PT = void>
 __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_constant__ ExpandParams prm)
 {
     constexpr int TS = A == 4 ? 4 : 8;
+    constexpr bool PROFILE = !std::is_void<PT>::value;
+    if (PROFILE) zero_words(prm.zero, prm.n_zero);
     __shared__ unsigned s_vb;
     if (threadIdx.x == 0) s_vb = (unsigned)atomicAdd(prm.wk.ticket, 1ull);
     __syncthreads();
@@ -362,9 +379,28 @@ __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_c
 #pragma unroll
         for (int i = 0; i < 8; i++) m[i] = make_uint4(0u, 0u, 0u, 0u);
     }
+    unsigned n_struct = 0;                                  // profile mode: structure scores this lane computed
     auto score_entry = [&](uint32_t e) {
         const unsigned long long kk = warp_k + (e >> 16);
         const int64_t pos = warp_pos + (e & 0xFFFFu);
+        if constexpr (PROFILE) {
+            if ((int64_t)kk >= prm.capacity) return;
+            // sequence first: only a window whose exact sequence score passes has its profile rows read
+            const double sq = fin_window_score<4, 4>(prm.codes, pos, prm.W, prm.ta);
+            bool is_hit = (double)(float)sq > prm.threshold;                    // _pwm.c:65 / note N1
+            if (is_hit) {
+                n_struct++;
+                const double sc = rs_exact_profile_window<PT>(
+                    reinterpret_cast<const PT *>(prm.profile) + pos * RS_CHANNELS, prm.sd, prm.W);
+                is_hit = sc > prm.threshold;                                     // rnascan.py:308, 416-434
+                if (is_hit) {
+                    prm.od.seq[kk] = (float)sq;
+                    prm.od.str[kk] = sc;
+                }
+            }
+            prm.od.pos[kk] = is_hit ? pos : -1;
+            return;
+        }
         if ((int64_t)kk < prm.capacity) {
             const double sc = fin_window_score<A, TS>(prm.codes, pos, prm.W, prm.ta);
             bool is_hit = true;
@@ -405,6 +441,7 @@ __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_c
         }
         __syncwarp();
         for (unsigned r = lane; r < warp_total; r += 32) score_entry(q[warp][r]);
+        if (PROFILE) add_warp_count(prm.counters + 1, n_struct);
         return;
     }
     // dense segments: word by word through a 64-entry ring of the same queue
@@ -437,6 +474,7 @@ __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_c
         }
     }
     while (count) drain(count < 32u ? count : 32u);
+    if (PROFILE) add_warp_count(prm.counters + 1, n_struct);
 }
 
 // ---- one-hot threshold scan, W <= 16, any alphabet: exact scores, hit bits by warp ballot ----------
@@ -640,6 +678,140 @@ static int finish_mask_scan(const uint8_t *d_codes, const KmerWork &wk, int64_t 
     return RS_OK;
 }
 
+struct OneHotGeom {
+    bool kmer;
+    int64_t n_tiles, n_segs, n_masks;
+    int n_ctas, ppm;
+};
+static OneHotGeom onehot_geom(int A, int W, int64_t n)
+{
+    OneHotGeom g;
+    g.kmer = A == 4 && W <= 8;
+    if (g.kmer) {
+        g.n_tiles = (n + KM_TILE - 1) / KM_TILE;
+        g.n_segs = g.n_tiles * KM_WARPS;
+        g.n_masks = g.n_tiles * KM_CONSUMERS;
+        g.ppm = KM_P;
+    } else {
+        g.n_tiles = (n + MS_TILE - 1) / MS_TILE;
+        g.n_segs = g.n_tiles * (MS_THREADS / 32);
+        g.n_masks = g.n_segs * 32;
+        g.ppm = 32;
+    }
+    g.n_ctas = fin_ctas(g.n_segs);
+    return g;
+}
+
+// ---- combined mode, sequence first: compaction of the candidates' verdicts ----------------------------------
+// kmer_finish_kernel<4, PT> leaves every candidate at its candidate index (position order) in the staging arrays,
+// position -1 unless both scores passed.  One thread per CP_PER consecutive candidates takes part in an exclusive
+// prefix sum of the survivors (CTAs chained by ticket + look-back, as in the finish kernel) and copies them out.
+#define CP_THREADS 1024
+#define CP_PER     8
+#define CP_SPAN    (CP_THREADS * CP_PER)
+
+struct CompactParams {
+    const int64_t *pos;                    // staged verdicts, capacity entries
+    const float *seq;
+    const double *str;
+    const unsigned long long *cand;        // [0] candidates (may exceed capacity), [1] structure scores computed
+    int64_t capacity;
+    unsigned long long *ticket, *agg;      // zeroed by the finish kernel
+    int n_ctas;
+    int64_t *out_pos;
+    float *out_seq;
+    double *out_str;
+    unsigned long long *counters;          // [0] hits, [1] structure scores computed
+};
+
+__global__ void __launch_bounds__(CP_THREADS) compact_hits_kernel(const __grid_constant__ CompactParams prm)
+{
+    __shared__ unsigned s_vb;
+    if (threadIdx.x == 0) s_vb = (unsigned)atomicAdd(prm.ticket, 1ull);
+    __syncthreads();
+    const unsigned vb = s_vb;
+    const unsigned long long n_cand = prm.cand[0];
+    const int64_t lim = (int64_t)n_cand < prm.capacity ? (int64_t)n_cand : prm.capacity;
+    const int64_t k0 = ((int64_t)vb * CP_THREADS + threadIdx.x) * CP_PER;
+    unsigned keep = 0;
+#pragma unroll
+    for (int i = 0; i < CP_PER; i++)
+        if (k0 + i < lim && prm.pos[k0 + i] >= 0) keep |= 1u << i;
+    unsigned long long total;
+    const unsigned long long excl = fin_block_scan((unsigned long long)__popc(keep), total);
+    if (threadIdx.x == 0) {
+        __threadfence();
+        ((volatile unsigned long long *)prm.agg)[vb] = total + 1ull;
+    }
+    unsigned long long part = 0;
+    for (unsigned p = threadIdx.x; p < vb; p += CP_THREADS) {
+        unsigned long long v;
+        unsigned spins = 0;
+        unsigned long long t_start = 0ull;
+        while ((v = ((volatile unsigned long long *)prm.agg)[p]) == 0ull) {
+            __nanosleep(20);
+            if ((++spins & 0xFFFFu) == 0u && rs_spin_expired(t_start)) __trap();   // a minute without the predecessor's aggregate
+        }
+        part += v - 1ull;
+    }
+    __threadfence();
+    unsigned long long before;
+    fin_block_scan(part, before);
+    if (vb == (unsigned)(prm.n_ctas - 1) && threadIdx.x == 0) {
+        // candidates beyond the staging room were never scored: report their count, an upper bound of the hits,
+        // so that the caller regrows the buffers
+        prm.counters[0] = (int64_t)n_cand > prm.capacity ? n_cand : before + total;
+        prm.counters[1] = prm.cand[1];
+        *prm.ticket = 0ull;
+    }
+    unsigned long long dst = before + excl;
+    for (uint32_t h = keep; h; h &= h - 1, dst++) {
+        const int64_t k = k0 + __ffs(h) - 1;
+        if ((int64_t)dst < prm.capacity) {
+            prm.out_pos[dst] = prm.pos[k];
+            prm.out_seq[dst] = prm.seq[k];
+            prm.out_str[dst] = prm.str[k];
+        }
+    }
+}
+
+// Finish of the sequence-first combined scan: the masks in the workspace hold the sequence candidates (exact or
+// provisional table); staging = the workspace's hit staging arrays, compaction state in its segment table.
+template <typename PT>
+static int finish_profile(const uint8_t *d_codes, const void *d_profile, int64_t n, const double *seq_table,
+                          const double *struct_table, int W, double threshold, int64_t cap, int64_t *d_hit_pos,
+                          float *d_hit_seq, double *d_hit_str, uint64_t *d_cand2, uint64_t *d_counters2,
+                          uint8_t *d_work, cudaStream_t st)
+{
+    const WorkLayout wl = rs_work_layout(n, cap);
+    const OneHotGeom g = onehot_geom(4, W, n);
+    ExpandParams ep = {};
+    carve_work(d_work + wl.off_lut, g.n_masks, g.n_segs, g.n_ctas, ep.wk);
+    ep.codes = d_codes; ep.n_segs = g.n_segs; ep.capacity = cap; ep.W = W; ep.ppm = g.ppm; ep.n_ctas = g.n_ctas;
+    ep.counters = (unsigned long long *)d_cand2; ep.threshold = threshold; ep.verify = 1;
+    int64_t *s_pos = (int64_t *)(d_work + wl.off_pos);
+    float *s_seq = (float *)(d_work + wl.off_seq);
+    double *s_str = (double *)(d_work + wl.off_str);
+    ep.od = OrderDest{s_pos, s_seq, s_str, nullptr, nullptr, 0};
+    for (int k = 0; k < W * 4; k++) ep.ta[k] = seq_table[k];
+    ep.profile = d_profile;
+    for (int k = 0; k < W * RS_CHANNELS; k++) ep.sd[k] = struct_table[k];
+    const int64_t span = cap < n ? cap : n;                   // never more candidates than windows
+    const int cp_ctas = (int)(span / CP_SPAN + 1);
+    unsigned long long *cp_state = (unsigned long long *)(d_work + wl.off_seg);   // ticket, pad, agg[cp_ctas]
+    ep.zero = cp_state; ep.n_zero = 2 + cp_ctas;
+    kmer_finish_kernel<4, PT><<<(unsigned)g.n_ctas, FIN_THREADS, 0, st>>>(ep);
+    RS_CUDA(cudaGetLastError());
+    CompactParams cp = {};
+    cp.pos = s_pos; cp.seq = s_seq; cp.str = s_str; cp.cand = (const unsigned long long *)d_cand2;
+    cp.capacity = cap; cp.ticket = cp_state; cp.agg = cp_state + 2; cp.n_ctas = cp_ctas;
+    cp.out_pos = d_hit_pos; cp.out_seq = d_hit_seq; cp.out_str = d_hit_str;
+    cp.counters = (unsigned long long *)d_counters2;
+    compact_hits_kernel<<<(unsigned)cp_ctas, CP_THREADS, 0, st>>>(cp);
+    RS_CUDA(cudaGetLastError());
+    return RS_OK;
+}
+
 template <int W>
 static int launch_kmer(const KmerParams &prm, cudaStream_t stream)
 {
@@ -672,29 +844,6 @@ int64_t rs_kmer_work_bytes(int64_t n)
 // begin : decision masks + segment counts into the workspace (k-mer table scan for A = 4, W <= 8, ballot
 //         mask scan otherwise), from the exact host table or from a device-resident provisional table;
 // finish: segment prefix + expansion with the exact host table (verify = the masks were only candidates).
-struct OneHotGeom {
-    bool kmer;
-    int64_t n_tiles, n_segs, n_masks;
-    int n_ctas, ppm;
-};
-static OneHotGeom onehot_geom(int A, int W, int64_t n)
-{
-    OneHotGeom g;
-    g.kmer = A == 4 && W <= 8;
-    if (g.kmer) {
-        g.n_tiles = (n + KM_TILE - 1) / KM_TILE;
-        g.n_segs = g.n_tiles * KM_WARPS;
-        g.n_masks = g.n_tiles * KM_CONSUMERS;
-        g.ppm = KM_P;
-    } else {
-        g.n_tiles = (n + MS_TILE - 1) / MS_TILE;
-        g.n_segs = g.n_tiles * (MS_THREADS / 32);
-        g.n_masks = g.n_segs * 32;
-        g.ppm = 32;
-    }
-    g.n_ctas = fin_ctas(g.n_segs);
-    return g;
-}
 
 template <int A>
 static int onehot_begin(const uint8_t *d_codes, int64_t n, const double *table, const uint64_t *d_counts8,
@@ -780,6 +929,28 @@ int rs_scan_seq_kmer(const uint8_t *d_codes, int64_t n, const double *table, int
 {
     return rs_scan_onehot_masks(4, d_codes, n, table, W, threshold, cap, d_hit_pos, d_hit_score, nullptr, d_counters2,
                                 d_work, st);
+}
+
+// Combined mode (RS_MODE_AND) of rs_scan_fused for W <= 16, sequence first: the k-mer / mask scan with the exact
+// sequence table, then only the windows that pass it have their profile rows read and scored.  Same hits, scores and
+// order as the structure-first kernels (same exact arithmetic).  d_cand2 (device, or NULL = inside the workspace):
+// [0] sequence candidates, [1] structure scores computed; d_counters2[0] = hits (the candidate count instead when
+// the candidates outgrew hit_capacity: regrow), [1] = structure scores computed.
+int rs_scan_fused_seqfirst(const uint8_t *d_codes, const void *d_profile, int profile_dtype, int64_t n,
+                           const double *seq_table, const double *struct_table, int W, double threshold, int64_t cap,
+                           int64_t *d_hit_pos, float *d_hit_seq, double *d_hit_str, uint64_t *d_cand2,
+                           uint64_t *d_counters2, void *d_work, cudaStream_t st)
+{
+    const WorkLayout wl = rs_work_layout(n, cap);
+    uint8_t *wk = (uint8_t *)d_work;
+    int rc = onehot_begin<4>(d_codes, n, seq_table, nullptr, nullptr, 0.0, W, threshold, wk + wl.off_lut, st);
+    if (rc) return rc;
+    if (!d_cand2) d_cand2 = (uint64_t *)(wk + wl.off_scan);      // unused by this path otherwise
+    return profile_dtype == RS_F64
+        ? finish_profile<double>(d_codes, d_profile, n, seq_table, struct_table, W, threshold, cap, d_hit_pos,
+                                 d_hit_seq, d_hit_str, d_cand2, d_counters2, wk, st)
+        : finish_profile<float>(d_codes, d_profile, n, seq_table, struct_table, W, threshold, cap, d_hit_pos,
+                                d_hit_seq, d_hit_str, d_cand2, d_counters2, wk, st);
 }
 
 static int begin_finish_args(int alphabet, const uint8_t *d_codes, int64_t n, int W, double threshold)

@@ -521,6 +521,15 @@ static int scan_fused_impl(const uint8_t *d_codes, const void *d_profile, int pr
     WorkLayout wl = rs_work_layout(n, hit_capacity);
     if (!d_work || work_bytes < wl.total) { rs_set_error("workspace too small: need %lld bytes", (long long)wl.total); return RS_ERR_WORKSPACE; }
 
+    // Combined mode: a window's profile rows only matter where its sequence score passes too (combine() is an AND,
+    // rnascan.py:416-434) -- a fraction of a per cent of the windows at typical thresholds -- so the sequence scan
+    // runs first and the rows of its hits alone are read (DESIGN.md 3.1).  Batched and staged callers keep the
+    // structure-first kernels.
+    if (mode == RS_MODE_AND && W <= RS_KMER_WMAX && !staged_tiles_out && !d_counts8 && !d_out_base && !d_hit_motif)
+        return rs_scan_fused_seqfirst(d_codes, d_profile, profile_dtype, n, seq_table, struct_table, W, threshold,
+                                      hit_capacity, d_hit_pos, d_hit_seq, d_hit_struct, nullptr, d_counters2, d_work,
+                                      st);
+
     ProfileParams prm = {};
     prm.codes = d_codes; prm.profile = d_profile; prm.n = n; prm.padded = rs_padded_count(n);
     prm.threshold = threshold; prm.mode = mode; prm.W = W; prm.dense = 0;
@@ -628,6 +637,35 @@ extern "C" int rs_scan_fused(const uint8_t *d_codes, const void *d_profile, int 
     return scan_fused_impl(d_codes, d_profile, profile_dtype, n, seq_table, struct_table, W, threshold,
                            profile_absrow_max, mode, hit_capacity, d_hit_pos, d_hit_seq, d_hit_struct, d_counters2,
                            d_work, work_bytes, stream, nullptr, nullptr, 0);
+}
+
+extern "C" int rs_scan_fused_seqfirst_counted(const uint8_t *d_codes, const void *d_profile, int profile_dtype,
+                                              int64_t n, const double *seq_table, const double *struct_table, int W,
+                                              double threshold, int64_t hit_capacity, int64_t *d_hit_pos,
+                                              float *d_hit_seq, double *d_hit_struct, uint64_t *d_cand_counters2,
+                                              uint64_t *d_counters2, void *d_work, int64_t work_bytes, void *stream)
+{
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc = check_common(d_profile, profile_dtype, n, struct_table, W);
+    if (rc) return rc;
+    if (!d_codes || ((uintptr_t)d_codes & 15)) { rs_set_error("codes pointer null or not 16-byte aligned"); return RS_ERR_INVALID; }
+    if (W > RS_KMER_WMAX) { rs_set_error("the sequence-first scan covers motif widths 1..%d (got %d)", RS_KMER_WMAX, W); return RS_ERR_INVALID; }
+    if (!seq_table || !d_cand_counters2 || !d_counters2 || hit_capacity < 0 ||
+        (hit_capacity > 0 && (!d_hit_pos || !d_hit_seq || !d_hit_struct))) {
+        rs_set_error("rs_scan_fused_seqfirst_counted: bad argument"); return RS_ERR_INVALID;
+    }
+    if ((const void *)d_cand_counters2 == (const void *)d_counters2) { rs_set_error("d_cand_counters2 and d_counters2 must differ"); return RS_ERR_INVALID; }
+    if (threshold != threshold) { rs_set_error("threshold is NaN"); return RS_ERR_INVALID; }
+    if (n < W) {
+        RS_CUDA(cudaMemsetAsync(d_counters2, 0, 2 * sizeof(uint64_t), st));
+        RS_CUDA(cudaMemsetAsync(d_cand_counters2, 0, 2 * sizeof(uint64_t), st));
+        return RS_OK;
+    }
+    WorkLayout wl = rs_work_layout(n, hit_capacity);
+    if (!d_work || work_bytes < wl.total) { rs_set_error("workspace too small: need %lld bytes", (long long)wl.total); return RS_ERR_WORKSPACE; }
+    return rs_scan_fused_seqfirst(d_codes, d_profile, profile_dtype, n, seq_table, struct_table, W, threshold,
+                                  hit_capacity, d_hit_pos, d_hit_seq, d_hit_struct, d_cand_counters2, d_counters2,
+                                  d_work, st);
 }
 
 // ---- filter + gather + resolve: candidate positions only; the exact rows live on the host (resolve.cu)

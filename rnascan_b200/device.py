@@ -491,17 +491,24 @@ class BackgroundFusedScan(object):
     The reference runs compute_background over the whole input, then builds the log-odds, then
     scans (rnascan.py:507-521).  Only the SEQUENCE table depends on those counts (the averaged
     profile mode cannot compute a structure background, rnascan.py:533-540), and combine() is an
-    AND of two separately thresholded result sets (rnascan.py:416-434).  So the structure-only
-    candidate scan starts at once on the caller's stream while histogram -> all-reduce -> counts
-    D2H run on a side stream and the host turns the counts into the sequence table;
-    rs_refine_hits_seq then keeps the candidates whose sequence score passes too.  Results are
-    identical to histogram -> tables -> rs_scan_fused(RS_MODE_AND).
+    AND of two separately thresholded result sets (rnascan.py:416-434).
+
+    W <= 16 (sequence first): histogram -> (all-reduce) -> counts to the host -> exact sequence table ->
+    rs_scan_fused_seqfirst_counted, which reads the profile rows of the windows whose sequence score
+    passes and of no other (a fraction of a per cent of the 28 B per position at typical thresholds).
+
+    W > 16, or structure_first=True (kept for A/B measurements): the structure-only candidate scan
+    starts at once on the caller's stream while histogram -> all-reduce -> counts D2H run on a side
+    stream; rs_scan_fused_resolve then keeps the candidates whose sequence score passes too.
+
+    Both orders give results identical to histogram -> tables -> rs_scan_fused(RS_MODE_AND).
     """
 
-    def __init__(self, n, device=None, capacity=None):
+    def __init__(self, n, device=None, capacity=None, structure_first=False):
         require_cuda()
         self.device = torch.device(device or "cuda")
         self.n = int(n)
+        self.structure_first = bool(structure_first)
         self.side = torch.cuda.Stream(device=self.device, priority=-1)
         self.counts = torch.zeros(8, dtype=torch.int64, device=self.device)
         self.counts_host = torch.zeros(8, dtype=torch.int64).pin_memory()
@@ -523,6 +530,9 @@ class BackgroundFusedScan(object):
         n, hb = self.n, self.hb
         tq = _table(struct_table, 7)
         main = torch.cuda.current_stream(self.device)
+        if W <= self.SEQUENCE_FIRST_MAX_W and not self.structure_first:
+            return self._launch_sequence_first(codes, profile_rows, profile_dtype, W, tq, seq_table_fn, threshold,
+                                               all_reduce, main)
         self.side.wait_stream(main)                         # inputs ready; previous pass finished with the buffers
         # the big kernel first, so that the host-side cost of the side-stream calls (the collective above
         # all) is spent while the device is already busy
@@ -570,6 +580,28 @@ class BackgroundFusedScan(object):
                                         _ptr(hb.counters), _ptr(hb.work), hb.work_bytes, main.cuda_stream))
         main.wait_stream(self.side)
         self.launches = 3          # hist, candidate scan, sequence check + ordering
+        return ts
+
+    SEQUENCE_FIRST_MAX_W = 16
+
+    def _launch_sequence_first(self, codes, profile_rows, profile_dtype, W, tq, seq_table_fn, threshold, all_reduce,
+                               main):
+        n, hb = self.n, self.hb
+        self.counts.zero_()
+        check(lib.rs_hist_rna(_ptr(codes), n, _ptr(self.counts), main.cuda_stream))
+        if all_reduce is not None:
+            all_reduce(self.counts)                         # the path's only collective
+        self.counts_host.copy_(self.counts, non_blocking=True)
+        self.ready.record(main)
+        self.ready.synchronize()
+        ts = _table(seq_table_fn(self.counts_host.numpy()), 4)
+        if ts.shape[0] != W:
+            raise ValueError("sequence and structure motifs must have the same width")
+        check(lib.rs_scan_fused_seqfirst_counted(_ptr(codes), _ptr(profile_rows), profile_dtype, n, ts.ctypes.data,
+                                                 tq.ctypes.data, W, float(threshold), hb.capacity, _ptr(hb.pos),
+                                                 _ptr(hb.seq), _ptr(hb.struct), _ptr(hb.cand_counters),
+                                                 _ptr(hb.counters), _ptr(hb.work), hb.work_bytes, main.cuda_stream))
+        self.launches = 5          # hist, decision table, sequence scan, finish (profile rows), compaction
         return ts
 
     def results(self):
