@@ -40,6 +40,7 @@
 #define KM_WARPS       (KM_CONSUMERS / 32)
 #define KM_SEG         (32 * KM_P)                 // 896 positions per warp segment
 #define FIN_THREADS    1024                        // segments per CTA of the finish kernel (one per thread)
+#define FIN_STAGE_BYTES 6048                       // profile finish: per-warp stage, 29 float windows of W <= 7
 
 struct KmerWork {                 // carved out of the caller's workspace
     uint8_t  *lut;                // [65536]
@@ -250,9 +251,10 @@ struct ExpandParams {
     double ta[16 * 8];        // exact table, row stride A_STRIDE
     const uint8_t *codes_b;   // pair mode: structure stream scored with tb (row stride 8) into od.str
     double tb[16 * 8];
-    // profile mode (kmer_finish_kernel<4, PT>): every candidate whose exact sequence score passes gets its W profile
-    // rows scored with sd (row stride 7); od receives every candidate at its candidate index, position -1 unless
-    // both scores pass, and counters[1] counts the structure scores computed.  compact_hits_kernel then keeps the hits.
+    // profile mode (kmer_finish_kernel<4, PT>): every candidate gets its W profile rows scored with sd (row stride 7),
+    // and its exact sequence score is recomputed where the structure score passes; od receives every candidate at its
+    // candidate index, position -1 unless both scores pass, and counters[1] counts the structure scores computed.
+    // compact_hits_kernel then keeps the hits.
     const void *profile;
     double sd[16 * RS_CHANNELS];
     unsigned long long *zero;  // compact_hits_kernel's ticket + aggregates, zeroed here
@@ -314,6 +316,17 @@ __device__ __forceinline__ double fin_window_score(const uint8_t *codes, int64_t
         }
     }
     return s;
+}
+
+// 16-byte global -> shared copy that bypasses the registers (LDGSTS); cp_async_wait_all waits for all of this
+// thread's copies (the other lanes' copies are visible after a __syncwarp that follows their wait)
+__device__ __forceinline__ void cp_async16(void *dst, const void *src)
+{
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all()
+{
+    asm volatile("cp.async.wait_all;" ::: "memory");
 }
 
 // A = 4: float32 sequence scores (row stride 4); A = 7: float64 structure scores (row stride 8).
@@ -379,28 +392,9 @@ __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_c
 #pragma unroll
         for (int i = 0; i < 8; i++) m[i] = make_uint4(0u, 0u, 0u, 0u);
     }
-    unsigned n_struct = 0;                                  // profile mode: structure scores this lane computed
     auto score_entry = [&](uint32_t e) {
         const unsigned long long kk = warp_k + (e >> 16);
         const int64_t pos = warp_pos + (e & 0xFFFFu);
-        if constexpr (PROFILE) {
-            if ((int64_t)kk >= prm.capacity) return;
-            // sequence first: only a window whose exact sequence score passes has its profile rows read
-            const double sq = fin_window_score<4, 4>(prm.codes, pos, prm.W, prm.ta);
-            bool is_hit = (double)(float)sq > prm.threshold;                    // _pwm.c:65 / note N1
-            if (is_hit) {
-                n_struct++;
-                const double sc = rs_exact_profile_window<PT>(
-                    reinterpret_cast<const PT *>(prm.profile) + pos * RS_CHANNELS, prm.sd, prm.W);
-                is_hit = sc > prm.threshold;                                     // rnascan.py:308, 416-434
-                if (is_hit) {
-                    prm.od.seq[kk] = (float)sq;
-                    prm.od.str[kk] = sc;
-                }
-            }
-            prm.od.pos[kk] = is_hit ? pos : -1;
-            return;
-        }
         if ((int64_t)kk < prm.capacity) {
             const double sc = fin_window_score<A, TS>(prm.codes, pos, prm.W, prm.ta);
             bool is_hit = true;
@@ -414,6 +408,57 @@ __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_c
             if (A == 4 && prm.codes_b)                                     // pair mode: structure score of the same window
                 prm.od.str[kk] = fin_window_score<7, 8>(prm.codes_b, pos, prm.W, prm.tb);
             if (prm.od.out_motif) prm.od.out_motif[kk] = prm.od.motif_id;
+        }
+    };
+    // Profile mode: the windows of queue entries first .. first + n - 1 (slot index & qm), in rounds of R.  A window's
+    // W rows are 28 W (float) or 56 W (double) contiguous bytes; the lanes copy the 16-byte pieces of every window's
+    // aligned hull into the warp's stage (all copies of a round in flight together, neighbouring windows served by the
+    // same lines), then each lane scores one window from shared memory with the exact arithmetic.  Only a window whose
+    // structure score passes has its symbols re-read for the sequence score.  The masks come from the exact sequence
+    // table, so every in-capacity candidate is a structure score computed (counters[1]).
+    using RowT = std::conditional_t<PROFILE, PT, float>;
+    constexpr unsigned ROWB = RS_CHANNELS * sizeof(RowT);
+    const unsigned WB = (unsigned)prm.W * ROWB;
+    const unsigned NP = (WB + (16 - (unsigned)sizeof(RowT)) + 15) / 16;      // pieces of the widest hull
+    const unsigned R = min(32u, (unsigned)FIN_STAGE_BYTES / (NP * 16));
+    extern __shared__ __align__(16) uint8_t fin_stage[];
+    unsigned n_struct = 0;
+    auto score_profile = [&](unsigned first, unsigned n, unsigned qm) {
+        uint8_t *stage = fin_stage + warp * FIN_STAGE_BYTES;
+        const uint8_t *rows = reinterpret_cast<const uint8_t *>(prm.profile);
+        for (unsigned r0 = 0; r0 < n; r0 += R) {
+            const unsigned nr = min(R, n - r0);
+            for (unsigned p = lane; p < nr * NP; p += 32) {
+                const unsigned i = p / NP, k = p - i * NP;
+                const uint32_t e = q[warp][(first + r0 + i) & qm];
+                const int64_t b = (warp_pos + (e & 0xFFFFu)) * ROWB;
+                const int64_t a = (b & ~(int64_t)15) + 16 * k;
+                if ((int64_t)(warp_k + (e >> 16)) < prm.capacity && a < b + WB)
+                    cp_async16(stage + (i * NP + k) * 16, rows + a);
+            }
+            cp_async_wait_all();
+            __syncwarp();
+            if ((unsigned)lane < nr) {
+                const uint32_t e = q[warp][(first + r0 + lane) & qm];
+                const unsigned long long kk = warp_k + (e >> 16);
+                const int64_t pos = warp_pos + (e & 0xFFFFu);
+                if ((int64_t)kk < prm.capacity) {
+                    n_struct++;
+                    const RowT *win = reinterpret_cast<const RowT *>(stage + lane * NP * 16 + ((pos * ROWB) & 15));
+                    const double sc = rs_exact_profile_window<RowT>(win, prm.sd, prm.W);
+                    bool is_hit = sc > prm.threshold;                                // rnascan.py:308, 416-434
+                    if (is_hit) {
+                        const double sq = fin_window_score<4, 4>(prm.codes, pos, prm.W, prm.ta);
+                        is_hit = (double)(float)sq > prm.threshold;                  // _pwm.c:65 / note N1
+                        if (is_hit) {
+                            prm.od.seq[kk] = (float)sq;
+                            prm.od.str[kk] = sc;
+                        }
+                    }
+                    prm.od.pos[kk] = is_hit ? pos : -1;
+                }
+            }
+            __syncwarp();
         }
     };
     // queue slots by a warp prefix over the lanes' hit counts (== segcnt): no per-slot coordination
@@ -440,36 +485,69 @@ __global__ void __launch_bounds__(FIN_THREADS) kmer_finish_kernel(const __grid_c
             }
         }
         __syncwarp();
-        for (unsigned r = lane; r < warp_total; r += 32) score_entry(q[warp][r]);
-        if (PROFILE) add_warp_count(prm.counters + 1, n_struct);
+        if constexpr (PROFILE) {
+            score_profile(0, warp_total, QCAP - 1);
+            add_warp_count(prm.counters + 1, n_struct);
+        } else {
+            for (unsigned r = lane; r < warp_total; r += 32) score_entry(q[warp][r]);
+        }
         return;
     }
     // dense segments: word by word through a 64-entry ring of the same queue
     unsigned head = 0, count = 0, koff = koff0;            // head, count: warp-uniform ring state
     auto drain = [&](unsigned n_take) {
         __syncwarp();
-        if ((unsigned)lane < n_take) score_entry(q[warp][(head + lane) & 63u]);
+        if constexpr (PROFILE) score_profile(head, n_take, 63u);
+        else if ((unsigned)lane < n_take) score_entry(q[warp][(head + lane) & 63u]);
         __syncwarp();
         head = (head + n_take) & 63u;
         count -= n_take;
     };
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const uint32_t w4[4] = {m[i].x, m[i].y, m[i].z, m[i].w};
-#pragma unroll
-        for (int t = 0; t < 4; t++) {
-            uint32_t h = w4[t];
-            const unsigned poff = (unsigned)((lane * 32 + i * 4 + t) * prm.ppm);
+    if constexpr (PROFILE) {
+        // the words in a run-time loop: one copy of the round code here instead of one per word (32 copies of a
+        // profile round do not fit the instruction cache); the groups after the second are fetched again, one
+        // group ahead, so that only two stay in registers
+        const uint4 *mv = reinterpret_cast<const uint4 *>(prm.wk.mask + seg * 32);
+        uint4 cur = m[0], nxt = m[1];
+#pragma unroll 1
+        for (int w = 0; w < 32; w++) {
+            uint32_t h = (w & 2) ? ((w & 1) ? cur.w : cur.z) : ((w & 1) ? cur.y : cur.x);
+            if ((w & 3) == 3) {
+                cur = nxt;
+                if (w < 24) nxt = segcnt ? mv[(w >> 2) + 2] : make_uint4(0u, 0u, 0u, 0u);
+            }
+            const unsigned poff = (unsigned)((lane * 32 + w) * prm.ppm);
             for (;;) {
                 const unsigned has = __ballot_sync(0xffffffffu, h != 0);
                 if (!has) break;
-                if (count > 32u) drain(32u);
+                while (count >= R) drain(R);                      // whole rounds
                 if (h) {
                     const unsigned e = (head + count + __popc(has & ((1u << lane) - 1u))) & 63u;
                     q[warp][e] = (koff++ << 16) | (poff + (unsigned)(__ffs(h) - 1));
                     h &= h - 1;
                 }
                 count += __popc(has);
+            }
+        }
+    } else {
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const uint32_t w4[4] = {m[i].x, m[i].y, m[i].z, m[i].w};
+#pragma unroll
+            for (int t = 0; t < 4; t++) {
+                uint32_t h = w4[t];
+                const unsigned poff = (unsigned)((lane * 32 + i * 4 + t) * prm.ppm);
+                for (;;) {
+                    const unsigned has = __ballot_sync(0xffffffffu, h != 0);
+                    if (!has) break;
+                    if (count > 32u) drain(32u);
+                    if (h) {
+                        const unsigned e = (head + count + __popc(has & ((1u << lane) - 1u))) & 63u;
+                        q[warp][e] = (koff++ << 16) | (poff + (unsigned)(__ffs(h) - 1));
+                        h &= h - 1;
+                    }
+                    count += __popc(has);
+                }
             }
         }
     }
@@ -800,7 +878,14 @@ static int finish_profile(const uint8_t *d_codes, const void *d_profile, int64_t
     const int cp_ctas = (int)(span / CP_SPAN + 1);
     unsigned long long *cp_state = (unsigned long long *)(d_work + wl.off_seg);   // ticket, pad, agg[cp_ctas]
     ep.zero = cp_state; ep.n_zero = 2 + cp_ctas;
-    kmer_finish_kernel<4, PT><<<(unsigned)g.n_ctas, FIN_THREADS, 0, st>>>(ep);
+    constexpr size_t smem = (size_t)(FIN_THREADS / 32) * FIN_STAGE_BYTES;     // the warps' window stages
+    static bool configured[RS_MAX_DEVICES] = {};          // the attribute is per device
+    const int dev = rs_current_device();
+    if (!configured[dev]) {
+        RS_CUDA(cudaFuncSetAttribute(kmer_finish_kernel<4, PT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        configured[dev] = true;
+    }
+    kmer_finish_kernel<4, PT><<<(unsigned)g.n_ctas, FIN_THREADS, smem, st>>>(ep);
     RS_CUDA(cudaGetLastError());
     CompactParams cp = {};
     cp.pos = s_pos; cp.seq = s_seq; cp.str = s_str; cp.cand = (const unsigned long long *)d_cand2;
